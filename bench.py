@@ -1,10 +1,13 @@
 #!/usr/bin/env python3
 """RawBoost throughput benchmark: augmented utterances/sec on 64600-sample 16 kHz synthetic waveforms.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--algo 5] [--batch 4096] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--algo 5] [--batch 4096] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (process_Rawboost_feature, fused on the device) over one batch of synthetic
-utterances. Rank 0 prints ONE JSON line.
+utterances. Rank 0 prints ONE JSON line. ``--dump-outputs DIR`` also writes rank 0's result of the last timed step of the
+headline configuration (inputs are seeded, so two builds can be compared output for output): ``DIR/y.npy`` (float32
+[rows, length], every utterance of the batch or a fixed seeded sample of them, under 64 MB) and ``DIR/rows.npy`` (their batch
+rows, float64).
 
 * N = 1 (the default): BASELINE config 3 -- algo 5, 4096 utterances resident on the GPU. The same line carries, under
   ``configs``, the other configurations the metric names (algo 1 / 3 at 4096, config 2 = algo 2 and 3 at 1024, config 4 =
@@ -464,6 +467,22 @@ class Bench:
                 "ok": bool(worst <= (0.0 if algo == 2 else 1e-5))}
 
 
+DUMP_BYTES = 60 * 2 ** 20  # --dump-outputs stays under 64 MB: larger batches are sampled by row
+
+
+def dump_outputs(path, y, B, length):
+    """Write rows of the [B, ld] result ``y`` (their first ``length`` samples, float32) to ``path/y.npy`` and their batch
+    indices to ``path/rows.npy``; every row when they fit DUMP_BYTES, otherwise a sample fixed by its own seed (at least one
+    row, cut to its first DUMP_BYTES / 4 samples when a single row is larger than that)."""
+    import torch
+    cols = min(length, DUMP_BYTES // 4)
+    n = min(B, DUMP_BYTES // (4 * cols))
+    rows = np.arange(B) if n == B else np.sort(np.random.RandomState(0).choice(B, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "y.npy"), y[torch.from_numpy(rows).to(y.device), :cols].cpu().numpy())
+    np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+
+
 def gpu_arm(a):
     b = Bench(a)
     torch, eng, sharding, workload = b.torch, b.eng, b.sharding, b.workload
@@ -481,6 +500,8 @@ def gpu_arm(a):
     # ---- device-resident timing of the headline configuration -----------------------------------------------------------------
     rec, (x, ln, dp, y, bp, seeds, ld) = b.resident(algo, B, L, a.steps, a.warmup, lo=lo, planner=a.bank_planner, parity_n=16,
                                                       clocks=True, keep=True)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, y, B, L)
     if bp is not None and rank == 0:  # guard: the native planner must reproduce numpy's own draws on a sample
         from scl_deepfake_audio_detection_b200 import plans as _pl
         ref = _pl.draw_batch([L] * 4, workload.SAMPLE_RATE, b.args, algo, seeds=seeds[:4], ld=ld)
@@ -854,7 +875,8 @@ def emit(line: dict):
 def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of the headline configuration (its 'value', and what "
+                    "--dump-outputs writes); the sub-records under 'configs' and 'e2e' time their own step counts and report them")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--algo", type=int, default=5, help="RawBoost algo (BASELINE config 3: algo 5 = LnL -> ISD)")
@@ -873,7 +895,12 @@ def main():
     ap.add_argument("--no-config4", action="store_true")
     ap.add_argument("--no-config5", action="store_true")
     ap.add_argument("--cpu-per-core", type=int, default=32, help="utterances per host core per CPU-baseline step (SURVEY.md 8d: >= 32)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline configuration's last timed result to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     quiet_stdout()
     if a.impl == "reference":

@@ -3,7 +3,7 @@
 
 Run in the build container only (``/root/reference`` does not exist on the GPU box):
 
-    python oracle/make_golden.py            # rewrites tests/golden/rawboost_golden.*
+    python oracle/make_golden.py            # rewrites tests/golden/rawboost_golden.* (npz parts of at most 1 MB)
     python oracle/make_golden.py --multiview   # tests/golden/multiview_golden.*
     python oracle/make_golden.py --round2      # tests/golden/round2_golden.* (edge inputs, long utterances, reverb, __getitem__)
 
@@ -32,6 +32,7 @@ REF = "/root/reference"
 OUT = os.path.join(ROOT, "tests", "golden")
 
 sys.path.insert(0, ROOT)
+from oracle import golden_files  # noqa: E402
 from oracle.rawboost_oracle import (CORPUS_IDS, CORPUS_VOCODERS, corpus_wave, make_args, overscale_utterance, seed_for,  # noqa: E402
                                     synth_utterance)
 
@@ -176,11 +177,11 @@ def main():
                 s["stream"] = stream_digest()
                 meta["full"][f"algo{algo}_loud{loud}_u{u}"] = s
 
-    np.savez_compressed(os.path.join(OUT, "rawboost_golden.npz"), **arrays)
+    paths = golden_files.save(OUT, "rawboost_golden", arrays)
     with open(os.path.join(OUT, "rawboost_golden.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
-    size = os.path.getsize(os.path.join(OUT, "rawboost_golden.npz"))
-    print(f"wrote {len(arrays)} arrays ({size/1e6:.2f} MB) and {len(meta['cases'])+len(meta['full'])} case records to {OUT}")
+    size = sum(os.path.getsize(p) for p in paths)
+    print(f"wrote {len(arrays)} arrays ({size/1e6:.2f} MB in {len(paths)} files) and {len(meta['cases'])+len(meta['full'])} case records to {OUT}")
 
 
 def main_multiview():
@@ -341,11 +342,11 @@ def main_round2():
                                             "num_additional_real": 2, "vocoders": vocoders, "stream": stream_digest()}
     meta["getitem"]["ids"] = ids
 
-    np.savez_compressed(os.path.join(OUT, "round2_golden.npz"), **arrays)
+    paths = golden_files.save(OUT, "round2_golden", arrays)
     with open(os.path.join(OUT, "round2_golden.json"), "w") as f:
         json.dump(meta, f, indent=1, sort_keys=True)
-    size = os.path.getsize(os.path.join(OUT, "round2_golden.npz"))
-    print(f"wrote {len(arrays)} round-2 arrays ({size/1e6:.2f} MB) to {OUT}")
+    size = sum(os.path.getsize(p) for p in paths)
+    print(f"wrote {len(arrays)} round-2 arrays ({size/1e6:.2f} MB in {len(paths)} files) to {OUT}")
 
 
 if __name__ == "__main__":

@@ -10,6 +10,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+from oracle import golden_files  # noqa: E402
+
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 
 
@@ -20,7 +22,7 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden():
     """(arrays, meta) produced by oracle/make_golden.py from the unmodified reference."""
-    arrays = np.load(os.path.join(GOLDEN_DIR, "rawboost_golden.npz"))
+    arrays = golden_files.load(GOLDEN_DIR, "rawboost_golden")
     with open(os.path.join(GOLDEN_DIR, "rawboost_golden.json")) as f:
         meta = json.load(f)
     return arrays, meta
@@ -42,7 +44,7 @@ def stream_digest():
 def golden2():
     """Round-2 fixtures (oracle/make_golden.py --round2): inputs above full scale, float64 / zero / NaN inputs, utterances
     longer than 65536 samples, the reverb augmentor and whole Dataset items -- all from the unmodified reference."""
-    arrays = np.load(os.path.join(GOLDEN_DIR, "round2_golden.npz"))
+    arrays = golden_files.load(GOLDEN_DIR, "round2_golden")
     with open(os.path.join(GOLDEN_DIR, "round2_golden.json")) as f:
         meta = json.load(f)
     return arrays, meta

@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 from conftest import GOLDEN_DIR, stream_digest  # noqa: E402
-from oracle import rawboost_oracle as orc  # noqa: E402  (checker only)
+from oracle import golden_files, rawboost_oracle as orc  # noqa: E402  (checker only)
 
 
 @pytest.fixture(scope="module")
@@ -109,7 +109,7 @@ def test_reverb_view_matches_reference_arithmetic(eng, L, K):
 # ---------------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def g2():
-    arrays = np.load(os.path.join(GOLDEN_DIR, "round2_golden.npz"))
+    arrays = golden_files.load(GOLDEN_DIR, "round2_golden")
     with open(os.path.join(GOLDEN_DIR, "round2_golden.json")) as f:
         return arrays, json.load(f)
 

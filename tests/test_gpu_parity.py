@@ -181,7 +181,7 @@ def test_ragged_batch_matches_oracle_and_golden(eng, P, golden):
         assert g.shape == (L,)
         assert max_err(g, w) <= TOL, f"L={L}: {max_err(g, w):.3e}"
         key = f"ragged_algo5_L{L}"
-        if key in arrays.files:
+        if key in arrays:
             assert max_err(g, arrays[key]) <= TOL
 
 
@@ -336,7 +336,7 @@ def test_inputs_above_full_scale_match_reference(eng, golden2):
         assert abs(float(y.astype(np.float64).max()) - s["max"]) <= TOL and abs(float(y.astype(np.float64).min()) - s["min"]) <= TOL, key
         if algo == 2:
             assert sha1_of(y) == s["sha1_f32"], "ISD must be bit-exact on float32 input, also above full scale"
-        if key in arrays.files:
+        if key in arrays:
             assert max_err(y, arrays[key]) <= TOL, key
     for u in (0, 1):
         np.random.seed(orc.seed_for(50 + u))
@@ -459,3 +459,33 @@ def test_rawboost12_offline_cache_branch(eng, tmp_path, monkeypatch):
     np.random.seed(17)
     rb.RawBoost12(x, args, 16000, audio_path="/corpus/bonafide/LA_T_1.wav")
     assert stream_digest() == untouched and after_first != untouched  # the cached call draws nothing
+
+
+def test_bench_dump_outputs_is_the_timed_result_and_repeats(tmp_path):
+    """``bench.py --dump-outputs`` from the command line: the dumped rows are the algo-5 result of the headline batch (checked
+    against the oracle), ``--steps`` is the number of timed steps reported, and two runs with different step counts dump the
+    same arrays."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT
+    from scl_deepfake_audio_detection_b200 import workload
+    B, L = 16, 64600
+    runs = []
+    for steps in (1, 3):
+        out = tmp_path / f"s{steps}"
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3", "--batch", str(B), "--no-e2e",
+               "--no-cpu", "--no-configs", "--dump-outputs", str(out)]
+        res = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps and line["config"]["batch_per_gpu"] == B
+        runs.append((np.load(out / "rows.npy"), np.load(out / "y.npy")))
+    (rows, y), (rows3, y3) = runs
+    assert rows.dtype == np.float64 and rows.tolist() == list(range(B)) and y.dtype == np.float32 and y.shape == (B, L)
+    assert np.array_equal(rows, rows3) and np.array_equal(y, y3)
+    for u in (0, B - 1):
+        np.random.seed(workload.seed_for(u))
+        ref = orc.process(workload.synth_utterance(u, L, bool(u % 2)), 16000, ARGS, 5)
+        assert max_err(y[u], ref) <= TOL, u

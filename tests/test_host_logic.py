@@ -353,12 +353,22 @@ def test_header_is_plain_c(tmp_path):
 
 
 # -----------------------------------------------------------------------------------------------------------------------------
-# the compiled FIR-bank kernel keeps its shape: packed FFMA2 body loop, no spills, 4 CTAs per SM worth of registers
-def test_fir_kernel_sass_contract():
+@pytest.fixture
+def cuobjdump_on_path(monkeypatch):
+    """The toolkit's cuobjdump on PATH: found there or where csrc/build.sh takes it from, next to $NVCC (default
+    /usr/local/cuda/bin/nvcc), so that a shell without the toolkit on PATH still runs the SASS checks against the built library."""
     import shutil
     from scl_deepfake_audio_detection_b200 import _lib
+    nvcc = shutil.which(os.environ.get("NVCC") or "/usr/local/cuda/bin/nvcc")
+    if shutil.which("cuobjdump") is None and nvcc and os.access(os.path.join(os.path.dirname(nvcc), "cuobjdump"), os.X_OK):
+        monkeypatch.setenv("PATH", os.path.dirname(nvcc) + os.pathsep + os.environ.get("PATH", ""))
     if shutil.which("cuobjdump") is None or not os.path.exists(_lib.LIB_PATH):
         pytest.skip("cuobjdump or the built library is not available")
+
+
+# the compiled FIR-bank kernel keeps its shape: packed FFMA2 body loop, no spills, 4 CTAs per SM worth of registers
+def test_fir_kernel_sass_contract(cuobjdump_on_path):
+    from scl_deepfake_audio_detection_b200 import _lib
     sys.path.insert(0, os.path.join(ROOT, "scripts"))
     import sass_loop_stats
     loops, reuse = {}, {}
@@ -392,14 +402,11 @@ def test_fir_kernel_sass_contract():
         assert regs and max(regs) <= 128, f"more than 128 registers: fewer than 4 CTAs of 128 threads per SM ({regs})"
 
 
-def test_sass_reuse_patch_is_idempotent_and_touches_control_bits_only(tmp_path):
+def test_sass_reuse_patch_is_idempotent_and_touches_control_bits_only(tmp_path, cuobjdump_on_path):
     """csrc/sass_reuse_patch.py on the (already patched) built library changes nothing; and against a library linked without it
     (when one can be produced here) it differs only in bits 45 and 58 of FFMA2 control words."""
-    import shutil
     import subprocess
     from scl_deepfake_audio_detection_b200 import _lib
-    if shutil.which("cuobjdump") is None or not os.path.exists(_lib.LIB_PATH):
-        pytest.skip("cuobjdump or the built library is not available")
     script = os.path.join(os.path.dirname(_lib.LIB_PATH), "..", "csrc", "sass_reuse_patch.py")
     out = tmp_path / "again.so"
     subprocess.run([sys.executable, script, _lib.LIB_PATH, str(out)], check=True, capture_output=True)
@@ -466,14 +473,11 @@ def test_sass_reuse_patch_rule_on_a_synthetic_stream():
     assert all(blob[16 * i:16 * i + 8] == (lo + i).to_bytes(8, "little") for i in range(len(text))), "the low words must not change"
 
 
-def test_fp32_peak_probe_uses_the_uniform_register_form():
+def test_fp32_peak_probe_uses_the_uniform_register_form(cuobjdump_on_path):
     """The roofline denominator of the FIR kernels is measured by rb_probe_fp32; its FFMA2 chain must be the fast form
     (multiplier in a uniform register), or the peak -- and with it every reported fraction -- would be off by 2 %."""
-    import shutil
     import subprocess
     from scl_deepfake_audio_detection_b200 import _lib
-    if shutil.which("cuobjdump") is None or not os.path.exists(_lib.LIB_PATH):
-        pytest.skip("cuobjdump or the built library is not available")
     sass = subprocess.run(["cuobjdump", "-sass", "-fun", "fp32_probe_kernel", _lib.LIB_PATH], capture_output=True, text=True).stdout
     if "FFMA2" not in sass:  # older cuobjdump: no -fun filter on mangled substrings
         sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
@@ -529,3 +533,28 @@ def test_native_planner_rejects_bad_arguments_instead_of_throwing():
     from scl_deepfake_audio_detection_b200 import plans
     want_idx, _ = plans.draw_isd(1000, 400)
     assert np.array_equal(got.isd_idx, want_idx.astype(np.int32))
+
+
+def test_bench_dump_outputs_every_row_or_a_fixed_sample_under_64_mb(tmp_path):
+    """``bench.py --dump-outputs``: a small result is written whole; of a 4096 x 64600 one the same seeded rows on every call,
+    float32 results and float64 row numbers, under 64 MB; of rows longer than the budget one row's head."""
+    import torch
+    import bench
+    y = torch.arange(3 * 40, dtype=torch.float32).reshape(3, 40)
+    bench.dump_outputs(str(tmp_path / "small"), y, 3, 37)
+    assert np.array_equal(np.load(tmp_path / "small" / "y.npy"), y[:, :37].numpy())
+    assert np.load(tmp_path / "small" / "rows.npy").tolist() == [0.0, 1.0, 2.0]
+    B, L = 4096, 64600
+    y = torch.arange(B, dtype=torch.float32)[:, None].expand(B, L + 4)  # row u holds u
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), y, B, L)
+    rows, out = np.load(tmp_path / "a" / "rows.npy"), np.load(tmp_path / "a" / "y.npy")
+    assert rows.dtype == np.float64 and out.dtype == np.float32 and out.shape == (rows.shape[0], L)
+    assert 100 < rows.shape[0] < B and np.all(np.diff(rows) > 0) and np.array_equal(out[:, 0], rows) and np.all(out == out[:, :1])
+    assert np.array_equal(np.load(tmp_path / "b" / "rows.npy"), rows)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in ("y.npy", "rows.npy")) <= 64 * 2 ** 20
+    y = torch.ones(1, 1).expand(2, 20_000_000)  # one row alone is larger than the budget: its head, not an empty file
+    bench.dump_outputs(str(tmp_path / "long"), y, 2, 20_000_000)
+    out = np.load(tmp_path / "long" / "y.npy", mmap_mode="r")
+    assert out.shape == (1, bench.DUMP_BYTES // 4) and float(out[0, -1]) == 1.0
+    assert os.path.getsize(tmp_path / "long" / "y.npy") <= 64 * 2 ** 20

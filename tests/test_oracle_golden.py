@@ -209,7 +209,7 @@ def test_oracle_inputs_above_full_scale(golden2):
         assert stream_digest() == s["stream"], key
         if algo == 2:
             assert y.dtype == np.float32 and sha1_of(y) == s["sha1_f32"]
-        if key in arrays.files:
+        if key in arrays:
             assert np.max(np.abs(y.astype(np.float64) - arrays[key])) <= 1e-6, key
     for u in (0, 1):
         np.random.seed(orc.seed_for(50 + u))
@@ -290,19 +290,41 @@ def test_oracle_dataset_item_matches_reference(golden2):
         assert stream_digest() == m["stream"]
 
 
-def test_compiled_reference_matches_the_oracle():
-    """``oracle/_ref`` (the reference's own bytecode, oracle/build_ref.py) and the numpy restatement agree on every algo (bit for bit where no filter runs, within TOL where
-    float64 FIR sums are ordered differently), and consume the global stream identically -- the CPU arm of the bench times the former, the tests check with the latter."""
-    from oracle import build_ref
-    if not build_ref.available():
-        build_ref.build()  # possible only where /root/reference exists
-    ref = build_ref.load()
-    if ref is None:
-        pytest.skip(f"oracle/_ref not usable here: {build_ref.last_error}")
-    ops, dispatch = ref
+def _same_as_reference(a, stream_a, b, algo):
+    """Result ``b`` (and the stream state after it) of the numpy restatement against the reference's ``a``: bit for bit where no
+    filter runs, within TOL where float64 FIR sums are ordered differently (<= 1 ulp of the peak, measured 2.2e-16)."""
+    assert stream_digest() == stream_a, algo
+    assert np.asarray(a).dtype == np.asarray(b).dtype, algo
+    if algo in (0, 2):
+        assert np.array_equal(a, b), algo
+    else:
+        np.testing.assert_allclose(a, b, rtol=0, atol=TOL, err_msg=str(algo))
+
+
+def test_compiled_reference_matches_the_oracle(golden):
+    """The reference's own code and the numpy restatement agree on every algo, quiet and loud, and consume the global stream
+    identically; normWav too. On every checkout against the reference's outputs stored in tests/golden (oracle/make_golden.py);
+    where ``oracle/_ref`` (the reference's bytecode, oracle/build_ref.py, which the CPU arm of the bench times) can be built,
+    also against the live reference on further inputs."""
     import warnings
+    arrays, meta = golden
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
+        for algo in range(0, 9):
+            for loud in (0, 1):
+                for u in (0, 1):
+                    key = f"algo{algo}_loud{loud}_u{u}"
+                    x = orc.synth_utterance(u, meta["cases"][key]["L"], bool(loud))
+                    np.random.seed(orc.seed_for(u))
+                    _same_as_reference(arrays[key], meta["cases"][key]["stream"], orc.process(x, 16000, ARGS, algo), algo)
+        assert np.array_equal(arrays["norm_y0_loud"], orc.norm_wav(arrays["norm_x_loud"], 0))
+        from oracle import build_ref
+        if not build_ref.available():
+            build_ref.build()  # needs the reference's sources
+        ref = build_ref.load()
+        if ref is None:
+            return
+        ops, dispatch = ref
         for algo in range(0, 9):
             for loud in (False, True):
                 x = orc.synth_utterance(3, 8000, loud)
@@ -310,13 +332,7 @@ def test_compiled_reference_matches_the_oracle():
                 a = dispatch(x, 16000, ARGS, algo)
                 sa = stream_digest()
                 np.random.seed(77)
-                b = orc.process(x, 16000, ARGS, algo)
-                assert stream_digest() == sa, algo
-                assert np.asarray(a).dtype == np.asarray(b).dtype, algo
-                if algo in (0, 2):
-                    assert np.array_equal(a, b), algo  # no filtering: identical down to the bit
-                else:  # float64 FIR sums differ by summation order only (<= 1 ulp of the peak, measured 2.2e-16)
-                    np.testing.assert_allclose(a, b, rtol=0, atol=TOL, err_msg=str(algo))
+                _same_as_reference(a, sa, orc.process(x, 16000, ARGS, algo), algo)
         x = orc.synth_utterance(4, 5000, True)
         assert np.array_equal(ops.normWav(x * 3, 0), orc.norm_wav(x * 3, 0))
 
