@@ -219,6 +219,23 @@ RB_API int rb_multiview_assemble_ex(const float* views, const float* views_b, co
                                     int V, int ld, const int32_t* start, int length, int repeat_pad, int layout, float* out,
                                     int32_t* out_len, const float* view_label, float* labels, void* stream);
 
+/* ---- reverb view, batched  (SURVEY.md 8f-4; audio_augmentor/reverb.py:39-42) -------------------------------------------
+ * y_u = normWav(np.convolve(x_u, h_u), 1): the full convolution of each waveform with its room impulse response, peak-normalised.
+ * x [B, ld] float32 and len[B] (device); impulse responses as CSR like rb_filter_fir: rir float32[rir_off[B]], rir_off int32[B+1]
+ * (device), any K_u = rir_off[u+1] - rir_off[u]. y [B, ld_out] float32 (device), ld_out % 4 == 0, x != y. out_len int32[B]
+ * (device) receives len[u] + K_u - 1, or 0 for an empty row (len[u] == 0). A row with K_u < 1, len[u] < 0, len[u] > ld,
+ * len[u] + K_u - 1 > ld_out, or more taps than the workspace was sized for gets out_len[u] = -1 and is not written. Nothing is
+ * ever written outside [0, out_len[u]) of a row. Peak normalisation as numpy: an all-zero result is NaN, and NaN propagates.
+ * Uniformly partitioned FFT overlap-save (partitions of 8192 taps, 16384-point real FFTs; DESIGN.md 4.5): the cost per
+ * output sample grows with the number of partitions, not with every tap. Float32 throughout; max-abs error against a float64
+ * np.convolve is ~3e-7 after the normalisation.
+ * rb_reverb_workspace_bytes(B, max_taps): device workspace (256-byte aligned) for B rows of at most max_taps taps each.
+ * rb_reverb takes the partitions per row from workspace_bytes (one spectrum launch per row and partition), so pass the size
+ * this function returned rather than that of a larger buffer. */
+RB_API size_t rb_reverb_workspace_bytes(int B, int max_taps);
+RB_API int rb_reverb(const float* x, const int32_t* len, int B, int ld, const float* rir, const int32_t* rir_off, float* y,
+                     int ld_out, int32_t* out_len, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Streaming form of rb_process_host_seeded: queues the whole call and returns at once; *ticket identifies it. Up to two calls
  * may be in flight (a third submit first waits for the oldest), so the copies of consecutive batches follow each other
  * without a gap and steady-state throughput is bound by PCIe alone. x, len, seeds and y must stay valid -- and y must not

@@ -20,7 +20,7 @@ SYMBOLS = (
     "rb_probe_fp32", "rb_launch_count", "rb_profile_enable", "rb_profile_read", "rb_planner_create", "rb_planner_destroy",
     "rb_planner_draw", "rb_devplan_bytes", "rb_devplan_draw", "rb_process_host_seeded",
     "rb_ctx_set_chunk", "rb_ctx_set_plan_mode", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
-    "rb_multiview_assemble_ex", "rb_submit_seeded_ex",
+    "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
 )
 RB_IO_HOST_F32, RB_IO_HOST_PCM16, RB_IO_DEVICE_F32 = 0, 1, 2
 
@@ -135,6 +135,10 @@ def load() -> C.CDLL:
     lib.rb_multiview_assemble_ex.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, i32, i32, i32, vp, vp, vp, vp, vp]
     lib.rb_submit_seeded_ex.restype = i32
     lib.rb_submit_seeded_ex.argtypes = [vp, i32, C.POINTER(RbArgs), vp, i32, vp, vp, i32, i32, vp, i32, vp, i32, C.POINTER(C.c_uint64)]
+    lib.rb_reverb_workspace_bytes.restype = sz
+    lib.rb_reverb_workspace_bytes.argtypes = [i32, i32]
+    lib.rb_reverb.restype = i32
+    lib.rb_reverb.argtypes = [vp, vp, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp]
     lib.rb_submit_host_seeded.restype = i32
     lib.rb_submit_host_seeded.argtypes = [vp, i32, C.POINTER(RbArgs), vp, vp, vp, i32, i32, vp, C.POINTER(C.c_uint64)]
     lib.rb_ctx_wait.restype = i32

@@ -48,8 +48,10 @@ class Engine:
     # -- memory ---------------------------------------------------------------------------------------
     def workspace(self, B: int, ld: int, algo: int = 8) -> torch.Tensor:
         """Growable device workspace, sized for what ``algo`` needs (algo 8 needs the most)."""
-        need = int(self.lib.rb_workspace_bytes_for(int(algo), B, ld))
-        if self._ws is None or self._ws.numel() < need:
+        return self._scratch(int(self.lib.rb_workspace_bytes_for(int(algo), B, ld)))
+
+    def _scratch(self, need: int) -> torch.Tensor:
+        if self._ws is None or self._ws.numel() < need + 256:
             self._ws = None
             self._ws = torch.empty(need + 256, dtype=torch.uint8, device=self.device)
         return self._ws
@@ -176,6 +178,60 @@ class Engine:
                                      ws.numel() - 256, C.c_void_p(stream))
         _lib.check(rc, "rb_normwav")
         return out
+
+    def reverb(self, x: torch.Tensor, lengths: torch.Tensor, rir: torch.Tensor, rir_off: torch.Tensor,
+               out: Optional[torch.Tensor] = None, ld_out: Optional[int] = None, max_taps: Optional[int] = None):
+        """Reverb view of every row (``rb_reverb``): ``normWav(np.convolve(x_u, h_u), 1)`` with h_u = ``rir[rir_off[u]:rir_off[u+1]]``.
+        All tensors live on the engine's device: x [B, ld] float32, lengths / rir_off int32, rir float32. Returns
+        (y [B, ld_out] float32, out_len int32 [B]) with out_len[u] = lengths[u] + K_u - 1 (0 for an empty row, -1 for a row that
+        was not computed: K_u < 1, or an output longer than ld_out); samples of y beyond out_len[u] are untouched.
+
+        The row stride of the result is ``out.shape[1]`` when ``out`` is given, else ``ld_out``. With neither, it is sized from
+        the lengths and offsets, which this READS BACK to the host; the call then also waits for the result and raises
+        ``ValueError`` if any row was not computed. Otherwise it is asynchronous on torch's current stream, with no host
+        synchronisation, and the caller inspects ``out_len``.
+
+        ``max_taps`` (the longest impulse response, when the caller knows it) sizes the workspace and the spectrum grid
+        without a read-back: one 64 KB spectrum per row and 8192 taps. Without it the asynchronous form sizes for the longest
+        impulse response the output stride allows. A row with more taps than the workspace then holds (``max_taps`` rounded up to
+        whole 8192-tap partitions) is not computed (out_len -1)."""
+        self._check_batch(x, lengths)
+        B, ld = x.shape
+        if rir.device != self.device or rir_off.device != self.device:
+            raise ValueError(f"tensors must live on {self.device}")
+        if rir.dtype != torch.float32 or not rir.is_contiguous() or rir_off.dtype != torch.int32 or rir_off.numel() != B + 1:
+            raise ValueError("rir must be a contiguous float32 tensor and rir_off int32 [B + 1]")
+        if out is not None:
+            if out.device != self.device or out.dtype != torch.float32 or out.dim() != 2 or out.shape[0] != B or not out.is_contiguous():
+                raise ValueError("out must be a contiguous [B, ld_out] float32 tensor on the engine's device")
+            if ld_out is not None and int(ld_out) != out.shape[1]:
+                raise ValueError(f"ld_out={ld_out} but out has {out.shape[1]} columns")
+            ld_out = out.shape[1]
+        read_back = ld_out is None
+        if read_back:
+            n = lengths.cpu().numpy().astype(np.int64)
+            k = np.diff(rir_off.cpu().numpy().astype(np.int64))
+            max_taps = int(k.max()) if B else 1
+            ld_out = padded_ld(int(np.max(np.where((n > 0) & (k > 0), n + k - 1, 0))) if B else 0)
+        elif max_taps is None:
+            # a computed row never has more taps than output samples; rir.numel() bounds every row as well
+            max_taps = max(1, min(int(ld_out), rir.numel()))
+        if out is None:
+            out = torch.zeros((B, int(ld_out)), dtype=torch.float32, device=self.device)
+        out_len = torch.empty(B, dtype=torch.int32, device=self.device)
+        need = int(self.lib.rb_reverb_workspace_bytes(B, int(max_taps)))
+        ws = self._scratch(need)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_reverb(_ptr(x), _ptr(lengths), B, ld, _ptr(rir), _ptr(rir_off), _ptr(out), int(ld_out), _ptr(out_len),
+                                    C.c_void_p(self._ws_ptr(ws)), need, C.c_void_p(stream))  # exactly `need`: sets the partitions
+        _lib.check(rc, "rb_reverb")
+        if read_back:
+            bad = np.flatnonzero(out_len.cpu().numpy() < 0)
+            if bad.size:
+                raise ValueError(f"rb_reverb did not compute rows {bad.tolist()[:8]}: every impulse response needs at least one "
+                                 f"tap and every length must lie in [0, {ld}]")
+        return out, out_len
 
     def _check_batch(self, x: torch.Tensor, lengths: torch.Tensor) -> None:
         if x.device != self.device or lengths.device != self.device:

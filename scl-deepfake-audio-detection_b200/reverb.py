@@ -1,7 +1,11 @@
 """Reverb view on the device (SURVEY.md 8f-4): the arithmetic of ``ReverbAugmentor.transform``
 (``/root/reference/datautils/audio_augmentor/reverb.py:33-44``) -- a full convolution of the waveform with a room impulse
-response followed by peak normalisation -- on the FIR-bank kernel (long filters run as 512-tap segments) and the one-kernel
-``normWav``.
+response followed by peak normalisation. Two device paths:
+
+* ``reverb_batch`` / ``reverb_convolve`` (host waveforms): the FIR-bank kernel (long filters run as 512-tap segments) and the
+  one-kernel ``normWav``;
+* ``reverb_device`` / ``Engine.reverb`` (waveforms already on the device, C entry ``rb_reverb``): FFT overlap-save with
+  8192-tap partitions, whose cost grows with the number of partitions rather than with every tap (DESIGN.md 4.5).
 
     reverberate = np.convolve(data, rir_data)            # length len(data) + len(rir) - 1
     reverberate /= np.max(np.abs(reverberate))
@@ -37,13 +41,36 @@ def reverb_batch(eng: Engine, waves: Sequence[np.ndarray], rirs: Sequence[np.nda
     for u, (w, s) in enumerate(zip(waves, shift)):
         host[u, s:s + w.shape[0]] = np.asarray(w, dtype=np.float32)
     x = torch.from_numpy(host).to(eng.device)
-    taps = torch.from_numpy(np.concatenate(rirs) if B else np.zeros(0, np.float32)).to(eng.device)
-    off = torch.from_numpy(np.concatenate([[0], np.cumsum([r.shape[0] for r in rirs])]).astype(np.int32)).to(eng.device)
+    taps, off = pack_rirs(eng, rirs)
     # the kernel takes one length per row for both input and output: run over the delayed input's length; the outputs beyond
     # len + K - 1 are exact zeros (no tap reaches a sample there), so they do not disturb the peak
     ln_in = torch.from_numpy(in_len).to(eng.device)
     y = eng.filter_fir(x, ln_in, taps, off)
     return eng.normwav(y, ln_in, True), torch.from_numpy(out_len).to(eng.device)
+
+
+def pack_rirs(eng: Engine, rirs: Sequence[np.ndarray]):
+    """Host impulse responses -> (float32 taps, int32 CSR offsets [B + 1]) on the engine's device."""
+    rirs = [np.asarray(r, dtype=np.float32).reshape(-1) for r in rirs]
+    taps = np.concatenate(rirs) if rirs else np.zeros(0, np.float32)
+    off = np.concatenate([[0], np.cumsum([r.shape[0] for r in rirs])]).astype(np.int32)
+    return torch.from_numpy(taps).to(eng.device), torch.from_numpy(off).to(eng.device)
+
+
+def reverb_device(eng: Engine, x: torch.Tensor, lengths: torch.Tensor, rirs: Sequence[np.ndarray], ld_out=None):
+    """Reverb views of waveforms that already live on the device: x [B, ld] float32 and int32 lengths on ``eng.device``, one
+    host impulse response per row (as the caller loads them from the RIR corpus). Returns ([B, ld_out] float32 device tensor,
+    int32 device lengths len + K - 1). FFT overlap-save on the device (``Engine.reverb``); raises ``ValueError`` if a row could
+    not be computed (an empty impulse response, or ``ld_out`` too small for its result)."""
+    if len(rirs) != x.shape[0]:
+        raise ValueError("one impulse response per waveform")
+    taps, off = pack_rirs(eng, rirs)
+    y, out_len = eng.reverb(x, lengths, taps, off, ld_out=ld_out, max_taps=max((len(r) for r in rirs), default=1))
+    if ld_out is not None:
+        bad = np.flatnonzero(out_len.cpu().numpy() < 0)
+        if bad.size:
+            raise ValueError(f"rows {bad.tolist()[:8]} were not computed: empty impulse response or ld_out={ld_out} too small")
+    return y, out_len
 
 
 def reverb_convolve(data, rir_data) -> np.ndarray:
