@@ -236,6 +236,36 @@ RB_API size_t rb_reverb_workspace_bytes(int B, int max_taps);
 RB_API int rb_reverb(const float* x, const int32_t* len, int B, int ld, const float* rir, const int32_t* rir_off, float* y,
                      int ld_out, int32_t* out_len, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- whole items, each seeded on its own  (Dataset_for.__getitem__, asvspoof_2019_augall_3.py:103-146) ------------------
+ * np.random.seed(seeds[g]) precedes item g, as in a loader that seeds every __getitem__; items are independent and are drawn in
+ * parallel. Item g of index idx = indices[g] consumes its stream in the loader's order: RawBoost (algo 5) on each of the nvoc
+ * vocoded copies in vocoder order, then on the anchor; np.random.choice(others, n_add, replace=False), i.e. permutation(N-1)[:n_add]
+ * mapped through others = [0, N) without idx (consumed even when n_add == 0); then int(rand() * (L_anchor - trim)), drawn only
+ * when L_anchor >= trim. The crop is batch_pad_for_multiview's with random_trim_nosil set.
+ * Corpus (device): rows [R, ld] float32, R = N * (1 + nvoc), ld % 4 == 0, 16-byte aligned, lengths corpus_len[R] >= 1. Row idx is
+ * bona fide utterance idx, row N + idx*nvoc + v is vocoder v's copy of it. indices (int32[G], each in [0, N)) and seeds
+ * (uint32[G]) are device arrays. Batch rows, as multiview.ItemBatcher lays them out: rows g*(nvoc+1) + v are item g's vocoded
+ * copies (v < nvoc) and its anchor (v = nvoc), the RawBoost inputs; rows G*(nvoc+1) + g*n_add + k its additional bona fide
+ * utterances. Integer draws (tap counts, impulse positions, extra utterances, crop starts) and the float64 impulse gains equal
+ * numpy's bit for bit; taps agree to 1 ulp.
+ * rb_items_workspace_bytes: device workspace (256-byte aligned) of rb_items_run, which holds the gathered batch
+ * [G*(nvoc+1+n_add), ld] and its RawBoost results [G*(nvoc+1), ld]; it is more than rb_items_draw needs. 0 for invalid shapes.
+ * rb_items_draw: the plan of the G*(nvoc+1) RawBoost utterances (*plan, a HOST struct, receives device pointers into the
+ * workspace), src_row / row_len (int32[G*(nvoc+1+n_add)]: each batch row's corpus row and its length), start (int32[G]: crop
+ * starts, 0 where none is drawn) and, when end_state is not NULL, each item's stream state after its last draw (uint32[G][625]:
+ * numpy's key[624] and pos, pos in 0..623).
+ * rb_items_run: draw, gather, rb_process(5) and rb_multiview_assemble_ex in one call: out [G][trim][V] (layout 0) or
+ * [G][V][trim] (layout 1), V = 2 + n_add + 2*nvoc in the Dataset's view order (anchor, augmented anchor, additional, vocoded,
+ * augmented vocoded), out_len (nullable, int32[G]) and labels (nullable, float[G][V]: 1 for the anchor and its positives, 0 for
+ * the vocoded views). repeat_pad as batch_pad_for_multiview. */
+RB_API size_t rb_items_workspace_bytes(const rb_args* args, int G, int nvoc, int n_add, int N, int ld);
+RB_API int rb_items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
+                         const int32_t* indices, const uint32_t* seeds, int32_t* src_row, int32_t* row_len, int32_t* start,
+                         uint32_t* end_state, void* workspace, size_t workspace_bytes, rb_plan* plan, void* stream);
+RB_API int rb_items_run(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
+                        const float* corpus, const int32_t* corpus_len, const int32_t* indices, const uint32_t* seeds, float* out,
+                        int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Streaming form of rb_process_host_seeded: queues the whole call and returns at once; *ticket identifies it. Up to two calls
  * may be in flight (a third submit first waits for the oldest), so the copies of consecutive batches follow each other
  * without a gap and steady-state throughput is bound by PCIe alone. x, len, seeds and y must stay valid -- and y must not

@@ -11,7 +11,7 @@ NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
 FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden
        -Xptxas -v -I"$root/include" -I"$here" ${RB_EXTRA_FLAGS:-})
 objs=()
-for src in rb_fir_bank rb_dense rb_api rb_probe rb_devplan rb_multiview rb_reverb; do
+for src in rb_fir_bank rb_dense rb_api rb_probe rb_devplan rb_multiview rb_reverb rb_items; do
   extra=()
   # the FP32 peak probe wants its multiplier in a uniform register (FFMA2 R, R, UR, R: two register-file operands instead of
   # three); ptxas does that at the lower register-usage levels only (rb_probe.cu)

@@ -120,13 +120,19 @@ int launch_fir_bank(const float* x, const int32_t* len, int B, int ld, const flo
                     const uint32_t* mask /*nullable*/, int mask_ld, const FirTail& tail, cudaStream_t st);
 
 // Device-side planner, stage by stage (rb_devplan.cu); rb_devplan_draw runs all four for the whole batch. The pipelined host
-// entry interleaves stages 2/3 of one chunk with the kernels of the previous chunk.
+// entry interleaves stages 2/3 of one chunk with the kernels of the previous chunk. With `snaps` (device, [B][625] words in
+// numpy's state form, rb_mt.cuh) utterance u's stream starts at snaps[u] instead of np.random.seed(seeds[u]).
 int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds, void* storage,
-                  size_t storage_bytes, rb_plan* plan, cudaStream_t st);
+                  size_t storage_bytes, rb_plan* plan, cudaStream_t st, const uint32_t* snaps = nullptr);
 int devplan_body(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds, void* storage, int first,
-                 int count, cudaStream_t st);
+                 int count, cudaStream_t st, const uint32_t* snaps = nullptr);
 int devplan_apply(const rb_args* args, int algo, int B, int ld, const int32_t* len, void* storage, int first, int count,
                   cudaStream_t st);
 int devplan_end(const rb_args* args, int algo, int B, int ld, void* storage, cudaStream_t st);
+// np.random.permutation(len[u])[:off[u+1]-off[u]] -> out[off[u]...] for B rows of at most ld entries whose streams start at
+// snaps[u]; `storage` holds shuffle_prefix_bytes(B, ld) bytes, 256-byte aligned.
+size_t shuffle_prefix_bytes(int B, int ld);
+int shuffle_prefix(int B, int ld, const int32_t* len, const uint32_t* snaps, const int32_t* off, int32_t* out, void* storage,
+                   cudaStream_t st);
 
 }  // namespace rb

@@ -32,141 +32,13 @@
 #include <string.h>
 
 #include "rb_common.cuh"
+#include "rb_mt.cuh"
 
 namespace rb {
 
 namespace {
 
-constexpr int kMtN = 624, kMtM = 397;
 constexpr int kNarrowMax = 65536;  // longest row whose permutation is held as uint16 in shared memory
-constexpr uint32_t kFull = 0xffffffffu;
-
-// ---- MT19937, one warp per stream, state and two tempered blocks in shared memory ------------------------------------
-struct MtSmem {
-  uint32_t key[kMtN];
-  uint32_t blk[2][kMtN];
-};
-
-__device__ __forceinline__ uint32_t mt_twist(uint32_t a, uint32_t b, uint32_t far) {
-  const uint32_t y = (a & 0x80000000u) | (b & 0x7fffffffu);
-  return far ^ (y >> 1) ^ ((0u - (y & 1u)) & 0x9908b0dfu);
-}
-
-__device__ __forceinline__ uint32_t mt_temper(uint32_t y) {
-  y ^= (y >> 11);
-  y ^= (y << 7) & 0x9d2c5680u;
-  y ^= (y << 15) & 0xefc60000u;
-  y ^= (y >> 18);
-  return y;
-}
-
-// Advance the state by one block (624 words) and temper it into `out`. Warp-cooperative, three dependency phases.
-__device__ void mt_next_block(uint32_t* key, uint32_t* out, int lane) {
-  uint32_t v[8];
-  // phase 1: i in [0, 227) reads old key[i], key[i+1], key[i+397]
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int i = c * 32 + lane;
-    if (i < kMtN - kMtM) v[c] = mt_twist(key[i], key[i + 1], key[i + kMtM]);
-  }
-  __syncwarp();
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int i = c * 32 + lane;
-    if (i < kMtN - kMtM) key[i] = v[c];
-  }
-  __syncwarp();
-  // phase 2: i in [227, 454) reads new key[i-227], old key[i], key[i+1]
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int i = (kMtN - kMtM) + c * 32 + lane;
-    if (i < 2 * (kMtN - kMtM)) v[c] = mt_twist(key[i], key[i + 1], key[i - (kMtN - kMtM)]);
-  }
-  __syncwarp();
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const int i = (kMtN - kMtM) + c * 32 + lane;
-    if (i < 2 * (kMtN - kMtM)) key[i] = v[c];
-  }
-  __syncwarp();
-  // phase 3: i in [454, 623) reads new key[i-227], old key[i], key[i+1]
-#pragma unroll
-  for (int c = 0; c < 6; ++c) {
-    const int i = 2 * (kMtN - kMtM) + c * 32 + lane;
-    if (i < kMtN - 1) v[c] = mt_twist(key[i], key[i + 1], key[i - (kMtN - kMtM)]);
-  }
-  __syncwarp();
-#pragma unroll
-  for (int c = 0; c < 6; ++c) {
-    const int i = 2 * (kMtN - kMtM) + c * 32 + lane;
-    if (i < kMtN - 1) key[i] = v[c];
-  }
-  __syncwarp();
-  if (lane == 0) key[kMtN - 1] = mt_twist(key[kMtN - 1], key[0], key[kMtM - 1]);
-  __syncwarp();
-#pragma unroll
-  for (int c = 0; c < 20; ++c) {
-    const int i = c * 32 + lane;
-    if (i < kMtN) out[i] = mt_temper(key[i]);
-  }
-  __syncwarp();
-}
-
-// The stream as the warp sees it: the current and the next block are always tempered, so any window of up to 624 words
-// starting at the read position can be addressed without synchronisation.
-struct MtStream {
-  MtSmem* sm;
-  int cur;  // which blk[] holds the current block
-  int pos;  // read position inside it, 0..623
-
-  __device__ void seed(uint32_t s, int lane) {
-    if (lane == 0) {
-      for (int i = 0; i < kMtN; ++i) {
-        sm->key[i] = s;
-        s = 1812433253u * (s ^ (s >> 30)) + (uint32_t)i + 1u;
-      }
-    }
-    __syncwarp();
-    mt_next_block(sm->key, sm->blk[0], lane);
-    mt_next_block(sm->key, sm->blk[1], lane);
-    cur = 0;
-    pos = 0;
-  }
-  // word k (0 <= k < 624) after the read position
-  __device__ __forceinline__ uint32_t word(int k) const {
-    const int idx = pos + k;
-    return idx < kMtN ? sm->blk[cur][idx] : sm->blk[cur ^ 1][idx - kMtN];
-  }
-  // consume n <= 624 words
-  __device__ __forceinline__ void advance(int n, int lane) {
-    pos += n;
-    if (pos >= kMtN) {
-      pos -= kMtN;
-      __syncwarp();
-      mt_next_block(sm->key, sm->blk[cur], lane);  // the exhausted block becomes the one after next
-      cur ^= 1;
-    }
-  }
-  __device__ void skip(int n, int lane) {
-    while (n > 0) {
-      const int s = n < kMtN ? n : kMtN;
-      advance(s, lane);
-      n -= s;
-    }
-  }
-};
-
-// numpy legacy rk_double from two stream words
-__device__ __forceinline__ double mt_double(uint32_t wa, uint32_t wb) {
-  const int32_t a = (int32_t)(wa >> 5), b = (int32_t)(wb >> 6);
-  return __ddiv_rn(__dadd_rn(__dmul_rn((double)a, 67108864.0), (double)b), 9007199254740992.0);
-}
-// np.random.uniform(low, high): low + (high - low) * double, two roundings (no FMA contraction)
-__device__ __forceinline__ double mt_uniform(double lo, double hi, double d) { return __dadd_rn(lo, __dmul_rn(__dsub_rn(hi, lo), d)); }
-
-// ---- per-filter design parameters written by the head / body kernels, read by design_kernel ----------------------------
-// layout per filter: [f1, f2, c] x nBands, then G  -> 3*nBands + 1 doubles
-__device__ __forceinline__ int filter_stride(int nBands) { return 3 * nBands + 1; }
 
 // Draw one genNotchCoeffs parameter set (RawBoost.py:31-45) from stream words [w0, w0 + 2*(3*nBands+1)): returns K.
 __device__ int draw_filter_params(const MtStream& s, int w0, const rb_args& a, double minG, double maxG, double* out) {
@@ -198,14 +70,15 @@ constexpr int kHeadWarps = 4;
 
 __global__ void __launch_bounds__(32 * kHeadWarps)
 plan_head_kernel(rb_args a, int algo, int B, const int32_t* __restrict__ len_arr, const uint32_t* __restrict__ seeds,
-                 double* __restrict__ lnl_params, int32_t* __restrict__ lnl_cnt, int32_t* __restrict__ isd_cnt) {
+                 const uint32_t* __restrict__ snaps, double* __restrict__ lnl_params, int32_t* __restrict__ lnl_cnt, int32_t* __restrict__ isd_cnt) {
   __shared__ MtSmem sm[kHeadWarps];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int u = blockIdx.x * kHeadWarps + warp;
   if (u >= B) return;
   MtStream s;
   s.sm = &sm[warp];
-  s.seed(seeds[u], lane);
+  if (snaps) s.load(snaps + (size_t)u * kMtSnapWords, lane);
+  else s.seed(seeds[u], lane);
   const int per = 2 * filter_stride(a.nBands);  // stream words per filter
   if (uses_lnl(algo)) {
     // filters are consumed in windows that fit the two tempered blocks
@@ -272,10 +145,7 @@ scan_kernel(const int32_t* __restrict__ cnt, int n, int32_t* __restrict__ off) {
 //
 // plan_body_kernel (this one; one warp per utterance, many warps per SM, no permutation array) settles everything that does
 // not depend on the array contents:
-//   1. the swap targets j_i. A round looks at the next 32 stream words; word t is accepted iff
-//      (w_t & mask) <= i - (#accepted before t). The ballot fix-point settles lane t after at most t+1 iterations (lane 0 is
-//      exact at once), in practice after two. Accepted lanes are the consecutive steps i, i-1, ...; their targets go to
-//      jseq[step], step = L-1-i.
+//   1. the swap targets j_i (shuffle_walk_warp, rb_mt.cuh), into jseq[step], step = L-1-i.
 //   2. which consecutive steps may be applied together. Steps are taken in chunks of 32; inside a chunk, step t conflicts
 //      with an earlier step s when they share the target (j_t == j_s) or when s targets t's own slot (j_s == i_t). A set bit
 //      in cuts[chunk] starts a new conflict-free group.
@@ -287,35 +157,9 @@ constexpr int kBodyWarps = 4;  // 30 KB of MT19937 state per CTA: up to 7 CTAs =
 template <typename JT>  // uint16_t for rows of at most 65536 samples, uint32_t beyond
 __device__ void shuffle_scan_warp(MtStream& s, int L, JT* __restrict__ jseq, uint32_t* __restrict__ cuts, uint32_t* dupset,
                                   int lane) {
-  const uint32_t lt = (1u << lane) - 1u;
-  int i = L - 1;
-  while (i >= 1) {
-    uint32_t mask = (uint32_t)i;
-    mask |= mask >> 1;
-    mask |= mask >> 2;
-    mask |= mask >> 4;
-    mask |= mask >> 8;
-    mask |= mask >> 16;
-    const int lo = (int)(mask >> 1) + 1;  // smallest i that uses this mask
-    while (i >= lo) {
-      const int v = (int)(s.word(lane) & mask);
-      uint32_t acc = __ballot_sync(kFull, v <= i);
-      int A;
-      for (;;) {
-        A = __popc(acc & lt);
-        const uint32_t acc2 = __ballot_sync(kFull, v <= i - A);
-        if (acc2 == acc) break;
-        acc = acc2;
-      }
-      const int R = i - lo + 1;                                  // steps left under this mask
-      const uint32_t in_region = __ballot_sync(kFull, A < R);    // a prefix of the lanes: the words this mask consumes
-      const bool valid = ((acc >> lane) & 1u) && (A < R);
-      if (valid) jseq[(L - 1) - (i - A)] = (JT)v;
-      i -= __popc(acc & in_region);
-      s.advance(__popc(in_region), lane);
-    }
-  }
+  shuffle_walk_warp<true>(s, L, jseq, lane);
   __syncwarp();  // jseq was written by other lanes of this warp
+  const uint32_t lt = (1u << lane) - 1u;
   const int nsteps = L - 1;
   // Conflicts are rare (7 % of the chunks) and MATCH.ANY is slow (about a hundred cycles of a per-SM unit each), so every
   // chunk first goes through an exact-negative filter: each step sets the bit of its target in a 4096-bit shared-memory
@@ -371,7 +215,7 @@ __device__ void shuffle_scan_warp(MtStream& s, int L, JT* __restrict__ jseq, uin
 template <typename JT>
 __global__ void __launch_bounds__(32 * kBodyWarps)
 plan_body_kernel(rb_args a, int algo, int B, int ld, int jld, const int32_t* __restrict__ len_arr,
-                 const uint32_t* __restrict__ seeds, const int32_t* __restrict__ isd_off, double* __restrict__ isd_fr, JT* __restrict__ jseq_all,
+                 const uint32_t* __restrict__ seeds, const uint32_t* __restrict__ snaps, const int32_t* __restrict__ isd_off, double* __restrict__ isd_fr, JT* __restrict__ jseq_all,
                  uint32_t* __restrict__ cuts_all, int cuts_ld, float* __restrict__ ssi_noise, double* __restrict__ ssi_params,
                  int32_t* __restrict__ ssi_cnt, float* __restrict__ ssi_snr) {
   __shared__ MtSmem msm[kBodyWarps];
@@ -384,7 +228,8 @@ plan_body_kernel(rb_args a, int algo, int B, int ld, int jld, const int32_t* __r
   const int L = len_arr[u];
   MtStream s;
   s.sm = &msm[warp];
-  s.seed(seeds[u], lane);
+  if (snaps) s.load(snaps + (size_t)u * kMtSnapWords, lane);
+  else s.seed(seeds[u], lane);
   if (uses_lnl(algo)) s.skip(a.N_f * 2 * filter_stride(a.nBands), lane);
   if (uses_isd(algo)) {
     s.advance(2, lane);  // beta (the head kernel turned it into the impulse count)
@@ -434,6 +279,25 @@ plan_body_kernel(rb_args a, int algo, int B, int ld, int jld, const int32_t* __r
       ssi_snr[u] = (float)mt_uniform(a.SNRmin, a.SNRmax, mt_double(s.word(per), s.word(per + 1)));
     }
   }
+}
+
+// The swap targets and groups of a bare permutation whose stream starts at a snapshot (np.random.choice(..., replace=False)
+// of an item, rb_items.cu): one warp per row, as plan_body_kernel.
+template <typename JT>
+__global__ void __launch_bounds__(32 * kBodyWarps)
+shuffle_scan_kernel(int B, int jld, const int32_t* __restrict__ len_arr, const uint32_t* __restrict__ snaps, JT* __restrict__ jseq_all,
+                    uint32_t* __restrict__ cuts_all, int cuts_ld) {
+  __shared__ MtSmem msm[kBodyWarps];
+  __shared__ uint32_t dupset[kBodyWarps][kDupWords];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int u = blockIdx.x * kBodyWarps + warp;
+  if (u >= B) return;
+  for (int w = lane; w < kDupWords; w += 32) dupset[warp][w] = 0u;
+  __syncwarp();
+  MtStream s;
+  s.sm = &msm[warp];
+  s.load(snaps + (size_t)u * kMtSnapWords, lane);
+  shuffle_scan_warp(s, len_arr[u], jseq_all + (size_t)u * jld, cuts_all + (size_t)u * cuts_ld, dupset[warp], lane);
 }
 
 // ---- the swaps themselves: one warp per utterance, permutation in shared memory ------------------------------------------
@@ -755,6 +619,24 @@ design_kernel(int nBands, double fs, int n_filters, const double* __restrict__ p
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// swap targets, group masks and the permutation handed between the phases of perm_apply_kernel, for B rows of at most ld
+struct ShuffleLayout {
+  size_t jseq, cuts, state, bytes;
+  int jld, cuts_ld;
+};
+
+ShuffleLayout shuffle_layout(int B, int ld) {
+  ShuffleLayout l{};
+  l.jld = (int)align_up((size_t)ld, kStageSteps);  // rows padded to whole staging pieces of perm_apply_kernel
+  l.cuts_ld = l.jld / 32;
+  const size_t jbytes = ld > kNarrowMax ? 4 : 2;   // swap targets / permutation entries: uint16 up to 65536 samples, uint32 beyond
+  l.jseq = 0;
+  l.cuts = align_up((size_t)B * l.jld * jbytes, 256);
+  l.state = l.cuts + align_up((size_t)B * l.cuts_ld * 4, 256);
+  l.bytes = l.state + align_up((size_t)B * l.jld * jbytes, 256);
+  return l;
+}
+
 struct DevPlanLayout {
   size_t lnl_params, lnl_cnt, lnl_off, lnl_taps, isd_cnt, isd_off, isd_idx, isd_fr, isd_jseq, isd_cuts, isd_state, ssi_noise, ssi_params,
       ssi_cnt, ssi_off, ssi_taps, ssi_snr, bytes;
@@ -785,12 +667,13 @@ DevPlanLayout layout(const rb_args& a, int algo, int B, int ld) {
   const size_t nmax = isd ? (size_t)B * ((size_t)((double)ld * a.P / 100.0) + 1) : 0;
   l.isd_idx = take(nmax * 4);
   l.isd_fr = take(nmax * 8);
-  l.jld = (int)align_up((size_t)ld, kStageSteps);  // rows padded to whole staging pieces of perm_apply_kernel
-  l.cuts_ld = l.jld / 32;
-  const size_t jbytes = ld > kNarrowMax ? 4 : 2;   // swap targets / permutation entries: uint16 up to 65536 samples, uint32 beyond
-  l.isd_jseq = take(isd ? (size_t)B * l.jld * jbytes : 0);
-  l.isd_cuts = take(isd ? (size_t)B * l.cuts_ld * 4 : 0);
-  l.isd_state = take(isd ? (size_t)B * l.jld * jbytes : 0);
+  const ShuffleLayout sl = shuffle_layout(B, ld);
+  l.jld = sl.jld;
+  l.cuts_ld = sl.cuts_ld;
+  const size_t shuffle = take(isd ? sl.bytes : 0);
+  l.isd_jseq = shuffle + sl.jseq;
+  l.isd_cuts = shuffle + sl.cuts;
+  l.isd_state = shuffle + sl.state;
   l.ssi_noise = take(ssi ? (size_t)B * ld * 4 : 0);
   l.ssi_params = take(ssi ? (size_t)B * stride * 8 : 0);
   l.ssi_cnt = take(ssi ? (size_t)B * 4 : 0);
@@ -840,7 +723,7 @@ namespace rb {
 // Stage 1: validation, first draws of every utterance, CSR offsets of the LnL taps and the impulses, LnL filter design.
 // Fills *plan with device pointers into `storage` (their contents are complete once all four stages have run).
 int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds, void* storage,
-                  size_t storage_bytes, rb_plan* plan, cudaStream_t st) {
+                  size_t storage_bytes, rb_plan* plan, cudaStream_t st, const uint32_t* snaps) {
   if (!args || !plan || B < 0 || ld < 0) return RB_ERR_INVALID_ARG;
   memset(plan, 0, sizeof(*plan));
   const bool lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
@@ -849,7 +732,7 @@ int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* l
   plan->n_f = lnl ? args->N_f : 0;
   plan->g_sd = (float)args->g_sd;
   if (B == 0 || ld == 0 || !(lnl || isd || ssi)) return RB_OK;
-  if (!len || !seeds) return RB_ERR_INVALID_ARG;
+  if (!len || !(seeds || snaps)) return RB_ERR_INVALID_ARG;
   if (!args_ok(*args)) return RB_ERR_UNSUPPORTED;
   if (isd && ld > (1 << 30)) return RB_ERR_UNSUPPORTED;
   if (ld % 4 != 0) return RB_ERR_ALIGNMENT;
@@ -859,7 +742,7 @@ int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* l
   char* d = (char*)storage;
   const int nl = lnl ? B * args->N_f : 0;
   plan_head_kernel<<<(B + kHeadWarps - 1) / kHeadWarps, 32 * kHeadWarps, 0, st>>>(
-      *args, algo, B, len, seeds, (double*)(d + l.lnl_params), (int32_t*)(d + l.lnl_cnt), (int32_t*)(d + l.isd_cnt));
+      *args, algo, B, len, seeds, snaps, (double*)(d + l.lnl_params), (int32_t*)(d + l.lnl_cnt), (int32_t*)(d + l.isd_cnt));
   RB_LAUNCH_CHECK();
   if (isd) {
     scan_kernel<<<1, 1024, 0, st>>>((const int32_t*)(d + l.isd_cnt), B, (int32_t*)(d + l.isd_off));
@@ -888,7 +771,7 @@ int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* l
 
 // Stage 2, utterances [first, first+count): the rest of the stream (swap targets and groups, impulse gains, SSI draws).
 int devplan_body(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds, void* storage, int first,
-                 int count, cudaStream_t st) {
+                 int count, cudaStream_t st, const uint32_t* snaps) {
   const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
   const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
   if (!(isd || ssi) || count <= 0) return RB_OK;
@@ -896,15 +779,17 @@ int devplan_body(const rb_args* args, int algo, int B, int ld, const int32_t* le
   char* d = (char*)storage;
   const size_t stride = 3 * (size_t)args->nBands + 1;
   const unsigned grid = (count + kBodyWarps - 1) / kBodyWarps;
+  const uint32_t* sd = seeds ? seeds + first : nullptr;
+  const uint32_t* sn = snaps ? snaps + (size_t)first * kMtSnapWords : nullptr;
   if (ld > kNarrowMax)
     plan_body_kernel<uint32_t><<<grid, 32 * kBodyWarps, 0, st>>>(
-        *args, algo, count, ld, l.jld, len + first, seeds + first, (const int32_t*)(d + l.isd_off) + first, (double*)(d + l.isd_fr),
+        *args, algo, count, ld, l.jld, len + first, sd, sn, (const int32_t*)(d + l.isd_off) + first, (double*)(d + l.isd_fr),
         (uint32_t*)(d + l.isd_jseq) + (size_t)first * l.jld, (uint32_t*)(d + l.isd_cuts) + (size_t)first * l.cuts_ld, l.cuts_ld,
         (float*)(d + l.ssi_noise) + (size_t)first * ld, (double*)(d + l.ssi_params) + (size_t)first * stride,
         (int32_t*)(d + l.ssi_cnt) + first, (float*)(d + l.ssi_snr) + first);
   else
     plan_body_kernel<uint16_t><<<grid, 32 * kBodyWarps, 0, st>>>(
-        *args, algo, count, ld, l.jld, len + first, seeds + first, (const int32_t*)(d + l.isd_off) + first, (double*)(d + l.isd_fr),
+        *args, algo, count, ld, l.jld, len + first, sd, sn, (const int32_t*)(d + l.isd_off) + first, (double*)(d + l.isd_fr),
         (uint16_t*)(d + l.isd_jseq) + (size_t)first * l.jld, (uint32_t*)(d + l.isd_cuts) + (size_t)first * l.cuts_ld, l.cuts_ld,
         (float*)(d + l.ssi_noise) + (size_t)first * ld, (double*)(d + l.ssi_params) + (size_t)first * stride,
         (int32_t*)(d + l.ssi_cnt) + first, (float*)(d + l.ssi_snr) + first);
@@ -912,18 +797,13 @@ int devplan_body(const rb_args* args, int algo, int B, int ld, const int32_t* le
   return RB_OK;
 }
 
-// Stage 3, utterances [first, first+count): apply the swaps, emit the impulse positions.
-int devplan_apply(const rb_args* args, int algo, int B, int ld, const int32_t* len, void* storage, int first, int count,
-                  cudaStream_t st) {
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  if (!isd || count <= 0) return RB_OK;
-  const DevPlanLayout l = layout(*args, algo, B, ld);
-  char* d = (char*)storage;
+// Apply the swaps of `count` rows (stride ld, padded to jld / cuts_ld) and emit the first off[u+1]-off[u] entries of row u's
+// permutation to idx[off[u]...].
+int launch_perm_apply(int count, int ld, int jld, int cuts_ld, const int32_t* len, const void* jseq, const uint32_t* cuts,
+                      const int32_t* off, int32_t* idx, void* state, cudaStream_t st) {
   if (ld > kNarrowMax) {
     perm_apply_wide_kernel<<<(count + kWideWarps - 1) / kWideWarps, 32 * kWideWarps, 0, st>>>(
-        count, l.jld, len + first, (const uint32_t*)(d + l.isd_jseq) + (size_t)first * l.jld,
-        (const uint32_t*)(d + l.isd_cuts) + (size_t)first * l.cuts_ld, l.cuts_ld, (const int32_t*)(d + l.isd_off) + first,
-        (int32_t*)(d + l.isd_idx), (uint32_t*)(d + l.isd_state) + (size_t)first * l.jld);
+        count, jld, len, (const uint32_t*)jseq, cuts, cuts_ld, off, idx, (uint32_t*)state);
     RB_LAUNCH_CHECK();
     return RB_OK;
   }
@@ -936,13 +816,43 @@ int devplan_apply(const rb_args* args, int algo, int B, int ld, const int32_t* l
     const size_t entries = (size_t)std::min(T_hi, (ld + 7) / 8 * 8) + 8;  // + the uint4 tail of the state copy
     const size_t smem = kApplyStageBytes + align_up(entries * 2, 16);
     if (smem > 227 * 1024) return RB_ERR_UNSUPPORTED;
-    perm_apply_kernel<<<count, 32, smem, st>>>(count, l.jld, len + first, (const uint16_t*)(d + l.isd_jseq) + (size_t)first * l.jld,
-                                              (const uint32_t*)(d + l.isd_cuts) + (size_t)first * l.cuts_ld, l.cuts_ld,
-                                              (const int32_t*)(d + l.isd_off) + first, (int32_t*)(d + l.isd_idx),
-                                              (uint16_t*)(d + l.isd_state) + (size_t)first * l.jld, T_hi, T_lo);
+    perm_apply_kernel<<<count, 32, smem, st>>>(count, jld, len, (const uint16_t*)jseq, cuts, cuts_ld, off, idx, (uint16_t*)state,
+                                              T_hi, T_lo);
     RB_LAUNCH_CHECK();
   }
   return RB_OK;
+}
+
+// Stage 3, utterances [first, first+count): apply the swaps, emit the impulse positions.
+int devplan_apply(const rb_args* args, int algo, int B, int ld, const int32_t* len, void* storage, int first, int count,
+                  cudaStream_t st) {
+  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
+  if (!isd || count <= 0) return RB_OK;
+  const DevPlanLayout l = layout(*args, algo, B, ld);
+  char* d = (char*)storage;
+  const size_t jbytes = ld > kNarrowMax ? 4 : 2;
+  return launch_perm_apply(count, ld, l.jld, l.cuts_ld, len + first, d + l.isd_jseq + (size_t)first * l.jld * jbytes,
+                           (const uint32_t*)(d + l.isd_cuts) + (size_t)first * l.cuts_ld, (const int32_t*)(d + l.isd_off) + first,
+                           (int32_t*)(d + l.isd_idx), d + l.isd_state + (size_t)first * l.jld * jbytes, st);
+}
+
+size_t shuffle_prefix_bytes(int B, int ld) { return B > 0 && ld > 0 ? shuffle_layout(B, ld).bytes : 0; }
+
+// np.random.permutation(len[u])[:off[u+1]-off[u]] -> out[off[u]...] for B rows whose streams start at snapshots[u].
+int shuffle_prefix(int B, int ld, const int32_t* len, const uint32_t* snaps, const int32_t* off, int32_t* out, void* storage,
+                   cudaStream_t st) {
+  if (B <= 0 || ld <= 0) return RB_OK;
+  const ShuffleLayout l = shuffle_layout(B, ld);
+  char* d = (char*)storage;
+  const unsigned grid = (B + kBodyWarps - 1) / kBodyWarps;
+  if (ld > kNarrowMax)
+    shuffle_scan_kernel<uint32_t><<<grid, 32 * kBodyWarps, 0, st>>>(B, l.jld, len, snaps, (uint32_t*)(d + l.jseq),
+                                                                   (uint32_t*)(d + l.cuts), l.cuts_ld);
+  else
+    shuffle_scan_kernel<uint16_t><<<grid, 32 * kBodyWarps, 0, st>>>(B, l.jld, len, snaps, (uint16_t*)(d + l.jseq),
+                                                                   (uint32_t*)(d + l.cuts), l.cuts_ld);
+  RB_LAUNCH_CHECK();
+  return launch_perm_apply(B, ld, l.jld, l.cuts_ld, len, d + l.jseq, (const uint32_t*)(d + l.cuts), off, out, d + l.state, st);
 }
 
 // Stage 4 (after stage 2 of ALL utterances): CSR offsets and design of the SSI filters.

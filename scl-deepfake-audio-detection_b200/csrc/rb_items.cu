@@ -1,0 +1,265 @@
+// rb_items.cu -- whole Dataset_for items (asvspoof_2019_augall_3.py:103-146, RawBoost12 with online_aug) for a batch of items
+// that are each seeded on their own: np.random.seed(seeds[g]) before item g, as a reproducible loader does per __getitem__.
+//
+// Item g consumes ONE stream, in this order: RawBoost (algo 5) on every vocoded copy in vocoder order, then on the anchor --
+// each of them N_f LnL parameter sets, ISD beta, permutation(L), rand(n) twice -- then np.random.choice(others, n_add,
+// replace=False), which legacy numpy computes as permutation(N-1)[:n_add] mapped through `others` (v -> v + (v >= idx)),
+// then the shared crop int(rand() * (L_anchor - trim)), drawn only when L_anchor >= trim. Different items are independent,
+// so they run in parallel; only the draws inside one item share a stream.
+//
+// Two passes:
+//   items_walk_kernel    one warp per item: seeds the stream and walks the whole item, counting words only (the shuffles
+//                        with the ballot fix-point of shuffle_walk_warp). It stores a snapshot of the stream (numpy's state
+//                        form) at the start of every RawBoost utterance and of the choice, and draws the crop start.
+//   then the per-utterance planner (rb_devplan.cu) runs unchanged over the G*(nvoc+1) utterances from their snapshots, and
+//   shuffle_prefix applies the choice permutations.
+//   items_rows_kernel    the batch's source rows in the corpus, their lengths, the view table of the assembly, the label vector
+//   items_gather_kernel  one CTA per batch row: corpus row -> batch row (rb_items_run only)
+// rb_items_run then finishes with rb_process(5) and rb_multiview_assemble_ex, exactly as ItemBatcher does.
+//
+// Corpus layout: rows [R, ld], R = N * (1 + nvoc); row idx is bona fide utterance idx, row N + idx*nvoc + v is vocoder v's copy.
+// Batch layout (ItemBatcher's): rows g*(nvoc+1) + v hold item g's vocoded copies (v < nvoc) and its anchor (v = nvoc); rows
+// G*(nvoc+1) + g*n_add + k hold its additional bona fide utterances (not augmented).
+#include <limits.h>
+#include <string.h>
+
+#include <algorithm>
+
+#include "rb_common.cuh"
+#include "rb_mt.cuh"
+
+namespace rb {
+namespace {
+
+constexpr int kWalkWarps = 4;  // 30 KB of MT19937 state per CTA, as plan_body_kernel
+
+__device__ __forceinline__ int clamp_index(int idx, int N) { return (idx >= 0 && idx < N) ? idx : 0; }
+
+__global__ void __launch_bounds__(32 * kWalkWarps)
+items_walk_kernel(rb_args a, int G, int nvoc, int n_add, int N, int trim, const int32_t* __restrict__ corpus_len,
+                  const int32_t* __restrict__ indices, const uint32_t* __restrict__ seeds, uint32_t* __restrict__ snaps,
+                  uint32_t* __restrict__ csnaps, int32_t* __restrict__ start, uint32_t* __restrict__ end_state,
+                  int32_t* __restrict__ choice_len, int32_t* __restrict__ choice_off) {
+  __shared__ MtSmem sm[kWalkWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = blockIdx.x * kWalkWarps + warp;
+  if (g >= G) return;
+  const int idx = clamp_index(indices[g], N);
+  const int U = nvoc + 1;
+  MtStream s;
+  s.sm = &sm[warp];
+  s.seed(seeds[g], lane);
+  const int lnl_words = a.N_f * 2 * filter_stride(a.nBands);
+  for (int v = 0; v < U; ++v) {
+    const int L = corpus_len[v < nvoc ? N + idx * nvoc + v : idx];
+    s.store(snaps + ((size_t)g * U + v) * kMtSnapWords, lane);
+    s.skip(lnl_words, lane);
+    const double beta = mt_uniform(0.0, a.P, mt_double(s.word(0), s.word(1)));  // as plan_head_kernel
+    const int n = (int)__dmul_rn((double)L, __ddiv_rn(beta, 100.0));
+    s.advance(2, lane);
+    shuffle_walk_warp<false, uint32_t>(s, L, nullptr, lane);
+    for (int k = 0; k < 4; ++k) s.skip(n, lane);  // f_r: rand(n) twice, two words per double
+  }
+  s.store(csnaps + (size_t)g * kMtSnapWords, lane);
+  shuffle_walk_warp<false, uint32_t>(s, N - 1, nullptr, lane);
+  const int La = corpus_len[idx];
+  int st = 0;
+  if (La >= trim) {
+    st = (int)__dmul_rn(mt_double(s.word(0), s.word(1)), (double)(La - trim));
+    s.advance(2, lane);
+  }
+  if (end_state) s.store(end_state + (size_t)g * kMtSnapWords, lane);
+  if (lane == 0) {
+    start[g] = st;
+    choice_len[g] = N - 1;
+    choice_off[g] = g * n_add;
+    if (g == G - 1) choice_off[G] = G * n_add;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+items_rows_kernel(int G, int nvoc, int n_add, int N, const int32_t* __restrict__ corpus_len, const int32_t* __restrict__ indices,
+                  const int32_t* __restrict__ choice, int32_t* __restrict__ src_row, int32_t* __restrict__ row_len,
+                  int32_t* __restrict__ view_row, float* __restrict__ view_label) {
+  const int U = nvoc + 1, V = 2 + n_add + 2 * nvoc;
+  const size_t nb = (size_t)G * U, rows = nb + (size_t)G * n_add;
+  const size_t step = (size_t)gridDim.x * blockDim.x, t0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  for (size_t r = t0; r < rows; r += step) {
+    int src;
+    if (r < nb) {
+      const int g = (int)(r / U), v = (int)(r - (size_t)g * U);
+      const int idx = clamp_index(indices[g], N);
+      src = v < nvoc ? N + idx * nvoc + v : idx;
+    } else {
+      const size_t q = r - nb;
+      const int idx = clamp_index(indices[q / n_add], N);
+      const int c = choice[q];
+      src = c + (c >= idx ? 1 : 0);  // position in others = list(range(N)) without idx
+    }
+    src_row[r] = src;
+    row_len[r] = corpus_len[src];
+  }
+  // view order of Dataset_for (line 133): anchor, augmented anchor, additional bona fide, vocoded, augmented vocoded; a row
+  // r >= 0 is read from the batch, -1-r from its RawBoost results
+  for (size_t e = t0; e < (size_t)G * V; e += step) {
+    const int g = (int)(e / V), k = (int)(e - (size_t)g * V);
+    const int base = g * U;
+    int r;
+    if (k < 2) r = k == 0 ? base + nvoc : -1 - (base + nvoc);
+    else if (k < 2 + n_add) r = (int)nb + g * n_add + (k - 2);
+    else if (k < 2 + n_add + nvoc) r = base + (k - 2 - n_add);
+    else r = -1 - (base + (k - 2 - n_add - nvoc));
+    view_row[e] = r;
+  }
+  for (size_t k = t0; k < (size_t)V; k += step) view_label[k] = k < (size_t)(2 + n_add) ? 1.f : 0.f;  // asvspoof_2019_augall_3.py:143-146
+}
+
+__global__ void __launch_bounds__(256)
+items_gather_kernel(const float* __restrict__ corpus, int ld, const int32_t* __restrict__ src_row, const int32_t* __restrict__ row_len,
+                    float* __restrict__ x) {
+  const size_t r = blockIdx.x;
+  const float4* src = reinterpret_cast<const float4*>(corpus + (size_t)src_row[r] * ld);
+  float4* dst = reinterpret_cast<float4*>(x + r * ld);
+  const int n4 = (row_len[r] + 3) >> 2;  // the row's padding up to ld is never read
+  for (int k = threadIdx.x; k < n4; k += blockDim.x) dst[k] = __ldg(src + k);
+}
+
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+struct ItemsLayout {
+  size_t snaps, csnaps, clen, coff, cpos, shuffle, view_row, view_label, plan, plan_bytes, draw_bytes;
+  size_t src_row, row_len, start, x, y, proc, proc_bytes, bytes;
+};
+
+ItemsLayout items_layout(const rb_args* args, int G, int nvoc, int n_add, int N, int ld) {
+  ItemsLayout l{};
+  size_t off = 0;
+  auto take = [&](size_t n) {
+    const size_t r = off;
+    off += align_up(n, 256);
+    return r;
+  };
+  const int U = nvoc + 1, V = 2 + n_add + 2 * nvoc;
+  const size_t nb = (size_t)G * U, rows = nb + (size_t)G * n_add;
+  l.snaps = take(nb * kMtSnapWords * 4);
+  l.csnaps = take((size_t)G * kMtSnapWords * 4);
+  l.clen = take((size_t)G * 4);
+  l.coff = take((size_t)(G + 1) * 4);
+  l.cpos = take((size_t)G * n_add * 4);
+  l.shuffle = take(n_add > 0 ? shuffle_prefix_bytes(G, N - 1) : 0);
+  l.view_row = take((size_t)G * V * 4);
+  l.view_label = take((size_t)V * 4);
+  l.plan_bytes = rb_devplan_bytes(args, 5, (int)nb, ld);
+  l.plan = take(l.plan_bytes);
+  l.draw_bytes = off;
+  l.src_row = take(rows * 4);
+  l.row_len = take(rows * 4);
+  l.start = take((size_t)G * 4);
+  l.x = take(rows * ld * 4);
+  l.y = take(nb * ld * 4);
+  l.proc_bytes = rb_workspace_bytes_for(5, (int)nb, ld);
+  l.proc = take(l.proc_bytes);
+  l.bytes = off;
+  return l;
+}
+
+// shape checks shared by the three entries; RB_OK when the shape is drawable
+int check_shape(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim) {
+  if (!args || G < 0 || nvoc < 0 || n_add < 0 || N < 1 || ld <= 0 || trim < 1) return RB_ERR_INVALID_ARG;
+  if (n_add > N - 1) return RB_ERR_INVALID_ARG;  // np.random.choice(..., replace=False) cannot take more than N-1
+  if ((int64_t)N * (1 + nvoc) > INT_MAX || (int64_t)G * (nvoc + 1 + n_add) > INT_MAX) return RB_ERR_INVALID_ARG;
+  if (G > 0 && (int64_t)G * (nvoc + 1) * args->N_f > INT_MAX) return RB_ERR_INVALID_ARG;
+  if (ld % 4 != 0) return RB_ERR_ALIGNMENT;
+  if (ld > (1 << 30) || N - 1 > (1 << 30)) return RB_ERR_UNSUPPORTED;
+  if (G > 0 && rb_devplan_bytes(args, 5, G * (nvoc + 1), ld) == 0) return RB_ERR_UNSUPPORTED;
+  return RB_OK;
+}
+
+int check_workspace(const void* ws, size_t have, size_t need) {
+  if (!ws) return RB_ERR_WORKSPACE;
+  if ((uintptr_t)ws & 255u) return RB_ERR_ALIGNMENT;
+  return have < need ? RB_ERR_WORKSPACE : RB_OK;
+}
+
+// every draw of the batch: snapshots, crop starts, choice, row tables, plan
+int items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
+               const int32_t* indices, const uint32_t* seeds, int32_t* src_row, int32_t* row_len, int32_t* start,
+               uint32_t* end_state, char* d, const ItemsLayout& l, rb_plan* plan, cudaStream_t st) {
+  const int nb = G * (nvoc + 1);
+  items_walk_kernel<<<(G + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, st>>>(
+      *args, G, nvoc, n_add, N, trim, corpus_len, indices, seeds, (uint32_t*)(d + l.snaps), (uint32_t*)(d + l.csnaps), start,
+      end_state, (int32_t*)(d + l.clen), (int32_t*)(d + l.coff));
+  RB_LAUNCH_CHECK();
+  int rc;
+  if (n_add > 0 && (rc = shuffle_prefix(G, N - 1, (const int32_t*)(d + l.clen), (const uint32_t*)(d + l.csnaps),
+                                        (const int32_t*)(d + l.coff), (int32_t*)(d + l.cpos), d + l.shuffle, st)) != RB_OK)
+    return rc;
+  const size_t work = (size_t)G * (nvoc + 1 + n_add) + (size_t)G * (2 + n_add + 2 * nvoc);
+  const int grid = (int)std::min<size_t>((work + 255) / 256, 148 * 8);
+  items_rows_kernel<<<grid, 256, 0, st>>>(G, nvoc, n_add, N, corpus_len, indices, (const int32_t*)(d + l.cpos), src_row, row_len,
+                                         (int32_t*)(d + l.view_row), (float*)(d + l.view_label));
+  RB_LAUNCH_CHECK();
+  const uint32_t* snaps = (const uint32_t*)(d + l.snaps);
+  void* pm = d + l.plan;
+  if ((rc = devplan_begin(args, 5, nb, ld, row_len, nullptr, pm, l.plan_bytes, plan, st, snaps)) != RB_OK) return rc;
+  if ((rc = devplan_body(args, 5, nb, ld, row_len, nullptr, pm, 0, nb, st, snaps)) != RB_OK) return rc;
+  if ((rc = devplan_apply(args, 5, nb, ld, row_len, pm, 0, nb, st)) != RB_OK) return rc;
+  return devplan_end(args, 5, nb, ld, pm, st);
+}
+
+}  // namespace
+}  // namespace rb
+
+using namespace rb;
+
+extern "C" {
+
+size_t rb_items_workspace_bytes(const rb_args* args, int G, int nvoc, int n_add, int N, int ld) {
+  if (check_shape(args, G, nvoc, n_add, N, ld, 1) != RB_OK || G == 0) return 0;
+  return items_layout(args, G, nvoc, n_add, N, ld).bytes;
+}
+
+int rb_items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
+                  const int32_t* indices, const uint32_t* seeds, int32_t* src_row, int32_t* row_len, int32_t* start,
+                  uint32_t* end_state, void* workspace, size_t workspace_bytes, rb_plan* plan, void* stream) {
+  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
+  if (rc != RB_OK) return rc;
+  if (!plan) return RB_ERR_INVALID_ARG;
+  memset(plan, 0, sizeof(*plan));
+  if (G == 0) return RB_OK;
+  if (!corpus_len || !indices || !seeds || !src_row || !row_len || !start) return RB_ERR_INVALID_ARG;
+  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
+  if ((rc = check_workspace(workspace, workspace_bytes, l.draw_bytes)) != RB_OK) return rc;
+  return items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, seeds, src_row, row_len, start, end_state,
+                    (char*)workspace, l, plan, (cudaStream_t)stream);
+}
+
+int rb_items_run(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
+                 const float* corpus, const int32_t* corpus_len, const int32_t* indices, const uint32_t* seeds, float* out,
+                 int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
+  if (rc != RB_OK) return rc;
+  const int V = 2 + n_add + 2 * nvoc;
+  if ((layout != 0 && layout != 1) || (labels && V > 256)) return RB_ERR_INVALID_ARG;
+  if (G == 0) return RB_OK;
+  if (!corpus || !corpus_len || !indices || !seeds || !out) return RB_ERR_INVALID_ARG;
+  if ((uintptr_t)corpus & 15u) return RB_ERR_ALIGNMENT;
+  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
+  if ((rc = check_workspace(workspace, workspace_bytes, l.bytes)) != RB_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  char* d = (char*)workspace;
+  int32_t *src_row = (int32_t*)(d + l.src_row), *row_len = (int32_t*)(d + l.row_len), *start = (int32_t*)(d + l.start);
+  rb_plan plan;
+  if ((rc = items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, seeds, src_row, row_len, start, end_state, d, l,
+                       &plan, st)) != RB_OK)
+    return rc;
+  const int rows = G * (nvoc + 1 + n_add), nb = G * (nvoc + 1);
+  float *x = (float*)(d + l.x), *y = (float*)(d + l.y);
+  items_gather_kernel<<<rows, 256, 0, st>>>(corpus, ld, src_row, row_len, x);
+  RB_LAUNCH_CHECK();
+  if ((rc = rb_process(5, x, row_len, nb, ld, &plan, y, d + l.proc, l.proc_bytes, stream)) != RB_OK) return rc;
+  return rb_multiview_assemble_ex(x, y, (const int32_t*)(d + l.view_row), row_len, G, V, ld, start, trim, repeat_pad, layout, out,
+                                  out_len, labels ? (const float*)(d + l.view_label) : nullptr, labels, stream);
+}
+
+}  // extern "C"

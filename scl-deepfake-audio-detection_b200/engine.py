@@ -123,6 +123,89 @@ class Engine:
             bp.ssi_snr_db = fetch(s.ssi_snr_db, B, np.float32)
         return bp
 
+    def _item_arrays(self, indices, seeds):
+        """indices / seeds as int32 device tensors (seeds hold the uint32 bit patterns)."""
+        if not torch.is_tensor(indices):
+            indices = torch.from_numpy(np.ascontiguousarray(indices, dtype=np.int32)).to(self.device)
+        if not torch.is_tensor(seeds):
+            seeds = torch.from_numpy(np.ascontiguousarray(np.asarray(seeds, dtype=np.int64).astype(np.uint32)).view(np.int32)).to(self.device)
+        for name, t in (("indices", indices), ("seeds", seeds)):
+            if t.device != self.device or t.element_size() != 4 or t.dim() != 1 or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous 1-D 32-bit integer tensor on {self.device}")
+        if indices.numel() != seeds.numel():
+            raise ValueError("one seed per item")
+        return indices, seeds
+
+    def items_draw(self, args, sr, corpus_len: torch.Tensor, nvoc: int, n_add: int, ld: int, trim: int, indices, seeds,
+                   end_state: bool = False):
+        """Every draw of G independently seeded items (``rb_items_draw``; see ``multiview.SeededItemBatcher``). ``corpus_len``:
+        int32 [N*(1+nvoc)] device lengths of the corpus rows. Returns a dict: ``plan`` (a :class:`DevicePlan` of the G*(nvoc+1)
+        RawBoost utterances, owning its device buffer), ``src_row`` and ``row_len`` (int32 [G*(nvoc+1+n_add)]), ``start``
+        (int32 [G]) and, with ``end_state``, ``end_state`` (int32 [G, 625]: each item's numpy state key[624], pos after its
+        last draw, as uint32 bit patterns). Asynchronous on torch's current stream."""
+        indices, seeds = self._item_arrays(indices, seeds)
+        G, R = int(indices.numel()), int(corpus_len.numel())
+        if corpus_len.dtype != torch.int32 or corpus_len.device != self.device or R % (1 + nvoc):
+            raise ValueError("corpus_len must be int32 [N*(1+nvoc)] on the engine's device")
+        N = R // (1 + nvoc)
+        a = _lib.args_struct(args, sr)
+        need = int(self.lib.rb_items_workspace_bytes(C.byref(a), G, int(nvoc), int(n_add), N, int(ld)))
+        if G and need == 0:
+            raise ValueError(f"unsupported item shape: G={G}, nvoc={nvoc}, n_add={n_add}, N={N}, ld={ld}")
+        store = torch.empty(need + 256, dtype=torch.uint8, device=self.device)
+        rows = G * (nvoc + 1 + n_add)
+        src_row = torch.empty(rows, dtype=torch.int32, device=self.device)
+        row_len = torch.empty(rows, dtype=torch.int32, device=self.device)
+        start = torch.empty(G, dtype=torch.int32, device=self.device)
+        end = torch.empty((G, 625), dtype=torch.int32, device=self.device) if end_state else None
+        s = _lib.RbPlan()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_draw(C.byref(a), G, int(nvoc), int(n_add), N, int(ld), int(trim), _ptr(corpus_len), _ptr(indices),
+                                        _ptr(seeds), _ptr(src_row), _ptr(row_len), _ptr(start), _ptr(end),
+                                        C.c_void_p(self._ws_ptr(store)), need, C.byref(s), C.c_void_p(stream))
+        _lib.check(rc, "rb_items_draw")
+        B = G * (nvoc + 1)
+        plan = DevicePlan(B=B, ld=int(ld), lengths=row_len[:B], tensors={"storage": store}, struct=s, host=None)
+        return {"plan": plan, "src_row": src_row, "row_len": row_len, "start": start, "end_state": end}
+
+    def items_run(self, args, sr, corpus: torch.Tensor, corpus_len: torch.Tensor, nvoc: int, n_add: int, trim: int, indices, seeds,
+                  repeat_pad: bool = True, layout: int = 0, out: Optional[torch.Tensor] = None, with_labels: bool = True,
+                  end_state: Optional[torch.Tensor] = None):
+        """Whole items, every step on the device (``rb_items_run``): draw, gather, RawBoost (algo 5), crop and view assembly.
+        ``corpus`` [N*(1+nvoc), ld] float32 with lengths ``corpus_len`` (int32). Returns ``(out, out_len, labels)``: out
+        [G, trim, V] (layout 0) or [G, V, trim] (layout 1), zero past out_len[g]; labels [G, V] (None without ``with_labels``).
+        ``end_state``: optional int32 [G, 625] device tensor for each item's final stream state. Asynchronous on torch's
+        current stream; with device ``indices`` / ``seeds`` nothing synchronises with the host."""
+        indices, seeds = self._item_arrays(indices, seeds)
+        if corpus.dtype != torch.float32 or corpus.dim() != 2 or not corpus.is_contiguous() or corpus.device != self.device:
+            raise ValueError("corpus must be a contiguous [R, ld] float32 tensor on the engine's device")
+        R, ld = corpus.shape
+        if corpus_len.dtype != torch.int32 or corpus_len.device != self.device or corpus_len.numel() != R or R % (1 + nvoc):
+            raise ValueError("corpus_len must be int32 [R] on the engine's device, R = N*(1+nvoc)")
+        N, G, V = R // (1 + nvoc), int(indices.numel()), 2 + n_add + 2 * nvoc
+        shape = (G, trim, V) if layout == 0 else (G, V, trim)
+        if out is None:
+            out = torch.zeros(shape, dtype=torch.float32, device=self.device)
+        elif tuple(out.shape) != shape or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 tensor {shape} on the engine's device")
+        if end_state is not None and (end_state.shape != (G, 625) or end_state.element_size() != 4 or end_state.device != self.device):
+            raise ValueError("end_state must be a 32-bit [G, 625] tensor on the engine's device")
+        out_len = torch.empty(G, dtype=torch.int32, device=self.device)
+        labels = torch.empty((G, V), dtype=torch.float32, device=self.device) if with_labels else None
+        a = _lib.args_struct(args, sr)
+        need = int(self.lib.rb_items_workspace_bytes(C.byref(a), G, int(nvoc), int(n_add), N, int(ld)))
+        if G and need == 0:
+            raise ValueError(f"unsupported item shape: G={G}, nvoc={nvoc}, n_add={n_add}, N={N}, ld={ld}")
+        ws = self._scratch(need)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_run(C.byref(a), G, int(nvoc), int(n_add), N, int(ld), int(trim), int(bool(repeat_pad)), int(layout),
+                                       _ptr(corpus), _ptr(corpus_len), _ptr(indices), _ptr(seeds), _ptr(out), _ptr(out_len), _ptr(labels),
+                                       _ptr(end_state), C.c_void_p(self._ws_ptr(ws)), need, C.c_void_p(stream))
+        _lib.check(rc, "rb_items_run")
+        return out, out_len, labels
+
     def pack_waveforms(self, waves: Sequence[np.ndarray], ld: Optional[int] = None):
         """Host list of 1-D float arrays -> ([B, ld] float32 device tensor, int32 lengths on device)."""
         lengths = np.array([int(w.shape[0]) for w in waves], dtype=np.int32)

@@ -10,6 +10,9 @@
   or ``[G, V, length]`` (what the model consumes after main.py:57-60) without visiting the host.
 * :func:`item_views` -- one call for whole items in the loader's order (RawBoost12 on the vocoded copies, then on the
   anchor, then the crop: asvspoof_2019_augall_3.py:109-138).
+* :class:`ItemBatcher` -- whole ``Dataset_for`` items, every draw on the host from the global numpy stream.
+* :class:`DeviceCorpus` + :class:`SeededItemBatcher` -- whole items seeded one by one (``np.random.seed(s)`` before each
+  ``__getitem__``), every draw replayed on the device from a corpus that lives there.
 
 Integer work (crop start, index map) is bit-exact; the samples are copies of the views' float32 values.
 """
@@ -243,6 +246,88 @@ class ItemBatcher:
         label = torch.from_numpy(item_labels(nvoc, n_add))
         out, out_len, labels = assemble_ex(eng, x, y, rows, ln, V, starts, self.trim_length, self.repeat_pad, layout, view_label=label)
         return [self.list_ids[i] for i in indices], out, labels, out_len
+
+
+class DeviceCorpus:
+    """Every bona fide utterance of ``list_ids`` and its vocoded copies, loaded once into device memory in the layout the
+    per-item device path reads: rows [R, ld] float32 with R = N * (1 + nvoc); row ``idx`` is bona fide utterance ``idx``
+    (``<base_dir>/bonafide/<id>``), row ``N + idx*nvoc + v`` is vocoder v's copy (``<base_dir>/vocoded/<vocoder>_<id>``), as
+    ``Dataset_for`` names them. ld is the longest waveform rounded up to 4 samples, so the corpus costs R * ld * 4 bytes of
+    device memory (2.7 GB for the 2580 bona fide utterances of ASVspoof 2019 LA train with 3 vocoders at 64 600 samples).
+
+    ``load_audio(path) -> float32 waveform`` is the caller's reader (``librosa.load`` in the reference). Every waveform needs at
+    least one sample."""
+
+    def __init__(self, list_ids, base_dir, load_audio, vocoders=(), engine: Optional[Engine] = None):
+        import os
+        self.list_ids, self.vocoders = list(list_ids), list(vocoders)
+        self.eng = engine or default_engine()
+        self.N, self.nvoc = len(self.list_ids), len(self.vocoders)
+        if self.N < 1:
+            raise ValueError("the corpus needs at least one utterance")
+        paths = [os.path.join(base_dir, "bonafide", name) for name in self.list_ids]
+        paths += [os.path.join(base_dir, "vocoded", v + "_" + name) for name in self.list_ids for v in self.vocoders]
+        waves = [np.asarray(load_audio(p), dtype=np.float32).reshape(-1) for p in paths]
+        lengths = np.array([w.shape[0] for w in waves], dtype=np.int32)
+        if lengths.min() < 1:
+            raise ValueError(f"empty waveform: {paths[int(np.argmin(lengths))]}")
+        self.ld = _plans.padded_ld(int(lengths.max()))
+        self.data = torch.zeros((len(waves), self.ld), dtype=torch.float32, device=self.eng.device)
+        chunk = max(1, (256 << 20) // (4 * self.ld))  # rows per host staging buffer of at most 256 MB
+        for r0 in range(0, len(waves), chunk):
+            part = waves[r0:r0 + chunk]
+            host = np.zeros((len(part), self.ld), dtype=np.float32)
+            for k, w in enumerate(part):
+                host[k, :w.shape[0]] = w
+            self.data[r0:r0 + len(part)].copy_(torch.from_numpy(host))
+        self.lengths = torch.from_numpy(lengths).to(self.eng.device)
+
+
+class SeededItemBatcher:
+    """``Dataset_for.__getitem__`` (asvspoof_2019_augall_3.py:103-146, ``augmentation_methods == ['RawBoost12']`` with
+    ``online_aug``) for a batch of items seeded one by one: item g equals
+
+        np.random.seed(seeds[g]); __getitem__(indices[g])
+
+    -- RawBoost (algo 5) on each vocoded copy and on the anchor, ``np.random.choice`` of ``num_additional_real`` other bona fide
+    utterances, one shared crop (``random_trim_nosil``) -- with every draw replayed on the device. Items are independent, so a
+    whole batch runs in one pass with no host work beyond the indices and seeds. numpy's global stream is never touched;
+    :class:`ItemBatcher` keeps the unseeded semantics, where consecutive items share one stream."""
+
+    def __init__(self, args, corpus: DeviceCorpus, num_additional_real=2, trim_length=64000, repeat_pad=True, wav_samp_rate=16000):
+        self.args, self.corpus = args, corpus
+        self.num_additional_real, self.trim_length = int(num_additional_real), int(trim_length)
+        self.repeat_pad, self.sr = bool(repeat_pad), int(wav_samp_rate)
+        if not 0 <= self.num_additional_real <= corpus.N - 1:
+            raise ValueError(f"num_additional_real must lie in [0, {corpus.N - 1}] for a corpus of {corpus.N} utterances")
+
+    def _indices(self, indices):
+        if torch.is_tensor(indices):
+            return indices, indices
+        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= self.corpus.N):
+            raise IndexError(f"indices must lie in [0, {self.corpus.N})")
+        return idx.astype(np.int32), [self.corpus.list_ids[i] for i in idx]
+
+    def items(self, indices, seeds, layout: int = LAYOUT_ITEM, end_state: Optional[torch.Tensor] = None):
+        """``(ids, data, labels, out_len)`` as :meth:`ItemBatcher.items`: ``data`` [G, trim_length, V] (LAYOUT_ITEM) or
+        [G, V, trim_length] (LAYOUT_MODEL), ``labels`` [G, V], ``out_len`` int32 [G], all on the device. ``indices`` and ``seeds``
+        are host sequences or 32-bit device tensors; with device tensors nothing synchronises with the host and ``ids`` is the
+        indices tensor itself (the utterance names stay with the caller). Device indices must lie in [0, N).
+        ``end_state``: optional int32 [G, 625] device tensor that receives each item's numpy stream state after its last draw."""
+        idx, ids = self._indices(indices)
+        c = self.corpus
+        data, out_len, labels = c.eng.items_run(self.args, self.sr, c.data, c.lengths, c.nvoc, self.num_additional_real,
+                                                self.trim_length, idx, seeds, self.repeat_pad, layout, end_state=end_state)
+        return ids, data, labels, out_len
+
+    def draw(self, indices, seeds, end_state: bool = False):
+        """The draws alone (:meth:`Engine.items_draw`): the RawBoost plan of the G*(nvoc+1) utterances, each batch row's
+        corpus row and length, the crop starts and optionally the end states."""
+        idx, _ = self._indices(indices)
+        c = self.corpus
+        return c.eng.items_draw(self.args, self.sr, c.lengths, c.nvoc, self.num_additional_real, c.ld, self.trim_length, idx, seeds,
+                                end_state=end_state)
 
 
 def _repad(bp, ld):
