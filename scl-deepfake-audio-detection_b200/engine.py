@@ -67,6 +67,10 @@ class Engine:
             arr = getattr(plan, name)
             if arr is not None:
                 src = torch.from_numpy(np.ascontiguousarray(arr))
+                if src.numel() == 0:
+                    # an empty CUDA tensor has a NULL data pointer, which the ABI reads as a missing plan field; a batch
+                    # whose utterances draw no impulses at all has empty isd_idx / isd_fr and must still run
+                    src = torch.zeros(1, dtype=src.dtype)
                 t[name] = src.to(self.device, non_blocking=False)
             else:
                 t[name] = None
