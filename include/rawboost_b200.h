@@ -266,6 +266,27 @@ RB_API int rb_items_run(const rb_args* args, int G, int nvoc, int n_add, int N, 
                         const float* corpus, const int32_t* corpus_len, const int32_t* indices, const uint32_t* seeds, float* out,
                         int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Items that share numpy's running stream (Dataset_for.__getitem__ called for them one after another, no per-item seed):
+ * S independent streams; the items of stream s are [stream_off[s], stream_off[s+1]) of indices (device int32[S+1],
+ * stream_off[0] = 0, non-decreasing, stream_off[S] = G). start_state (device uint32[S][625]) is numpy's key[624], pos (0..624),
+ * as RandomState.get_state()[1:3]; end_state (nullable, device uint32[S][625]) receives each stream's state after its last
+ * draw (pos 0..623). Every other argument, output, workspace and row layout as rb_items_draw / rb_items_run; the workspace is
+ * rb_items_workspace_bytes(args, G, nvoc, n_add, N, ld). S < 0, or S == 0 with G > 0, is RB_ERR_INVALID_ARG; empty streams
+ * are legal (S may exceed G; an empty stream's end state is its start state). G == 0 launches nothing and writes no end state.
+ * One warp walks each stream's items in order, so a stream's walk takes time in proportion to its item count.
+ * The table and the states are device data and are read defensively: offsets are clamped to [0, G], a decreasing step is an
+ * empty stream, the first stream starts at item 0 and the last ends at item G, and pos is clamped to 0..624. A malformed table
+ * never leads to an access out of bounds, but the items it does not describe (in no stream's range, or in two) and the end
+ * states of the streams involved are unspecified. */
+RB_API int rb_items_stream_draw(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld,
+                                int trim, const int32_t* corpus_len, const int32_t* indices, const uint32_t* start_state,
+                                int32_t* src_row, int32_t* row_len, int32_t* start, uint32_t* end_state,
+                                void* workspace, size_t workspace_bytes, rb_plan* plan, void* stream);
+RB_API int rb_items_stream_run(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld,
+                               int trim, int repeat_pad, int layout, const float* corpus, const int32_t* corpus_len,
+                               const int32_t* indices, const uint32_t* start_state, float* out, int32_t* out_len, float* labels,
+                               uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Streaming form of rb_process_host_seeded: queues the whole call and returns at once; *ticket identifies it. Up to two calls
  * may be in flight (a third submit first waits for the oldest), so the copies of consecutive batches follow each other
  * without a gap and steady-state throughput is bound by PCIe alone. x, len, seeds and y must stay valid -- and y must not

@@ -21,7 +21,7 @@ SYMBOLS = (
     "rb_planner_draw", "rb_devplan_bytes", "rb_devplan_draw", "rb_process_host_seeded",
     "rb_ctx_set_chunk", "rb_ctx_set_plan_mode", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
     "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
-    "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run",
+    "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run", "rb_items_stream_draw", "rb_items_stream_run",
 )
 RB_IO_HOST_F32, RB_IO_HOST_PCM16, RB_IO_DEVICE_F32 = 0, 1, 2
 
@@ -165,6 +165,12 @@ def load() -> C.CDLL:
                                   C.POINTER(RbPlan), vp]
     lib.rb_items_run.restype = i32
     lib.rb_items_run.argtypes = [C.POINTER(RbArgs), i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    lib.rb_items_stream_draw.restype = i32
+    lib.rb_items_stream_draw.argtypes = [C.POINTER(RbArgs), i32, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, sz,
+                                         C.POINTER(RbPlan), vp]
+    lib.rb_items_stream_run.restype = i32
+    lib.rb_items_stream_run.argtypes = [C.POINTER(RbArgs), i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp,
+                                        vp, vp, sz, vp]
     if lib.rb_abi_version() != RB_ABI_VERSION:
         raise RawBoostLibraryError(f"ABI mismatch: library {lib.rb_abi_version()}, binding {RB_ABI_VERSION}; rebuild")
     _lib = lib

@@ -1,21 +1,25 @@
-// rb_items.cu -- whole Dataset_for items (asvspoof_2019_augall_3.py:103-146, RawBoost12 with online_aug) for a batch of items
-// that are each seeded on their own: np.random.seed(seeds[g]) before item g, as a reproducible loader does per __getitem__.
+// rb_items.cu -- whole Dataset_for items (asvspoof_2019_augall_3.py:103-146, RawBoost12 with online_aug) for a batch of items,
+// either each seeded on its own (np.random.seed(seeds[g]) before item g, as a reproducible loader does per __getitem__) or
+// sharing numpy's running stream (__getitem__ called for them one after another with no seed in between, as the reference's
+// loader does).
 //
-// Item g consumes ONE stream, in this order: RawBoost (algo 5) on every vocoded copy in vocoder order, then on the anchor --
+// Item g consumes its stream in this order: RawBoost (algo 5) on every vocoded copy in vocoder order, then on the anchor --
 // each of them N_f LnL parameter sets, ISD beta, permutation(L), rand(n) twice -- then np.random.choice(others, n_add,
 // replace=False), which legacy numpy computes as permutation(N-1)[:n_add] mapped through `others` (v -> v + (v >= idx)),
-// then the shared crop int(rand() * (L_anchor - trim)), drawn only when L_anchor >= trim. Different items are independent,
-// so they run in parallel; only the draws inside one item share a stream.
+// then the shared crop int(rand() * (L_anchor - trim)), drawn only when L_anchor >= trim.
 //
 // Two passes:
-//   items_walk_kernel    one warp per item: seeds the stream and walks the whole item, counting words only (the shuffles
-//                        with the ballot fix-point of shuffle_walk_warp). It stores a snapshot of the stream (numpy's state
-//                        form) at the start of every RawBoost utterance and of the choice, and draws the crop start.
+//   the walk             walk_item below, for one item on one warp: counts the item's words only (the shuffles with the ballot
+//                        fix-point of shuffle_walk_warp), stores a snapshot of the stream (numpy's state form) at the start of
+//                        every RawBoost utterance and of the choice, and draws the crop start. Two kernels run it:
+//     items_walk_kernel         one warp per seeded item: seeds the stream, walks the item
+//     items_stream_walk_kernel  one warp per running stream: loads the stream's state, walks its items in order, item k+1
+//                               starting where item k ended, and stores the final state
 //   then the per-utterance planner (rb_devplan.cu) runs unchanged over the G*(nvoc+1) utterances from their snapshots, and
 //   shuffle_prefix applies the choice permutations.
 //   items_rows_kernel    the batch's source rows in the corpus, their lengths, the view table of the assembly, the label vector
-//   items_gather_kernel  one CTA per batch row: corpus row -> batch row (rb_items_run only)
-// rb_items_run then finishes with rb_process(5) and rb_multiview_assemble_ex, exactly as ItemBatcher does.
+//   items_gather_kernel  one CTA per batch row: corpus row -> batch row (rb_items_run / rb_items_stream_run only)
+// The run entries then finish with rb_process(5) and rb_multiview_assemble_ex, exactly as ItemBatcher does.
 //
 // Corpus layout: rows [R, ld], R = N * (1 + nvoc); row idx is bona fide utterance idx, row N + idx*nvoc + v is vocoder v's copy.
 // Batch layout (ItemBatcher's): rows g*(nvoc+1) + v hold item g's vocoded copies (v < nvoc) and its anchor (v = nvoc); rows
@@ -35,20 +39,14 @@ constexpr int kWalkWarps = 4;  // 30 KB of MT19937 state per CTA, as plan_body_k
 
 __device__ __forceinline__ int clamp_index(int idx, int N) { return (idx >= 0 && idx < N) ? idx : 0; }
 
-__global__ void __launch_bounds__(32 * kWalkWarps)
-items_walk_kernel(rb_args a, int G, int nvoc, int n_add, int N, int trim, const int32_t* __restrict__ corpus_len,
-                  const int32_t* __restrict__ indices, const uint32_t* __restrict__ seeds, uint32_t* __restrict__ snaps,
-                  uint32_t* __restrict__ csnaps, int32_t* __restrict__ start, uint32_t* __restrict__ end_state,
-                  int32_t* __restrict__ choice_len, int32_t* __restrict__ choice_off) {
-  __shared__ MtSmem sm[kWalkWarps];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int g = blockIdx.x * kWalkWarps + warp;
-  if (g >= G) return;
+// Every draw of item g from the warp's stream `s`, which stands at the item's first word: the utterance snapshots, the choice
+// snapshot, choice_len / choice_off and the crop start. Leaves `s` after the item's last word.
+__device__ __forceinline__ void walk_item(const rb_args& a, MtStream& s, int g, int G, int nvoc, int n_add, int N, int trim,
+                                          const int32_t* __restrict__ corpus_len, const int32_t* __restrict__ indices,
+                                          uint32_t* __restrict__ snaps, uint32_t* __restrict__ csnaps, int32_t* __restrict__ start,
+                                          int32_t* __restrict__ choice_len, int32_t* __restrict__ choice_off, int lane) {
   const int idx = clamp_index(indices[g], N);
   const int U = nvoc + 1;
-  MtStream s;
-  s.sm = &sm[warp];
-  s.seed(seeds[g], lane);
   const int lnl_words = a.N_f * 2 * filter_stride(a.nBands);
   for (int v = 0; v < U; ++v) {
     const int L = corpus_len[v < nvoc ? N + idx * nvoc + v : idx];
@@ -68,13 +66,52 @@ items_walk_kernel(rb_args a, int G, int nvoc, int n_add, int N, int trim, const 
     st = (int)__dmul_rn(mt_double(s.word(0), s.word(1)), (double)(La - trim));
     s.advance(2, lane);
   }
-  if (end_state) s.store(end_state + (size_t)g * kMtSnapWords, lane);
   if (lane == 0) {
     start[g] = st;
     choice_len[g] = N - 1;
     choice_off[g] = g * n_add;
     if (g == G - 1) choice_off[G] = G * n_add;
   }
+}
+
+__global__ void __launch_bounds__(32 * kWalkWarps)
+items_walk_kernel(rb_args a, int G, int nvoc, int n_add, int N, int trim, const int32_t* __restrict__ corpus_len,
+                  const int32_t* __restrict__ indices, const uint32_t* __restrict__ seeds, uint32_t* __restrict__ snaps,
+                  uint32_t* __restrict__ csnaps, int32_t* __restrict__ start, uint32_t* __restrict__ end_state,
+                  int32_t* __restrict__ choice_len, int32_t* __restrict__ choice_off) {
+  __shared__ MtSmem sm[kWalkWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = blockIdx.x * kWalkWarps + warp;
+  if (g >= G) return;
+  MtStream s;
+  s.sm = &sm[warp];
+  s.seed(seeds[g], lane);
+  walk_item(a, s, g, G, nvoc, n_add, N, trim, corpus_len, indices, snaps, csnaps, start, choice_len, choice_off, lane);
+  if (end_state) s.store(end_state + (size_t)g * kMtSnapWords, lane);
+}
+
+// One warp per running stream, one stream per CTA so that few streams spread over as many SMs. Stream q walks the items
+// [stream_off[q], stream_off[q+1]). The table is device data the host cannot check, so it is read defensively: every offset is
+// clamped to [0, G], a decreasing step gives an empty stream, and the first stream starts at 0 and the last ends at G whatever
+// the table says. Every item then belongs to at least one stream, so every output is written and stays in bounds; with a
+// malformed table the items' values are unspecified (two streams that overlap both write the items they share).
+// MtStream::load clamps the start states' pos.
+__global__ void __launch_bounds__(32)
+items_stream_walk_kernel(rb_args a, int S, const int32_t* __restrict__ stream_off, int G, int nvoc, int n_add, int N, int trim,
+                         const int32_t* __restrict__ corpus_len, const int32_t* __restrict__ indices,
+                         const uint32_t* __restrict__ start_state, uint32_t* __restrict__ snaps, uint32_t* __restrict__ csnaps,
+                         int32_t* __restrict__ start, uint32_t* __restrict__ end_state, int32_t* __restrict__ choice_len,
+                         int32_t* __restrict__ choice_off) {
+  __shared__ MtSmem sm;
+  const int q = blockIdx.x, lane = threadIdx.x;
+  const int lo = q == 0 ? 0 : min(max(stream_off[q], 0), G);
+  const int hi = q == S - 1 ? G : max(lo, min(stream_off[q + 1], G));
+  MtStream s;
+  s.sm = &sm;
+  s.load(start_state + (size_t)q * kMtSnapWords, lane);
+  for (int g = lo; g < hi; ++g)
+    walk_item(a, s, g, G, nvoc, n_add, N, trim, corpus_len, indices, snaps, csnaps, start, choice_len, choice_off, lane);
+  if (end_state) s.store(end_state + (size_t)q * kMtSnapWords, lane);
 }
 
 __global__ void __launch_bounds__(256)
@@ -181,30 +218,92 @@ int check_workspace(const void* ws, size_t have, size_t need) {
   return have < need ? RB_ERR_WORKSPACE : RB_OK;
 }
 
+// Where the items' streams start: item g seeded with seeds[g] (end_state per item), or S running streams (end_state per
+// stream): the items of stream q are [stream_off[q], stream_off[q+1]), its state before the first of them start_state[q].
+struct WalkSource {
+  bool seeded;
+  const uint32_t* seeds;
+  int S;
+  const int32_t* stream_off;
+  const uint32_t* start_state;
+
+  // checked before G == 0 returns: S >= 0, and at least one stream when there are items
+  bool shape_ok(int G) const { return seeded || (S >= 0 && (S > 0 || G == 0)); }
+  bool pointers_ok() const { return seeded ? seeds != nullptr : (stream_off && start_state); }
+};
+
 // every draw of the batch: snapshots, crop starts, choice, row tables, plan
 int items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
-               const int32_t* indices, const uint32_t* seeds, int32_t* src_row, int32_t* row_len, int32_t* start,
+               const int32_t* indices, const WalkSource& src, int32_t* src_row, int32_t* row_len, int32_t* start,
                uint32_t* end_state, char* d, const ItemsLayout& l, rb_plan* plan, cudaStream_t st) {
   const int nb = G * (nvoc + 1);
-  items_walk_kernel<<<(G + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, st>>>(
-      *args, G, nvoc, n_add, N, trim, corpus_len, indices, seeds, (uint32_t*)(d + l.snaps), (uint32_t*)(d + l.csnaps), start,
-      end_state, (int32_t*)(d + l.clen), (int32_t*)(d + l.coff));
+  uint32_t *snaps = (uint32_t*)(d + l.snaps), *csnaps = (uint32_t*)(d + l.csnaps);
+  int32_t *clen = (int32_t*)(d + l.clen), *coff = (int32_t*)(d + l.coff);
+  if (src.seeded)
+    items_walk_kernel<<<(G + kWalkWarps - 1) / kWalkWarps, 32 * kWalkWarps, 0, st>>>(
+        *args, G, nvoc, n_add, N, trim, corpus_len, indices, src.seeds, snaps, csnaps, start, end_state, clen, coff);
+  else
+    items_stream_walk_kernel<<<src.S, 32, 0, st>>>(*args, src.S, src.stream_off, G, nvoc, n_add, N, trim, corpus_len, indices,
+                                                   src.start_state, snaps, csnaps, start, end_state, clen, coff);
   RB_LAUNCH_CHECK();
   int rc;
-  if (n_add > 0 && (rc = shuffle_prefix(G, N - 1, (const int32_t*)(d + l.clen), (const uint32_t*)(d + l.csnaps),
-                                        (const int32_t*)(d + l.coff), (int32_t*)(d + l.cpos), d + l.shuffle, st)) != RB_OK)
+  if (n_add > 0 && (rc = shuffle_prefix(G, N - 1, clen, csnaps, coff, (int32_t*)(d + l.cpos), d + l.shuffle, st)) != RB_OK)
     return rc;
   const size_t work = (size_t)G * (nvoc + 1 + n_add) + (size_t)G * (2 + n_add + 2 * nvoc);
   const int grid = (int)std::min<size_t>((work + 255) / 256, 148 * 8);
   items_rows_kernel<<<grid, 256, 0, st>>>(G, nvoc, n_add, N, corpus_len, indices, (const int32_t*)(d + l.cpos), src_row, row_len,
                                          (int32_t*)(d + l.view_row), (float*)(d + l.view_label));
   RB_LAUNCH_CHECK();
-  const uint32_t* snaps = (const uint32_t*)(d + l.snaps);
   void* pm = d + l.plan;
   if ((rc = devplan_begin(args, 5, nb, ld, row_len, nullptr, pm, l.plan_bytes, plan, st, snaps)) != RB_OK) return rc;
   if ((rc = devplan_body(args, 5, nb, ld, row_len, nullptr, pm, 0, nb, st, snaps)) != RB_OK) return rc;
   if ((rc = devplan_apply(args, 5, nb, ld, row_len, pm, 0, nb, st)) != RB_OK) return rc;
   return devplan_end(args, 5, nb, ld, pm, st);
+}
+
+int draw_entry(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
+               const int32_t* indices, const WalkSource& src, int32_t* src_row, int32_t* row_len, int32_t* start,
+               uint32_t* end_state, void* workspace, size_t workspace_bytes, rb_plan* plan, void* stream) {
+  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
+  if (rc != RB_OK) return rc;
+  if (!plan) return RB_ERR_INVALID_ARG;
+  memset(plan, 0, sizeof(*plan));
+  if (!src.shape_ok(G)) return RB_ERR_INVALID_ARG;
+  if (G == 0) return RB_OK;
+  if (!corpus_len || !indices || !src.pointers_ok() || !src_row || !row_len || !start) return RB_ERR_INVALID_ARG;
+  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
+  if ((rc = check_workspace(workspace, workspace_bytes, l.draw_bytes)) != RB_OK) return rc;
+  return items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, src, src_row, row_len, start, end_state,
+                    (char*)workspace, l, plan, (cudaStream_t)stream);
+}
+
+int run_entry(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
+              const float* corpus, const int32_t* corpus_len, const int32_t* indices, const WalkSource& src, float* out,
+              int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
+  if (rc != RB_OK) return rc;
+  const int V = 2 + n_add + 2 * nvoc;
+  if ((layout != 0 && layout != 1) || (labels && V > 256)) return RB_ERR_INVALID_ARG;
+  if (!src.shape_ok(G)) return RB_ERR_INVALID_ARG;
+  if (G == 0) return RB_OK;
+  if (!corpus || !corpus_len || !indices || !src.pointers_ok() || !out) return RB_ERR_INVALID_ARG;
+  if ((uintptr_t)corpus & 15u) return RB_ERR_ALIGNMENT;
+  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
+  if ((rc = check_workspace(workspace, workspace_bytes, l.bytes)) != RB_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  char* d = (char*)workspace;
+  int32_t *src_row = (int32_t*)(d + l.src_row), *row_len = (int32_t*)(d + l.row_len), *start = (int32_t*)(d + l.start);
+  rb_plan plan;
+  if ((rc = items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, src, src_row, row_len, start, end_state, d, l,
+                       &plan, st)) != RB_OK)
+    return rc;
+  const int rows = G * (nvoc + 1 + n_add), nb = G * (nvoc + 1);
+  float *x = (float*)(d + l.x), *y = (float*)(d + l.y);
+  items_gather_kernel<<<rows, 256, 0, st>>>(corpus, ld, src_row, row_len, x);
+  RB_LAUNCH_CHECK();
+  if ((rc = rb_process(5, x, row_len, nb, ld, &plan, y, d + l.proc, l.proc_bytes, stream)) != RB_OK) return rc;
+  return rb_multiview_assemble_ex(x, y, (const int32_t*)(d + l.view_row), row_len, G, V, ld, start, trim, repeat_pad, layout, out,
+                                  out_len, labels ? (const float*)(d + l.view_label) : nullptr, labels, stream);
 }
 
 }  // namespace
@@ -222,44 +321,31 @@ size_t rb_items_workspace_bytes(const rb_args* args, int G, int nvoc, int n_add,
 int rb_items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, const int32_t* corpus_len,
                   const int32_t* indices, const uint32_t* seeds, int32_t* src_row, int32_t* row_len, int32_t* start,
                   uint32_t* end_state, void* workspace, size_t workspace_bytes, rb_plan* plan, void* stream) {
-  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
-  if (rc != RB_OK) return rc;
-  if (!plan) return RB_ERR_INVALID_ARG;
-  memset(plan, 0, sizeof(*plan));
-  if (G == 0) return RB_OK;
-  if (!corpus_len || !indices || !seeds || !src_row || !row_len || !start) return RB_ERR_INVALID_ARG;
-  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
-  if ((rc = check_workspace(workspace, workspace_bytes, l.draw_bytes)) != RB_OK) return rc;
-  return items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, seeds, src_row, row_len, start, end_state,
-                    (char*)workspace, l, plan, (cudaStream_t)stream);
+  return draw_entry(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, {true, seeds, 0, nullptr, nullptr}, src_row, row_len,
+                    start, end_state, workspace, workspace_bytes, plan, stream);
 }
 
 int rb_items_run(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
                  const float* corpus, const int32_t* corpus_len, const int32_t* indices, const uint32_t* seeds, float* out,
                  int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
-  int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
-  if (rc != RB_OK) return rc;
-  const int V = 2 + n_add + 2 * nvoc;
-  if ((layout != 0 && layout != 1) || (labels && V > 256)) return RB_ERR_INVALID_ARG;
-  if (G == 0) return RB_OK;
-  if (!corpus || !corpus_len || !indices || !seeds || !out) return RB_ERR_INVALID_ARG;
-  if ((uintptr_t)corpus & 15u) return RB_ERR_ALIGNMENT;
-  const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
-  if ((rc = check_workspace(workspace, workspace_bytes, l.bytes)) != RB_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  char* d = (char*)workspace;
-  int32_t *src_row = (int32_t*)(d + l.src_row), *row_len = (int32_t*)(d + l.row_len), *start = (int32_t*)(d + l.start);
-  rb_plan plan;
-  if ((rc = items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, seeds, src_row, row_len, start, end_state, d, l,
-                       &plan, st)) != RB_OK)
-    return rc;
-  const int rows = G * (nvoc + 1 + n_add), nb = G * (nvoc + 1);
-  float *x = (float*)(d + l.x), *y = (float*)(d + l.y);
-  items_gather_kernel<<<rows, 256, 0, st>>>(corpus, ld, src_row, row_len, x);
-  RB_LAUNCH_CHECK();
-  if ((rc = rb_process(5, x, row_len, nb, ld, &plan, y, d + l.proc, l.proc_bytes, stream)) != RB_OK) return rc;
-  return rb_multiview_assemble_ex(x, y, (const int32_t*)(d + l.view_row), row_len, G, V, ld, start, trim, repeat_pad, layout, out,
-                                  out_len, labels ? (const float*)(d + l.view_label) : nullptr, labels, stream);
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, corpus, corpus_len, indices, {true, seeds, 0, nullptr, nullptr},
+                   out, out_len, labels, end_state, workspace, workspace_bytes, stream);
+}
+
+int rb_items_stream_draw(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld, int trim,
+                         const int32_t* corpus_len, const int32_t* indices, const uint32_t* start_state, int32_t* src_row,
+                         int32_t* row_len, int32_t* start, uint32_t* end_state, void* workspace, size_t workspace_bytes, rb_plan* plan,
+                         void* stream) {
+  return draw_entry(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, {false, nullptr, S, stream_off, start_state}, src_row,
+                    row_len, start, end_state, workspace, workspace_bytes, plan, stream);
+}
+
+int rb_items_stream_run(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld, int trim,
+                        int repeat_pad, int layout, const float* corpus, const int32_t* corpus_len, const int32_t* indices,
+                        const uint32_t* start_state, float* out, int32_t* out_len, float* labels, uint32_t* end_state, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, corpus, corpus_len, indices,
+                   {false, nullptr, S, stream_off, start_state}, out, out_len, labels, end_state, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -119,10 +119,10 @@ struct MtStream {
     pos = 0;
   }
   // start from a snapshot in numpy's form: temper key into the current block (twisting first when pos == 624), then twist
-  // once more for the next block
+  // once more for the next block. pos is clamped to 0..624, so that a malformed snapshot cannot address outside the blocks.
   __device__ void load(const uint32_t* __restrict__ snap, int lane) {
     for (int i = lane; i < kMtN; i += 32) sm->key[i] = snap[i];
-    const int p = (int)snap[kMtN];
+    const int p = min(max((int)snap[kMtN], 0), kMtN);
     __syncwarp();
     if (p >= kMtN) {
       mt_next_block(sm->key, sm->blk[0], lane);
@@ -179,6 +179,9 @@ __device__ __forceinline__ int filter_stride(int nBands) { return 3 * nBands + 1
 // ballot fix-point settles lane t after at most t+1 iterations (lane 0 is exact at once), in practice after two. Accepted lanes
 // are the consecutive steps i, i-1, ...; with kRecord their targets go to jseq[step], step = L-1-i. Without it the walk only
 // consumes the words.
+// Fast round: a word with v > i is rejected and one with v <= i - 31 accepted whatever A (A <= 31), so when no word lies in
+// between, the first ballot is exact; when moreover at least 32 steps are left under the mask, all 32 words are consumed. For
+// large masks that is almost every round, and it takes the fix-point's and the region's ballots off the round's critical path.
 template <bool kRecord, typename JT>
 __device__ __forceinline__ void shuffle_walk_warp(MtStream& s, int L, JT* __restrict__ jseq, int lane) {
   const uint32_t lt = (1u << lane) - 1u;
@@ -194,6 +197,13 @@ __device__ __forceinline__ void shuffle_walk_warp(MtStream& s, int L, JT* __rest
     while (i >= lo) {
       const int v = (int)(s.word(lane) & mask);
       uint32_t acc = __ballot_sync(kFull, v <= i);
+      const uint32_t unsure = __ballot_sync(kFull, v <= i && v > i - 31);
+      if (unsure == 0 && i - lo + 1 >= 32) {
+        if (kRecord && ((acc >> lane) & 1u)) jseq[(L - 1) - (i - __popc(acc & lt))] = (JT)v;
+        i -= __popc(acc);
+        s.advance(32, lane);
+        continue;
+      }
       int A;
       for (;;) {
         A = __popc(acc & lt);

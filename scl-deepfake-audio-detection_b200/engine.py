@@ -210,6 +210,106 @@ class Engine:
         _lib.check(rc, "rb_items_run")
         return out, out_len, labels
 
+    def _stream_arrays(self, indices, stream_off, start_state):
+        """indices, stream_off and start_state as 32-bit device tensors (start_state [S, 625] holds the uint32 bit patterns of
+        numpy's key[624], pos)."""
+        if not torch.is_tensor(indices):
+            indices = torch.from_numpy(np.ascontiguousarray(indices, dtype=np.int32)).to(self.device)
+        if not torch.is_tensor(stream_off):
+            stream_off = torch.from_numpy(np.ascontiguousarray(stream_off, dtype=np.int32)).to(self.device)
+        if not torch.is_tensor(start_state):
+            host = np.asarray(start_state, dtype=np.int64).reshape(-1, 625).astype(np.uint32)
+            start_state = torch.from_numpy(np.ascontiguousarray(host).view(np.int32)).to(self.device)
+        for name, t, dim, dtypes in (("indices", indices, 1, (torch.int32,)), ("stream_off", stream_off, 1, (torch.int32,)),
+                                     ("start_state", start_state, 2, (torch.int32, torch.uint32))):
+            if t.device != self.device or t.dtype not in dtypes or t.dim() != dim or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous {dim}-D {' or '.join(map(str, dtypes))} tensor on {self.device}")
+        S = int(stream_off.numel()) - 1
+        if S < 0 or start_state.shape != (S, 625):
+            raise ValueError("stream_off needs S+1 entries and start_state S rows of 625 words")
+        return indices, stream_off, start_state, S
+
+    def _stream_end(self, S: int, end_state):
+        if end_state is None or torch.is_tensor(end_state):
+            if end_state is not None and (end_state.shape != (S, 625) or end_state.dtype not in (torch.int32, torch.uint32)
+                                          or end_state.device != self.device
+                                          or not end_state.is_contiguous()):
+                raise ValueError("end_state must be a contiguous 32-bit [S, 625] tensor on the engine's device")
+            return end_state
+        return torch.empty((S, 625), dtype=torch.int32, device=self.device) if end_state else None
+
+    def items_stream_draw(self, args, sr, corpus_len: torch.Tensor, nvoc: int, n_add: int, ld: int, trim: int, indices, stream_off,
+                          start_state, end_state=False):
+        """:meth:`items_draw` for items that share running numpy streams (``rb_items_stream_draw``; see
+        ``multiview.StreamItemBatcher``): stream q walks the items ``[stream_off[q], stream_off[q+1])`` of ``indices`` in order,
+        from ``start_state[q]`` (numpy's key[624], pos). ``stream_off`` ([S+1]) and ``start_state`` ([S, 625]) are host arrays or
+        32-bit device tensors. ``end_state``: True (a new tensor) or an int32 [S, 625] device tensor that receives each stream's
+        state after its last draw. Returns the dict of :meth:`items_draw`; its ``end_state`` is per stream. Asynchronous on torch's
+        current stream; with device inputs nothing synchronises with the host."""
+        indices, stream_off, start_state, S = self._stream_arrays(indices, stream_off, start_state)
+        end = self._stream_end(S, end_state)
+        G, R = int(indices.numel()), int(corpus_len.numel())
+        if corpus_len.dtype != torch.int32 or corpus_len.device != self.device or R % (1 + nvoc):
+            raise ValueError("corpus_len must be int32 [N*(1+nvoc)] on the engine's device")
+        N = R // (1 + nvoc)
+        a = _lib.args_struct(args, sr)
+        need = int(self.lib.rb_items_workspace_bytes(C.byref(a), G, int(nvoc), int(n_add), N, int(ld)))
+        if G and need == 0:
+            raise ValueError(f"unsupported item shape: G={G}, nvoc={nvoc}, n_add={n_add}, N={N}, ld={ld}")
+        store = torch.empty(need + 256, dtype=torch.uint8, device=self.device)
+        rows = G * (nvoc + 1 + n_add)
+        src_row = torch.empty(rows, dtype=torch.int32, device=self.device)
+        row_len = torch.empty(rows, dtype=torch.int32, device=self.device)
+        start = torch.empty(G, dtype=torch.int32, device=self.device)
+        s = _lib.RbPlan()
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_stream_draw(C.byref(a), S, _ptr(stream_off), G, int(nvoc), int(n_add), N, int(ld), int(trim),
+                                               _ptr(corpus_len), _ptr(indices), _ptr(start_state), _ptr(src_row), _ptr(row_len),
+                                               _ptr(start), _ptr(end), C.c_void_p(self._ws_ptr(store)), need, C.byref(s),
+                                               C.c_void_p(stream))
+        _lib.check(rc, "rb_items_stream_draw")
+        B = G * (nvoc + 1)
+        plan = DevicePlan(B=B, ld=int(ld), lengths=row_len[:B], tensors={"storage": store}, struct=s, host=None)
+        return {"plan": plan, "src_row": src_row, "row_len": row_len, "start": start, "end_state": end}
+
+    def items_stream_run(self, args, sr, corpus: torch.Tensor, corpus_len: torch.Tensor, nvoc: int, n_add: int, trim: int, indices,
+                         stream_off, start_state, repeat_pad: bool = True, layout: int = 0, out: Optional[torch.Tensor] = None,
+                         with_labels: bool = True, end_state=None):
+        """:meth:`items_run` for items that share running numpy streams (``rb_items_stream_run``): ``stream_off``,
+        ``start_state`` and ``end_state`` as :meth:`items_stream_draw`. Returns ``(out, out_len, labels)`` as :meth:`items_run`.
+        Asynchronous on torch's current stream; with device inputs nothing synchronises with the host."""
+        indices, stream_off, start_state, S = self._stream_arrays(indices, stream_off, start_state)
+        if end_state is not None and not torch.is_tensor(end_state):
+            raise ValueError("end_state must be None or an int32 [S, 625] device tensor")
+        end = self._stream_end(S, end_state)
+        if corpus.dtype != torch.float32 or corpus.dim() != 2 or not corpus.is_contiguous() or corpus.device != self.device:
+            raise ValueError("corpus must be a contiguous [R, ld] float32 tensor on the engine's device")
+        R, ld = corpus.shape
+        if corpus_len.dtype != torch.int32 or corpus_len.device != self.device or corpus_len.numel() != R or R % (1 + nvoc):
+            raise ValueError("corpus_len must be int32 [R] on the engine's device, R = N*(1+nvoc)")
+        N, G, V = R // (1 + nvoc), int(indices.numel()), 2 + n_add + 2 * nvoc
+        shape = (G, trim, V) if layout == 0 else (G, V, trim)
+        if out is None:
+            out = torch.zeros(shape, dtype=torch.float32, device=self.device)
+        elif tuple(out.shape) != shape or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 tensor {shape} on the engine's device")
+        out_len = torch.empty(G, dtype=torch.int32, device=self.device)
+        labels = torch.empty((G, V), dtype=torch.float32, device=self.device) if with_labels else None
+        a = _lib.args_struct(args, sr)
+        need = int(self.lib.rb_items_workspace_bytes(C.byref(a), G, int(nvoc), int(n_add), N, int(ld)))
+        if G and need == 0:
+            raise ValueError(f"unsupported item shape: G={G}, nvoc={nvoc}, n_add={n_add}, N={N}, ld={ld}")
+        ws = self._scratch(need)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_stream_run(C.byref(a), S, _ptr(stream_off), G, int(nvoc), int(n_add), N, int(ld), int(trim),
+                                              int(bool(repeat_pad)), int(layout), _ptr(corpus), _ptr(corpus_len), _ptr(indices),
+                                              _ptr(start_state), _ptr(out), _ptr(out_len), _ptr(labels), _ptr(end),
+                                              C.c_void_p(self._ws_ptr(ws)), need, C.c_void_p(stream))
+        _lib.check(rc, "rb_items_stream_run")
+        return out, out_len, labels
+
     def pack_waveforms(self, waves: Sequence[np.ndarray], ld: Optional[int] = None):
         """Host list of 1-D float arrays -> ([B, ld] float32 device tensor, int32 lengths on device)."""
         lengths = np.array([int(w.shape[0]) for w in waves], dtype=np.int32)

@@ -13,6 +13,8 @@
 * :class:`ItemBatcher` -- whole ``Dataset_for`` items, every draw on the host from the global numpy stream.
 * :class:`DeviceCorpus` + :class:`SeededItemBatcher` -- whole items seeded one by one (``np.random.seed(s)`` before each
   ``__getitem__``), every draw replayed on the device from a corpus that lives there.
+* :class:`StreamItemBatcher` -- the same for items that share numpy's running stream, one after another, as
+  :class:`ItemBatcher` draws them.
 
 Integer work (crop start, index map) is bit-exact; the samples are copies of the views' float32 values.
 """
@@ -328,6 +330,104 @@ class SeededItemBatcher:
         c = self.corpus
         return c.eng.items_draw(self.args, self.sr, c.lengths, c.nvoc, self.num_additional_real, c.ld, self.trim_length, idx, seeds,
                                 end_state=end_state)
+
+
+def numpy_state(row) -> tuple:
+    """A stream state of the device paths (625 32-bit words: key[624], pos) as the tuple ``np.random.set_state`` takes."""
+    w = np.asarray(row.cpu().numpy() if torch.is_tensor(row) else row).astype(np.int64).astype(np.uint32)
+    return ("MT19937", w[:624].copy(), int(w[624]), 0, 0.0)
+
+
+def _state_words(state) -> np.ndarray:
+    """numpy's state tuple (``np.random.get_state()``) -> its 625 words key[624], pos; ValueError if it is not one."""
+    if not isinstance(state, (tuple, list)) or len(state) < 3 or state[0] != "MT19937":
+        raise ValueError("a stream state must be an MT19937 state tuple, as np.random.get_state() returns")
+    key = np.asarray(state[1])
+    if key.shape != (624,) or not np.issubdtype(key.dtype, np.integer) or key.min() < 0 or key.max() > 0xFFFFFFFF:
+        raise ValueError("an MT19937 state needs a key of 624 32-bit words")
+    pos = int(state[2])
+    if not 0 <= pos <= 624:
+        raise ValueError(f"an MT19937 state's pos must lie in 0..624, not {pos}")
+    return np.append(key.astype(np.uint32), np.uint32(pos))
+
+
+class StreamItemBatcher:
+    """``Dataset_for.__getitem__`` (asvspoof_2019_augall_3.py:103-146, ``augmentation_methods == ['RawBoost12']`` with
+    ``online_aug``) for items that share numpy's running stream, as the reference's loader builds them with no per-item seed:
+
+        for idx in indices: __getitem__(idx)     # every draw from numpy's global stream, item after item
+
+    Every draw is replayed on the device from the stream's state (``rb_items_stream_run``): one warp walks the stream's items in
+    order, then the plans, the RawBoost of all items and the assembly run as a batch, as in :class:`SeededItemBatcher`. The walk
+    of one stream is serial, so its time grows with the number of items in it; several independent streams (one per loader
+    worker, say) walk in parallel.
+
+    The item draws never use numpy's Gaussian cache, so ``has_gauss`` / ``cached_gaussian`` of the global state carry over."""
+
+    def __init__(self, args, corpus: DeviceCorpus, num_additional_real=2, trim_length=64000, repeat_pad=True, wav_samp_rate=16000):
+        self.args, self.corpus = args, corpus
+        self.num_additional_real, self.trim_length = int(num_additional_real), int(trim_length)
+        self.repeat_pad, self.sr = bool(repeat_pad), int(wav_samp_rate)
+        if not 0 <= self.num_additional_real <= corpus.N - 1:
+            raise ValueError(f"num_additional_real must lie in [0, {corpus.N - 1}] for a corpus of {corpus.N} utterances")
+
+    def _indices(self, indices) -> np.ndarray:
+        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= self.corpus.N):
+            raise IndexError(f"indices must lie in [0, {self.corpus.N})")
+        return idx
+
+    def _run(self, idx, stream_off, states, layout, end):
+        c = self.corpus
+        data, out_len, labels = c.eng.items_stream_run(self.args, self.sr, c.data, c.lengths, c.nvoc, self.num_additional_real,
+                                                       self.trim_length, idx.astype(np.int32), stream_off, states, self.repeat_pad,
+                                                       layout, end_state=end)
+        return [c.list_ids[i] for i in idx], data, labels, out_len
+
+    def items(self, indices: Sequence[int], layout: int = LAYOUT_ITEM):
+        """Drop-in for :meth:`ItemBatcher.items`: ``(ids, data, labels, out_len)`` for ``indices`` drawn from numpy's global
+        stream, which afterwards stands exactly where ``for idx in indices: __getitem__(idx)`` leaves it. Synchronises once, to
+        read back the stream's end state."""
+        idx = self._indices(indices)
+        state = np.random.get_state()
+        words = _state_words(state)[None]
+        if idx.size == 0:  # nothing is drawn
+            return self._run(idx, [0, 0], words, layout, None)
+        end = torch.empty((1, 625), dtype=torch.int32, device=self.corpus.eng.device)
+        out = self._run(idx, [0, idx.size], words, layout, end)
+        e = numpy_state(end[0])
+        np.random.set_state(e[:3] + tuple(state[3:5]))
+        return out
+
+    def items_streams(self, index_lists: Sequence[Sequence[int]], states, layout: int = LAYOUT_ITEM):
+        """S independent streams, e.g. one per loader worker: the items of ``index_lists[q]`` are drawn one after another from
+        ``states[q]`` -- numpy state tuples, or an int32 [S, 625] device tensor of key[624], pos as the end states below.
+        Returns ``(ids, data, labels, out_len, end_states)``: the items in stream order (stream 0's, then stream 1's, ...) as
+        :meth:`items` returns them, and int32 [S, 625] device tensor of each stream's state after its last draw
+        (:func:`numpy_state` turns a row into a tuple for ``np.random.set_state``). numpy's global stream is not touched, and
+        nothing is read back from the device.
+
+        End states are stored with pos 0..623: a used-up block (pos 624, as right after ``np.random.seed``) comes back as the
+        next block at pos 0, also for an empty stream. The one exception is a call with no item at all: nothing is launched and
+        the end states are the start states exactly as given, so a pos of 624 stays 624. Both forms continue the same stream."""
+        lists = [self._indices(ix) for ix in index_lists]
+        S = len(lists)
+        if torch.is_tensor(states):
+            if states.dtype not in (torch.int32, torch.uint32) or tuple(states.shape) != (S, 625):
+                raise ValueError(f"states must be an int32 (or uint32) [S, 625] tensor with S = {S}")
+        else:
+            states = list(states)
+            if len(states) != S:
+                raise ValueError("one state per index list")
+            states = np.stack([_state_words(s) for s in states]) if S else np.zeros((0, 625), np.uint32)
+        idx = np.concatenate(lists) if S else np.zeros(0, np.int64)
+        stream_off = np.concatenate([[0], np.cumsum([ix.size for ix in lists])]).astype(np.int32)
+        dev = self.corpus.eng.device
+        if idx.size == 0:  # nothing is drawn: every stream ends where it starts
+            end = states.clone() if torch.is_tensor(states) else torch.from_numpy(states.view(np.int32)).to(dev)
+            return (*self._run(idx, stream_off, states, layout, None), end)
+        end = torch.empty((S, 625), dtype=torch.int32, device=dev)
+        return (*self._run(idx, stream_off, states, layout, end), end)
 
 
 def _repad(bp, ld):
