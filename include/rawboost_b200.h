@@ -141,9 +141,6 @@ typedef struct rb_ctx rb_ctx;
 RB_API int rb_ctx_create(rb_ctx** out, int device);
 RB_API int rb_ctx_destroy(rb_ctx* ctx);
 RB_API int rb_ctx_set_chunk(rb_ctx* ctx, int utterances /* 0 = default */);
-/* rb_process_host_seeded: 0 (default) = the device planner runs on its own streams beside the kernels; 1 = in line on the
- * kernels' stream (kept for measurement: it is slightly slower, see DESIGN.md) */
-RB_API int rb_ctx_set_plan_mode(rb_ctx* ctx, int mode);
 RB_API int rb_process_host(rb_ctx* ctx, int algo, const float* x, const int32_t* len, int B, int ld,
                     const rb_plan* plan, float* y);
 /* Tracing: with rb_ctx_trace(ctx, 1) every later call records, per pipeline chunk, six doubles -- first utterance, utterance

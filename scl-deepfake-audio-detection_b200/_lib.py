@@ -19,7 +19,7 @@ SYMBOLS = (
     "rb_ssi", "rb_process", "rb_ctx_create", "rb_ctx_destroy", "rb_process_host", "rb_ctx_last_traffic",
     "rb_probe_fp32", "rb_launch_count", "rb_profile_enable", "rb_profile_read", "rb_planner_create", "rb_planner_destroy",
     "rb_planner_draw", "rb_devplan_bytes", "rb_devplan_draw", "rb_process_host_seeded",
-    "rb_ctx_set_chunk", "rb_ctx_set_plan_mode", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
+    "rb_ctx_set_chunk", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
     "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
     "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run", "rb_items_stream_draw", "rb_items_stream_run",
 )
@@ -144,8 +144,6 @@ def load() -> C.CDLL:
     lib.rb_submit_host_seeded.argtypes = [vp, i32, C.POINTER(RbArgs), vp, vp, vp, i32, i32, vp, C.POINTER(C.c_uint64)]
     lib.rb_ctx_wait.restype = i32
     lib.rb_ctx_wait.argtypes = [vp, C.c_uint64]
-    lib.rb_ctx_set_plan_mode.restype = i32
-    lib.rb_ctx_set_plan_mode.argtypes = [vp, i32]
     lib.rb_ctx_trace.restype = i32
     lib.rb_ctx_trace.argtypes = [vp, i32]
     lib.rb_ctx_timeline.restype = i32

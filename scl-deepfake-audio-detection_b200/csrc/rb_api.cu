@@ -9,6 +9,7 @@
 #include <new>
 #include <vector>
 
+#include "rb_algo.h"
 #include "rb_common.cuh"
 #include "rb_dense.cuh"
 
@@ -297,7 +298,7 @@ constexpr int kSlots = 8;
 struct Slot {
   char* dev = nullptr;
   size_t bytes = 0;
-  cudaEvent_t ev_in = nullptr, ev_planned = nullptr, ev_done = nullptr, ev_out = nullptr;
+  cudaEvent_t ev_in = nullptr, ev_done = nullptr, ev_out = nullptr;
 };
 }  // namespace
 
@@ -318,7 +319,6 @@ struct rb_ctx {
   int device;
   int sm_count;
   int chunk;  // utterances per pipeline chunk (0: four per SM)
-  int plan_mode;  // device planner: 0 = on its own streams beside the kernels (default), 1 = in line on the kernels' stream
   cudaStream_t s_in, s_plan, s_apply, s_cmp, s_out;
   Slot slot[kSlots];
   uint64_t seq = 0;    // chunks issued so far (slot = seq % kSlots)
@@ -331,14 +331,24 @@ struct rb_ctx {
 
 namespace {
 
-int slot_reserve(Slot& sl, size_t need) {
-  if (need <= sl.bytes) return RB_OK;
-  if (sl.dev) RB_CUDA(cudaFree(sl.dev));
-  sl.dev = nullptr;
-  sl.bytes = 0;
-  need += need / 8;
-  RB_CUDA(cudaMalloc((void**)&sl.dev, need));
-  sl.bytes = need;
+// Grow a device buffer to hold `need` bytes (allocating need + slack) once the device has drained: queued work may still use it.
+int grow(char*& p, size_t& bytes, size_t need, size_t slack) {
+  if (need <= bytes) return RB_OK;
+  RB_CUDA(cudaDeviceSynchronize());
+  if (p) RB_CUDA(cudaFree(p));
+  p = nullptr;
+  bytes = 0;
+  RB_CUDA(cudaMalloc((void**)&p, need + slack));
+  bytes = need + slack;
+  return RB_OK;
+}
+
+int add_events(std::vector<cudaEvent_t>& v, int n) {
+  while ((int)v.size() < n) {
+    cudaEvent_t e;
+    RB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    v.push_back(e);
+  }
   return RB_OK;
 }
 
@@ -361,14 +371,179 @@ struct IoSpec {
   bool has_user = false;
 };
 
+// Events of a traced synchronous call (rb_ctx_trace): [0] its start, [1..4] per chunk: copy-in, plan, kernels, copy-out done.
+struct Trace {
+  bool on;
+  std::vector<cudaEvent_t> ev[5];
+  void mark(int stage, cudaStream_t st) {
+    if (!on) return;
+    cudaEvent_t e;
+    if (cudaEventCreate(&e) == cudaSuccess) {
+      cudaEventRecord(e, st);
+      ev[stage].push_back(e);
+    }
+  }
+  // rb_ctx_timeline's rows, once the device has drained (none if an event could not be created)
+  void rows(const std::vector<int>& first, std::vector<double>& out) const {
+    const size_t nchunks = first.size() - 1;
+    bool complete = ev[0].size() == 1;
+    for (int k = 1; k < 5; ++k) complete = complete && ev[k].size() == nchunks;
+    if (!complete) return;
+    for (size_t ci = 0; ci < nchunks; ++ci) {
+      out.push_back((double)first[ci]);
+      out.push_back((double)(first[ci + 1] - first[ci]));
+      for (int k = 1; k < 5; ++k) {
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, ev[0][0], ev[k][ci]);
+        out.push_back((double)ms);
+      }
+    }
+  }
+  ~Trace() {
+    for (auto& v : ev)
+      for (cudaEvent_t e : v) cudaEventDestroy(e);
+  }
+};
+
+// ---- host CSR plan (rb_process_host): each chunk's slices are uploaded beside its waveforms ---------------------------------
+struct HostPlanSlots {  // slot offsets of the slices
+  size_t lnl_off, lnl_taps, isd_off, isd_idx, isd_fr, ssi_noise, ssi_off, ssi_taps, ssi_snr;
+};
+
+// Slot space for the slices of chunks of at most `chunk` utterances, the tap and impulse arrays sized for the largest payload.
+HostPlanSlots host_plan_slots(Take& take, const rb_plan* plan, int algo, const std::vector<int>& first, int chunk, int ld) {
+  const bool lnl = algo_uses_lnl(algo), isd = algo_uses_isd(algo), ssi = algo_uses_ssi(algo);
+  const int n_f = plan->n_f;
+  size_t max_lt = 0, max_isd = 0, max_st = 0;
+  for (size_t ci = 0; ci + 1 < first.size(); ++ci) {
+    const int u0 = first[ci], u1 = first[ci + 1];
+    if (lnl) max_lt = std::max(max_lt, (size_t)(plan->lnl_tap_off[(size_t)u1 * n_f] - plan->lnl_tap_off[(size_t)u0 * n_f]));
+    if (isd) max_isd = std::max(max_isd, (size_t)(plan->isd_off[u1] - plan->isd_off[u0]));
+    if (ssi) max_st = std::max(max_st, (size_t)(plan->ssi_tap_off[u1] - plan->ssi_tap_off[u0]));
+  }
+  HostPlanSlots o;
+  o.lnl_off = take(lnl ? ((size_t)chunk * n_f + 1) * 4 : 0);
+  o.lnl_taps = take(max_lt * 4);
+  o.isd_off = take(isd ? (size_t)(chunk + 1) * 4 : 0);
+  o.isd_idx = take(max_isd * 4);
+  o.isd_fr = take(max_isd * 8);
+  o.ssi_noise = take(ssi ? (size_t)chunk * ld * sizeof(float) : 0);
+  o.ssi_off = take(ssi ? (size_t)(chunk + 1) * 4 : 0);
+  o.ssi_taps = take(max_st * 4);
+  o.ssi_snr = take(ssi ? (size_t)chunk * 4 : 0);
+  return o;
+}
+
+// Copy the slices of utterances [u0, u0 + bc) into slot memory d on stream st and return the chunk's plan in *dp. CSR slices
+// keep their absolute offsets; the value pointers are rebased so that ptr[off] lands in the slice.
+int upload_plan_slice(const rb_plan* plan, int algo, const HostPlanSlots& o, char* d, int u0, int bc, int ld, cudaStream_t st,
+                      uint64_t& h2d, rb_plan* dp) {
+  const int n_f = plan->n_f;
+  memset(dp, 0, sizeof(*dp));
+  dp->n_f = n_f;
+  dp->g_sd = plan->g_sd;
+  auto up = [&](size_t off, const void* src, size_t n) -> int {
+    if (n == 0) return RB_OK;
+    h2d += n;
+    return (int)cudaMemcpyAsync(d + off, src, n, cudaMemcpyHostToDevice, st);
+  };
+  if (algo_uses_lnl(algo)) {
+    const int32_t* off = plan->lnl_tap_off + (size_t)u0 * n_f;
+    const size_t base = (size_t)off[0], cnt = (size_t)off[(size_t)bc * n_f] - base;
+    RB_TRY(up(o.lnl_off, off, ((size_t)bc * n_f + 1) * 4));
+    RB_TRY(up(o.lnl_taps, plan->lnl_taps + base, cnt * 4));
+    dp->lnl_tap_off = (const int32_t*)(d + o.lnl_off);
+    dp->lnl_taps = (const float*)(d + o.lnl_taps) - base;
+  }
+  if (algo_uses_isd(algo)) {
+    const int32_t* off = plan->isd_off + u0;
+    const size_t base = (size_t)off[0], cnt = (size_t)off[bc] - base;
+    RB_TRY(up(o.isd_off, off, (size_t)(bc + 1) * 4));
+    RB_TRY(up(o.isd_idx, plan->isd_idx + base, cnt * 4));
+    RB_TRY(up(o.isd_fr, plan->isd_fr + base, cnt * 8));
+    dp->isd_off = (const int32_t*)(d + o.isd_off);
+    dp->isd_idx = (const int32_t*)(d + o.isd_idx) - base;
+    dp->isd_fr = (const double*)(d + o.isd_fr) - base;
+  }
+  if (algo_uses_ssi(algo)) {
+    const int32_t* off = plan->ssi_tap_off + u0;
+    const size_t base = (size_t)off[0], cnt = (size_t)off[bc] - base;
+    RB_TRY(up(o.ssi_noise, plan->ssi_noise + (size_t)u0 * ld, (size_t)bc * ld * sizeof(float)));
+    RB_TRY(up(o.ssi_off, off, (size_t)(bc + 1) * 4));
+    RB_TRY(up(o.ssi_taps, plan->ssi_taps + base, cnt * 4));
+    RB_TRY(up(o.ssi_snr, plan->ssi_snr_db + u0, (size_t)bc * 4));
+    dp->ssi_noise = (const float*)(d + o.ssi_noise);
+    dp->ssi_tap_off = (const int32_t*)(d + o.ssi_off);
+    dp->ssi_taps = (const float*)(d + o.ssi_taps) - base;
+    dp->ssi_snr_db = (const float*)(d + o.ssi_snr);
+  }
+  return RB_OK;
+}
+
+// ---- device plan (the seeded entries): drawn for the whole batch, read in place -----------------------------------------
+// The slice of utterances [u0, ...): CSR offsets are absolute, so only the owner arrays move.
+rb_plan device_plan_slice(const rb_plan& whole, int u0, int ld) {
+  rb_plan dp = whole;
+  if (dp.lnl_tap_off) dp.lnl_tap_off += (size_t)u0 * dp.n_f;
+  if (dp.isd_off) dp.isd_off += u0;
+  if (dp.ssi_tap_off) {
+    dp.ssi_noise += (size_t)u0 * ld;
+    dp.ssi_tap_off += u0;
+    dp.ssi_snr_db += u0;
+  }
+  return dp;
+}
+
+// Queue the device planner of a whole call; R.ev_planned[ci] fires once chunk ci's plan is complete. The plans need only
+// lengths and seeds. Its kernels are latency-bound (one warp per utterance: the stream replay of one utterance takes ~2 ms
+// however few utterances a launch holds), so they are issued in pieces -- chunk 0, chunk 1, then about 4096 utterances at a
+// time (one full wave of the replay kernel) -- so that the first results leave early (a host-buffer call is bound by the
+// copy-out stream, which starts with the first filtered chunk) while large batches pay the replay latency once per wave, not
+// once per chunk. Stream replay runs on s_plan, swap application on s_apply, both at low priority beside the kernels.
+// Measured (scripts/gpu_overlap_probe.py): while the FIR-bank kernel still has CTAs to dispatch, the hardware does not place
+// another kernel's CTAs in the registers / shared memory its resident CTAs leave free, so the planner really runs in the
+// gaps: during copies, at the tail of each FIR launch, and before the first chunk.
+int queue_devplan(rb_ctx* c, CallRes& R, const rb_args* args, int algo, int B, int ld, const int32_t* d_len, const uint32_t* d_seeds,
+                  const std::vector<int>& first, int chunk, bool x_dev, Trace& trace, rb_plan* whole) {
+  const bool ssi = algo_uses_ssi(algo);
+  const int nchunks = (int)first.size() - 1;
+  std::vector<int> piece_end;  // one past the last chunk of each piece
+  if (!ssi && nchunks >= 3) {  // SSI tap offsets need the stream positions of every utterance: one piece
+    const int per_wave = std::max(1, 4096 / chunk);
+    if (!x_dev) {
+      piece_end.push_back(1);
+      piece_end.push_back(2);
+    }
+    while ((piece_end.empty() ? 0 : piece_end.back()) < nchunks)
+      piece_end.push_back(std::min(nchunks, (piece_end.empty() ? 0 : piece_end.back()) + per_wave));
+  } else {
+    piece_end.push_back(nchunks);
+  }
+  RB_TRY(add_events(R.ev_planned, nchunks));
+  RB_TRY(add_events(R.ev_body, (int)piece_end.size()));
+  RB_TRY(devplan_begin(args, algo, B, ld, d_len, d_seeds, R.planmem, R.planmem_bytes, whole, c->s_plan));
+  for (int pc = 0; pc < (int)piece_end.size(); ++pc) {
+    const int cb = pc ? piece_end[pc - 1] : 0;
+    const int u0 = first[cb], u1 = first[piece_end[pc]];
+    RB_TRY(devplan_body(args, algo, B, ld, d_len, d_seeds, R.planmem, u0, u1 - u0, c->s_plan));
+    if (ssi) RB_TRY(devplan_end(args, algo, B, ld, R.planmem, c->s_plan));
+    RB_CUDA(cudaEventRecord(R.ev_body[pc], c->s_plan));
+    RB_CUDA(cudaStreamWaitEvent(c->s_apply, R.ev_body[pc], 0));
+    for (int ci = cb; ci < piece_end[pc]; ++ci) {
+      RB_TRY(devplan_apply(args, algo, B, ld, d_len, R.planmem, first[ci], first[ci + 1] - first[ci], c->s_apply));
+      RB_CUDA(cudaEventRecord(R.ev_planned[ci], c->s_apply));
+      trace.mark(2, c->s_apply);
+    }
+  }
+  return RB_OK;
+}
+
 // Common driver. plan != NULL: host CSR plan, sliced and uploaded per chunk. plan == NULL: seeds/args given, drawn on the device.
 int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int B, int ld, const rb_plan* plan, const rb_args* args,
                  const uint32_t* seeds, bool async, uint64_t* ticket) {
   const bool x_dev = io.x_kind == RB_IO_DEVICE_F32, x_pcm = io.x_kind == RB_IO_HOST_PCM16, y_dev = io.y_kind == RB_IO_DEVICE_F32;
   const float* x = (const float*)io.x;
   float* y = (float*)io.y;
-  if (x_pcm && ld % 8 != 0) return RB_ERR_ALIGNMENT;
-  if ((x_dev || x_pcm || y_dev) && plan != nullptr) return RB_ERR_INVALID_ARG;  // the host-plan form is host float32 in / out only
   RB_CUDA(cudaSetDevice(c->device));
   CallRes& R = c->res[c->calls & 1];
   if (R.inflight) {  // at most two calls in flight: the one that used this resource set must be complete
@@ -376,18 +551,8 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
     R.inflight = false;
   }
   const bool active = algo >= 1 && algo <= 8;
-  const bool use_lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
-  const bool use_isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool use_ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
   const bool devplan = active && plan == nullptr;
-  if (active && !devplan) {
-    if (use_lnl && (plan->n_f < 1 || !plan->lnl_taps || !plan->lnl_tap_off)) return RB_ERR_PLAN;
-    if (use_isd && (!plan->isd_off || !plan->isd_idx || !plan->isd_fr)) return RB_ERR_PLAN;
-    if (use_ssi && (!plan->ssi_noise || !plan->ssi_taps || !plan->ssi_tap_off || !plan->ssi_snr_db)) return RB_ERR_PLAN;
-  }
-  if (devplan && (!args || !seeds)) return RB_ERR_INVALID_ARG;
   const int chunk = std::max(1, std::min(B, c->chunk > 0 ? c->chunk : 4 * c->sm_count));
-  const int n_f = plan ? plan->n_f : (args ? args->N_f : 0);
   // Equal chunks. Shorter chunks at the start and / or the end (to get the first results out earlier, to shorten the last
   // copy-out) were measured and do not help: with both PCIe directions busy the call is bound by the two ~22 ms copy streams
   // and their mutual offset of one chunk's filtering.
@@ -398,15 +563,7 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
 
   // everything queued below is ordered by events only; the host blocks once, at the end
   // per-call metadata: lengths (+ seeds) for the whole batch
-  const size_t meta_need = align_up((size_t)B * 4, 256) * 2;
-  if (meta_need > R.meta_bytes) {
-    RB_CUDA(cudaDeviceSynchronize());
-    if (R.meta) RB_CUDA(cudaFree(R.meta));
-    R.meta = nullptr;
-    R.meta_bytes = 0;
-    RB_CUDA(cudaMalloc((void**)&R.meta, meta_need));
-    R.meta_bytes = meta_need;
-  }
+  RB_TRY(grow(R.meta, R.meta_bytes, align_up((size_t)B * 4, 256) * 2, 0));
   const int32_t* d_len = (int32_t*)R.meta;
   const uint32_t* d_seeds = (uint32_t*)(R.meta + align_up((size_t)B * 4, 256));
   uint64_t h2d = 0, d2h = 0;
@@ -434,110 +591,26 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
   const size_t ws_bytes = active ? rb_workspace_bytes_for(algo, chunk, ld) : 0;
   const size_t dp_bytes = devplan ? rb_devplan_bytes(args, algo, B, ld) : 0;
   if (devplan && dp_bytes == 0) return RB_ERR_UNSUPPORTED;
-  if (dp_bytes > R.planmem_bytes) {
-    RB_CUDA(cudaDeviceSynchronize());
-    if (R.planmem) RB_CUDA(cudaFree(R.planmem));
-    R.planmem = nullptr;
-    R.planmem_bytes = 0;
-    RB_CUDA(cudaMalloc((void**)&R.planmem, dp_bytes + dp_bytes / 8));
-    R.planmem_bytes = dp_bytes + dp_bytes / 8;
-  }
-  while (devplan && (int)R.ev_planned.size() < nchunks) {
-    cudaEvent_t e;
-    RB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    R.ev_planned.push_back(e);
-  }
-  size_t max_lt = 0, max_isd = 0, max_st = 0;  // largest per-chunk CSR payloads of a host plan
-  if (active && !devplan) {
-    for (int ci = 0; ci < nchunks; ++ci) {
-      const int u0 = first[ci], bc = first[ci + 1] - u0;
-      if (use_lnl) max_lt = std::max(max_lt, (size_t)(plan->lnl_tap_off[(size_t)(u0 + bc) * n_f] - plan->lnl_tap_off[(size_t)u0 * n_f]));
-      if (use_isd) max_isd = std::max(max_isd, (size_t)(plan->isd_off[u0 + bc] - plan->isd_off[u0]));
-      if (use_ssi) max_st = std::max(max_st, (size_t)(plan->ssi_tap_off[u0 + bc] - plan->ssi_tap_off[u0]));
-    }
-  }
+  RB_TRY(grow(R.planmem, R.planmem_bytes, dp_bytes, dp_bytes / 8));
   Take take;
   const size_t o_x = take(x_dev ? 0 : wave), o_x16 = take(x_pcm ? wave / 2 : 0), o_y = take(y_dev ? 0 : wave), o_ws = take(ws_bytes);
-  const size_t o_lo = take(use_lnl && !devplan ? ((size_t)chunk * n_f + 1) * 4 : 0), o_lt = take(max_lt * 4);
-  const size_t o_io = take(use_isd && !devplan ? (size_t)(chunk + 1) * 4 : 0), o_ii = take(max_isd * 4), o_if = take(max_isd * 8);
-  const size_t o_sn = take(use_ssi && !devplan ? wave : 0), o_so = take(use_ssi && !devplan ? (size_t)(chunk + 1) * 4 : 0),
-               o_st = take(max_st * 4), o_sr = take(use_ssi && !devplan ? (size_t)chunk * 4 : 0);
+  HostPlanSlots hp{};
+  if (active && !devplan) hp = host_plan_slots(take, plan, algo, first, chunk, ld);
   for (int k = 0; k < std::min(kSlots, nchunks); ++k) {
     Slot& sl = c->slot[(c->seq + k) % kSlots];
-    if (take.off > sl.bytes) {
-      RB_CUDA(cudaDeviceSynchronize());
-      RB_TRY(slot_reserve(sl, take.off));
-    }
+    RB_TRY(grow(sl.dev, sl.bytes, take.off, take.off / 8));
   }
 
-  std::vector<cudaEvent_t> tev[5];  // trace: [0] start of the call, [1..4] per chunk: copy-in, plan, kernels, copy-out
-  auto mark = [&](int stage, cudaStream_t st) {
-    if (!c->trace || async) return;
-    cudaEvent_t e;
-    if (cudaEventCreate(&e) == cudaSuccess) {
-      cudaEventRecord(e, st);
-      tev[stage].push_back(e);
-    }
-  };
-  mark(0, c->s_in);
-  // Device planner. The plans need only lengths and seeds. Its kernels are latency-bound (one warp per utterance: the stream
-  // replay of one utterance takes ~2 ms however few utterances a launch holds), so they are issued in pieces -- chunk 0,
-  // chunk 1, then about 4096 utterances at a time (one full wave of the replay kernel) -- so that the first results leave
-  // early (a host-buffer call is bound by the copy-out stream, which starts with the first filtered chunk) while large batches
-  // pay the replay latency once per wave, not once per chunk.
-  //   plan_mode 0 (default): stream replay on s_plan, swap application on s_apply, both at low priority beside the kernels.
-  //     Measured (scripts/gpu_overlap_probe.py): while the FIR-bank kernel still has CTAs to dispatch, the hardware does not
-  //     place another kernel's CTAs in the registers / shared memory its resident CTAs leave free, so the planner really runs
-  //     in the gaps: during copies, at the tail of each FIR launch, and before the first chunk.
-  //   plan_mode 1: in line on the kernels' stream, each piece right before the first chunk that needs it; kept for measurement.
-  std::vector<int> piece_end;
-  if (devplan && !use_ssi && nchunks >= 3) {  // SSI tap offsets need the stream positions of every utterance: one piece
-    const int per_wave = std::max(1, 4096 / chunk);
-    if (!x_dev) {
-      piece_end.push_back(1);
-      piece_end.push_back(2);
-    }
-    while ((piece_end.empty() ? 0 : piece_end.back()) < nchunks)
-      piece_end.push_back(std::min(nchunks, (piece_end.empty() ? 0 : piece_end.back()) + per_wave));
-  } else {
-    piece_end.push_back(nchunks);
-  }
-  const int npieces = (int)piece_end.size();
-  while (devplan && (int)R.ev_body.size() < npieces) {
-    cudaEvent_t e;
-    RB_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    R.ev_body.push_back(e);
-  }
-  auto plan_piece = [&](int pc, cudaStream_t s_body, cudaStream_t s_swap) -> int {
-    const int cb = pc ? piece_end[pc - 1] : 0;
-    const int u0 = first[cb], u1 = first[piece_end[pc]];
-    RB_TRY(devplan_body(args, algo, B, ld, d_len, d_seeds, R.planmem, u0, u1 - u0, s_body));
-    if (use_ssi) RB_TRY(devplan_end(args, algo, B, ld, R.planmem, s_body));
-    if (s_swap != s_body) {
-      RB_CUDA(cudaEventRecord(R.ev_body[pc], s_body));
-      RB_CUDA(cudaStreamWaitEvent(s_swap, R.ev_body[pc], 0));
-    }
-    for (int ci = cb; ci < piece_end[pc]; ++ci) {
-      RB_TRY(devplan_apply(args, algo, B, ld, d_len, R.planmem, first[ci], first[ci + 1] - first[ci], s_swap));
-      if (s_swap != c->s_cmp) RB_CUDA(cudaEventRecord(R.ev_planned[ci], s_swap));
-      mark(2, s_swap);
-    }
-    return RB_OK;
-  };
-  rb_plan whole;
-  memset(&whole, 0, sizeof(whole));
-  if (devplan) {
-    const cudaStream_t s0 = c->plan_mode ? c->s_cmp : c->s_plan;
-    RB_TRY(devplan_begin(args, algo, B, ld, d_len, d_seeds, R.planmem, R.planmem_bytes, &whole, s0));
-    if (!c->plan_mode)
-      for (int pc = 0; pc < npieces; ++pc) RB_TRY(plan_piece(pc, c->s_plan, c->s_apply));
-  }
+  Trace trace{c->trace && !async};
+  trace.mark(0, c->s_in);
+  rb_plan whole{};
+  if (devplan) RB_TRY(queue_devplan(c, R, args, algo, B, ld, d_len, d_seeds, first, chunk, x_dev, trace, &whole));
   for (int ci = 0; ci < nchunks; ++ci) {
     Slot& sl = c->slot[(c->seq + ci) % kSlots];
     char* d = sl.dev;
     const int u0 = first[ci], bc = first[ci + 1] - u0;
     const size_t cw = (size_t)bc * ld * sizeof(float);
-    // ---- stage 1: host -> device ------------------------------------------------------------------------------------
+    // ---- stage 1: host -> device: the waveforms and, of a host plan, the chunk's slices -------------------------------
     if (c->seq + ci >= kSlots) RB_CUDA(cudaStreamWaitEvent(c->s_in, sl.ev_out, 0));  // the slot's previous chunk has left the device
     if (x_pcm) {
       RB_CUDA(cudaMemcpyAsync(d + o_x16, (const int16_t*)io.x + (size_t)u0 * ld, cw / 2, cudaMemcpyHostToDevice, c->s_in));
@@ -546,68 +619,14 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
       RB_CUDA(cudaMemcpyAsync(d + o_x, x + (size_t)u0 * ld, cw, cudaMemcpyHostToDevice, c->s_in));
       h2d += cw;
     }
-    rb_plan dp;
-    memset(&dp, 0, sizeof(dp));
-    if (active && !devplan) {
-      dp.n_f = plan->n_f;
-      dp.g_sd = plan->g_sd;
-      auto up = [&](size_t o, const void* src, size_t n) -> int {
-        if (n == 0) return RB_OK;
-        h2d += n;
-        return (int)cudaMemcpyAsync(d + o, src, n, cudaMemcpyHostToDevice, c->s_in);
-      };
-      // CSR slices keep their absolute offsets; the value pointers are rebased so that ptr[off] lands in the slice
-      if (use_lnl) {
-        const int32_t* off = plan->lnl_tap_off + (size_t)u0 * n_f;
-        const size_t base = (size_t)off[0], cnt = (size_t)off[(size_t)bc * n_f] - base;
-        RB_TRY(up(o_lo, off, ((size_t)bc * n_f + 1) * 4));
-        RB_TRY(up(o_lt, plan->lnl_taps + base, cnt * 4));
-        dp.lnl_tap_off = (const int32_t*)(d + o_lo);
-        dp.lnl_taps = (const float*)(d + o_lt) - base;
-      }
-      if (use_isd) {
-        const int32_t* off = plan->isd_off + u0;
-        const size_t base = (size_t)off[0], cnt = (size_t)off[bc] - base;
-        RB_TRY(up(o_io, off, (size_t)(bc + 1) * 4));
-        RB_TRY(up(o_ii, plan->isd_idx + base, cnt * 4));
-        RB_TRY(up(o_if, plan->isd_fr + base, cnt * 8));
-        dp.isd_off = (const int32_t*)(d + o_io);
-        dp.isd_idx = (const int32_t*)(d + o_ii) - base;
-        dp.isd_fr = (const double*)(d + o_if) - base;
-      }
-      if (use_ssi) {
-        const int32_t* off = plan->ssi_tap_off + u0;
-        const size_t base = (size_t)off[0], cnt = (size_t)off[bc] - base;
-        RB_TRY(up(o_sn, plan->ssi_noise + (size_t)u0 * ld, cw));
-        RB_TRY(up(o_so, off, (size_t)(bc + 1) * 4));
-        RB_TRY(up(o_st, plan->ssi_taps + base, cnt * 4));
-        RB_TRY(up(o_sr, plan->ssi_snr_db + u0, (size_t)bc * 4));
-        dp.ssi_noise = (const float*)(d + o_sn);
-        dp.ssi_tap_off = (const int32_t*)(d + o_so);
-        dp.ssi_taps = (const float*)(d + o_st) - base;
-        dp.ssi_snr_db = (const float*)(d + o_sr);
-      }
-    }
+    rb_plan dp{};
+    if (devplan) dp = device_plan_slice(whole, u0, ld);
+    else if (active) RB_TRY(upload_plan_slice(plan, algo, hp, d, u0, bc, ld, c->s_in, h2d, &dp));
     RB_CUDA(cudaEventRecord(sl.ev_in, c->s_in));
-    mark(1, c->s_in);
-    // ---- stage 2: plan (own stream, overlaps the previous chunk's kernels) + kernels --------------------------------------
-    if (devplan) {  // the chunk's slice of the whole-batch plan: CSR offsets are absolute, so only the owner arrays move
-      dp = whole;
-      if (use_lnl) dp.lnl_tap_off = whole.lnl_tap_off + (size_t)u0 * n_f;
-      if (use_isd) dp.isd_off = whole.isd_off + u0;
-      if (use_ssi) {
-        dp.ssi_noise = whole.ssi_noise + (size_t)u0 * ld;
-        dp.ssi_tap_off = whole.ssi_tap_off + u0;
-        dp.ssi_snr_db = whole.ssi_snr_db + u0;
-      }
-      if (c->plan_mode) {
-        for (int pc = 0; pc < npieces; ++pc)
-          if (ci == (pc ? piece_end[pc - 1] : 0)) RB_TRY(plan_piece(pc, c->s_cmp, c->s_cmp));
-      } else {
-        RB_CUDA(cudaStreamWaitEvent(c->s_cmp, R.ev_planned[ci], 0));
-      }
-    }
-    if (!devplan) mark(2, c->s_in);
+    trace.mark(1, c->s_in);
+    // ---- stage 2: kernels, once the chunk's plan (drawn beside the previous chunks' kernels) and waveforms are there ------
+    if (devplan) RB_CUDA(cudaStreamWaitEvent(c->s_cmp, R.ev_planned[ci], 0));
+    else trace.mark(2, c->s_in);
     RB_CUDA(cudaStreamWaitEvent(c->s_cmp, sl.ev_in, 0));
     if (x_pcm) {
       RB_TRY(launch_pcm16_to_f32((const int16_t*)(d + o_x16), (float*)(d + o_x), (size_t)bc * ld, c->s_cmp));
@@ -616,7 +635,7 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
     float* yout = y_dev ? y + (size_t)u0 * ld : (float*)(d + o_y);
     RB_TRY(rb_process(algo, xin, d_len + u0, bc, ld, active ? &dp : nullptr, yout, d + o_ws, ws_bytes, c->s_cmp));
     RB_CUDA(cudaEventRecord(sl.ev_done, c->s_cmp));
-    mark(3, c->s_cmp);
+    trace.mark(3, c->s_cmp);
     // ---- stage 3: device -> host (or nothing: the results stay where the kernels wrote them) ---------------------------
     if (y_dev) {
       RB_CUDA(cudaEventRecord(sl.ev_out, c->s_cmp));
@@ -626,7 +645,7 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
       d2h += cw;
       RB_CUDA(cudaEventRecord(sl.ev_out, c->s_out));
     }
-    mark(4, y_dev ? c->s_cmp : c->s_out);
+    trace.mark(4, y_dev ? c->s_cmp : c->s_out);
   }
   c->seq += (uint64_t)nchunks;
   RB_CUDA(cudaEventRecord(R.ev_done, y_dev ? c->s_cmp : c->s_out));
@@ -642,25 +661,35 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
   if (c->trace) {
     c->timeline.clear();
     RB_CUDA(cudaDeviceSynchronize());
-    bool complete = tev[0].size() == 1;
-    for (int k = 1; k < 5; ++k) complete = complete && (int)tev[k].size() == nchunks;
-    if (complete) {
-      for (int ci = 0; ci < nchunks; ++ci) {
-        c->timeline.push_back((double)first[ci]);
-        c->timeline.push_back((double)(first[ci + 1] - first[ci]));
-        for (int k = 1; k < 5; ++k) {
-          float ms = 0.f;
-          cudaEventElapsedTime(&ms, tev[0][0], tev[k][ci]);
-          c->timeline.push_back((double)ms);
-        }
-      }
-    }
-    for (auto& v : tev)
-      for (cudaEvent_t e : v) cudaEventDestroy(e);
+    trace.rows(first, c->timeline);
   }
-  c->h2d = h2d;
-  c->d2h = d2h;
   return RB_OK;
+}
+
+int check_host_batch(const rb_ctx* c, const void* x, const int32_t* len, int B, int ld, const void* y) {
+  if (!c) return RB_ERR_INVALID_ARG;
+  if (B < 0 || ld < 0) return RB_ERR_INVALID_ARG;
+  if (B == 0 || ld == 0) return RB_OK;
+  if (!x || !len || !y) return RB_ERR_INVALID_ARG;
+  if (ld % 4 != 0) return RB_ERR_ALIGNMENT;
+  return RB_OK;
+}
+
+// The seeded entries: argument checks, then the pipeline with the plans drawn on the device.
+int run_seeded(rb_ctx* c, int algo, const rb_args* args, const void* x, int x_kind, const int32_t* len, const uint32_t* seeds, int B,
+               int ld, void* y, int y_kind, void* user_stream, int use_user_stream, bool async, uint64_t* ticket) {
+  if (ticket) *ticket = 0;
+  if (x_kind != RB_IO_HOST_F32 && x_kind != RB_IO_HOST_PCM16 && x_kind != RB_IO_DEVICE_F32) return RB_ERR_INVALID_ARG;
+  if (y_kind != RB_IO_HOST_F32 && y_kind != RB_IO_DEVICE_F32) return RB_ERR_INVALID_ARG;
+  RB_TRY(check_host_batch(c, x, len, B, ld, y));
+  if (B == 0 || ld == 0) return RB_OK;
+  if (algo >= 1 && algo <= 8 && (!args || !seeds)) return RB_ERR_INVALID_ARG;
+  if (x_kind == RB_IO_DEVICE_F32 && !use_user_stream) return RB_ERR_INVALID_ARG;  // device input needs the stream that produced it
+  if ((x_kind == RB_IO_DEVICE_F32 && ((uintptr_t)x & 15u)) || (y_kind == RB_IO_DEVICE_F32 && ((uintptr_t)y & 15u))) return RB_ERR_ALIGNMENT;
+  if (x_kind == RB_IO_DEVICE_F32 && x == y && algo >= 1 && algo <= 8) return RB_ERR_INVALID_ARG;
+  if (x_kind == RB_IO_HOST_PCM16 && ld % 8 != 0) return RB_ERR_ALIGNMENT;
+  const IoSpec io{x, x_kind, y, y_kind, (cudaStream_t)user_stream, use_user_stream != 0};
+  return run_pipeline(c, algo, io, len, B, ld, nullptr, args, seeds, async, ticket);
 }
 
 }  // namespace
@@ -680,7 +709,6 @@ int rb_ctx_create(rb_ctx** out, int device) {
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
   c->chunk = 0;
-  c->plan_mode = 0;
   c->h2d = c->d2h = 0;
   c->s_in = c->s_plan = c->s_apply = c->s_cmp = c->s_out = nullptr;
   // Stream priorities: copies first, then the FIR kernel's stream, the planner's streams last. The planner only needs to stay
@@ -697,7 +725,7 @@ int rb_ctx_create(rb_ctx** out, int device) {
     for (cudaEvent_t* ev : {&R.ev_meta, &R.ev_done, &R.ev_user})
       if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
   for (Slot& sl : c->slot)
-    for (cudaEvent_t* ev : {&sl.ev_in, &sl.ev_planned, &sl.ev_done, &sl.ev_out})
+    for (cudaEvent_t* ev : {&sl.ev_in, &sl.ev_done, &sl.ev_out})
       if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
   if (e != cudaSuccess) {
     rb_ctx_destroy(c);
@@ -713,7 +741,7 @@ int rb_ctx_destroy(rb_ctx* c) {
   cudaDeviceSynchronize();
   for (Slot& sl : c->slot) {
     if (sl.dev) cudaFree(sl.dev);
-    for (cudaEvent_t ev : {sl.ev_in, sl.ev_planned, sl.ev_done, sl.ev_out})
+    for (cudaEvent_t ev : {sl.ev_in, sl.ev_done, sl.ev_out})
       if (ev) cudaEventDestroy(ev);
   }
   for (CallRes& R : c->res) {
@@ -733,12 +761,6 @@ int rb_ctx_destroy(rb_ctx* c) {
 int rb_ctx_set_chunk(rb_ctx* c, int utterances) {
   if (!c || utterances < 0) return RB_ERR_INVALID_ARG;
   c->chunk = utterances;
-  return RB_OK;
-}
-
-int rb_ctx_set_plan_mode(rb_ctx* c, int mode) {
-  if (!c || (mode != 0 && mode != 1)) return RB_ERR_INVALID_ARG;
-  c->plan_mode = mode;
   return RB_OK;
 }
 
@@ -762,65 +784,34 @@ int rb_ctx_last_traffic(const rb_ctx* c, uint64_t* h2d, uint64_t* d2h) {
   return RB_OK;
 }
 
-static int check_host_batch(const rb_ctx* c, const float* x, const int32_t* len, int B, int ld, const float* y) {
-  if (!c) return RB_ERR_INVALID_ARG;
-  if (B < 0 || ld < 0) return RB_ERR_INVALID_ARG;
-  if (B == 0 || ld == 0) return RB_OK;
-  if (!x || !len || !y) return RB_ERR_INVALID_ARG;
-  if (ld % 4 != 0) return RB_ERR_ALIGNMENT;
-  return RB_OK;
-}
-
-static IoSpec host_io(const float* x, float* y) {
-  IoSpec io;
-  io.x = x;
-  io.y = y;
-  return io;
-}
-
 int rb_process_host(rb_ctx* c, int algo, const float* x, const int32_t* len, int B, int ld, const rb_plan* plan, float* y) {
   RB_TRY(check_host_batch(c, x, len, B, ld, y));
   if (B == 0 || ld == 0) return RB_OK;
-  if (algo >= 1 && algo <= 8 && !plan) return RB_ERR_PLAN;
-  return run_pipeline(c, algo, host_io(x, y), len, B, ld, plan, nullptr, nullptr, false, nullptr);
+  if (algo >= 1 && algo <= 8) {
+    if (!plan) return RB_ERR_PLAN;
+    if (algo_uses_lnl(algo) && (plan->n_f < 1 || !plan->lnl_taps || !plan->lnl_tap_off)) return RB_ERR_PLAN;
+    if (algo_uses_isd(algo) && (!plan->isd_off || !plan->isd_idx || !plan->isd_fr)) return RB_ERR_PLAN;
+    if (algo_uses_ssi(algo) && (!plan->ssi_noise || !plan->ssi_taps || !plan->ssi_tap_off || !plan->ssi_snr_db)) return RB_ERR_PLAN;
+  }
+  IoSpec io;
+  io.x = x;
+  io.y = y;
+  return run_pipeline(c, algo, io, len, B, ld, plan, nullptr, nullptr, false, nullptr);
 }
 
 int rb_process_host_seeded(rb_ctx* c, int algo, const rb_args* args, const float* x, const int32_t* len, const uint32_t* seeds, int B,
                            int ld, float* y) {
-  RB_TRY(check_host_batch(c, x, len, B, ld, y));
-  if (B == 0 || ld == 0) return RB_OK;
-  if (algo >= 1 && algo <= 8 && (!args || !seeds)) return RB_ERR_INVALID_ARG;
-  return run_pipeline(c, algo, host_io(x, y), len, B, ld, nullptr, args, seeds, false, nullptr);
+  return run_seeded(c, algo, args, x, RB_IO_HOST_F32, len, seeds, B, ld, y, RB_IO_HOST_F32, nullptr, 0, false, nullptr);
 }
 
 int rb_submit_host_seeded(rb_ctx* c, int algo, const rb_args* args, const float* x, const int32_t* len, const uint32_t* seeds, int B,
                           int ld, float* y, uint64_t* ticket) {
-  if (ticket) *ticket = 0;
-  RB_TRY(check_host_batch(c, x, len, B, ld, y));
-  if (B == 0 || ld == 0) return RB_OK;
-  if (algo >= 1 && algo <= 8 && (!args || !seeds)) return RB_ERR_INVALID_ARG;
-  return run_pipeline(c, algo, host_io(x, y), len, B, ld, nullptr, args, seeds, true, ticket);
+  return rb_submit_seeded_ex(c, algo, args, x, RB_IO_HOST_F32, len, seeds, B, ld, y, RB_IO_HOST_F32, nullptr, 0, ticket);
 }
 
 int rb_submit_seeded_ex(rb_ctx* c, int algo, const rb_args* args, const void* x, int x_kind, const int32_t* len, const uint32_t* seeds,
                         int B, int ld, void* y, int y_kind, void* user_stream, int use_user_stream, uint64_t* ticket) {
-  if (ticket) *ticket = 0;
-  if (x_kind != RB_IO_HOST_F32 && x_kind != RB_IO_HOST_PCM16 && x_kind != RB_IO_DEVICE_F32) return RB_ERR_INVALID_ARG;
-  if (y_kind != RB_IO_HOST_F32 && y_kind != RB_IO_DEVICE_F32) return RB_ERR_INVALID_ARG;
-  RB_TRY(check_host_batch(c, (const float*)x, len, B, ld, (const float*)y));
-  if (B == 0 || ld == 0) return RB_OK;
-  if (algo >= 1 && algo <= 8 && (!args || !seeds)) return RB_ERR_INVALID_ARG;
-  if (x_kind == RB_IO_DEVICE_F32 && !use_user_stream) return RB_ERR_INVALID_ARG;  // device input needs the stream that produced it
-  if ((x_kind == RB_IO_DEVICE_F32 && ((uintptr_t)x & 15u)) || (y_kind == RB_IO_DEVICE_F32 && ((uintptr_t)y & 15u))) return RB_ERR_ALIGNMENT;
-  if (x_kind == RB_IO_DEVICE_F32 && x == y && algo >= 1 && algo <= 8) return RB_ERR_INVALID_ARG;
-  IoSpec io;
-  io.x = x;
-  io.x_kind = x_kind;
-  io.y = y;
-  io.y_kind = y_kind;
-  io.user = (cudaStream_t)user_stream;
-  io.has_user = use_user_stream != 0;
-  return run_pipeline(c, algo, io, len, B, ld, nullptr, args, seeds, true, ticket);
+  return run_seeded(c, algo, args, x, x_kind, len, seeds, B, ld, y, y_kind, user_stream, use_user_stream, true, ticket);
 }
 
 int rb_ctx_wait(rb_ctx* c, uint64_t ticket) {

@@ -31,6 +31,7 @@
 #include <algorithm>
 #include <string.h>
 
+#include "rb_algo.h"
 #include "rb_common.cuh"
 #include "rb_mt.cuh"
 
@@ -61,10 +62,6 @@ __device__ int draw_filter_params(const MtStream& s, int w0, const rb_args& a, d
   return K - (a.nBands - 1);
 }
 
-__device__ __forceinline__ bool uses_lnl(int algo) { return algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8; }
-__device__ __forceinline__ bool uses_isd(int algo) { return algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8; }
-__device__ __forceinline__ bool uses_ssi(int algo) { return algo == 3 || algo == 4 || algo == 6 || algo == 7; }
-
 // ---- head: LnL design parameters + tap counts, ISD impulse count ----------------------------------------------------------
 constexpr int kHeadWarps = 4;
 
@@ -80,7 +77,7 @@ plan_head_kernel(rb_args a, int algo, int B, const int32_t* __restrict__ len_arr
   if (snaps) s.load(snaps + (size_t)u * kMtSnapWords, lane);
   else s.seed(seeds[u], lane);
   const int per = 2 * filter_stride(a.nBands);  // stream words per filter
-  if (uses_lnl(algo)) {
+  if (algo_uses_lnl(algo)) {
     // filters are consumed in windows that fit the two tempered blocks
     const int fpw = max(1, min(kMtN / per, 32));  // filters per window, one lane each
     for (int f0 = 0; f0 < a.N_f; f0 += fpw) {
@@ -95,7 +92,7 @@ plan_head_kernel(rb_args a, int algo, int B, const int32_t* __restrict__ len_arr
       s.advance(nf * per, lane);
     }
   }
-  if (uses_isd(algo) && lane == 0) {
+  if (algo_uses_isd(algo) && lane == 0) {
     const double beta = mt_uniform(0.0, a.P, mt_double(s.word(0), s.word(1)));
     isd_cnt[u] = (int)__dmul_rn((double)len_arr[u], __ddiv_rn(beta, 100.0));
   }
@@ -230,8 +227,8 @@ plan_body_kernel(rb_args a, int algo, int B, int ld, int jld, const int32_t* __r
   s.sm = &msm[warp];
   if (snaps) s.load(snaps + (size_t)u * kMtSnapWords, lane);
   else s.seed(seeds[u], lane);
-  if (uses_lnl(algo)) s.skip(a.N_f * 2 * filter_stride(a.nBands), lane);
-  if (uses_isd(algo)) {
+  if (algo_uses_lnl(algo)) s.skip(a.N_f * 2 * filter_stride(a.nBands), lane);
+  if (algo_uses_isd(algo)) {
     s.advance(2, lane);  // beta (the head kernel turned it into the impulse count)
     const int beg = isd_off[u], n = isd_off[u + 1] - beg;
     shuffle_scan_warp(s, L, jseq_all + (size_t)u * jld, cuts_all + (size_t)u * cuts_ld, dupset[warp], lane);
@@ -248,7 +245,7 @@ plan_body_kernel(rb_args a, int algo, int B, int ld, int jld, const int32_t* __r
       }
     }
   }
-  if (uses_ssi(algo)) {
+  if (algo_uses_ssi(algo)) {
     // np.random.normal(0, 1, L): legacy polar Box-Muller; every attempt uses four words and yields two values
     float* row = ssi_noise + (size_t)u * ld;
     const uint32_t lt = (1u << lane) - 1u;
@@ -653,9 +650,9 @@ DevPlanLayout layout(const rb_args& a, int algo, int B, int ld) {
     off += align_up(n, 256);
     return r;
   };
-  const bool lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
+  const bool lnl = algo_uses_lnl(algo);
+  const bool isd = algo_uses_isd(algo);
+  const bool ssi = algo_uses_ssi(algo);
   const size_t stride = 3 * (size_t)a.nBands + 1, kmax = (size_t)max_taps(a);
   const size_t nl = lnl ? (size_t)B * a.N_f : 0;
   l.lnl_params = take(nl * stride * 8);
@@ -726,9 +723,9 @@ int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* l
                   size_t storage_bytes, rb_plan* plan, cudaStream_t st, const uint32_t* snaps) {
   if (!args || !plan || B < 0 || ld < 0) return RB_ERR_INVALID_ARG;
   memset(plan, 0, sizeof(*plan));
-  const bool lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
+  const bool lnl = algo_uses_lnl(algo);
+  const bool isd = algo_uses_isd(algo);
+  const bool ssi = algo_uses_ssi(algo);
   plan->n_f = lnl ? args->N_f : 0;
   plan->g_sd = (float)args->g_sd;
   if (B == 0 || ld == 0 || !(lnl || isd || ssi)) return RB_OK;
@@ -772,9 +769,7 @@ int devplan_begin(const rb_args* args, int algo, int B, int ld, const int32_t* l
 // Stage 2, utterances [first, first+count): the rest of the stream (swap targets and groups, impulse gains, SSI draws).
 int devplan_body(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds, void* storage, int first,
                  int count, cudaStream_t st, const uint32_t* snaps) {
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
-  if (!(isd || ssi) || count <= 0) return RB_OK;
+  if (!(algo_uses_isd(algo) || algo_uses_ssi(algo)) || count <= 0) return RB_OK;
   const DevPlanLayout l = layout(*args, algo, B, ld);
   char* d = (char*)storage;
   const size_t stride = 3 * (size_t)args->nBands + 1;
@@ -826,8 +821,7 @@ int launch_perm_apply(int count, int ld, int jld, int cuts_ld, const int32_t* le
 // Stage 3, utterances [first, first+count): apply the swaps, emit the impulse positions.
 int devplan_apply(const rb_args* args, int algo, int B, int ld, const int32_t* len, void* storage, int first, int count,
                   cudaStream_t st) {
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  if (!isd || count <= 0) return RB_OK;
+  if (!algo_uses_isd(algo) || count <= 0) return RB_OK;
   const DevPlanLayout l = layout(*args, algo, B, ld);
   char* d = (char*)storage;
   const size_t jbytes = ld > kNarrowMax ? 4 : 2;
@@ -857,8 +851,7 @@ int shuffle_prefix(int B, int ld, const int32_t* len, const uint32_t* snaps, con
 
 // Stage 4 (after stage 2 of ALL utterances): CSR offsets and design of the SSI filters.
 int devplan_end(const rb_args* args, int algo, int B, int ld, void* storage, cudaStream_t st) {
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
-  if (!ssi || B <= 0) return RB_OK;
+  if (!algo_uses_ssi(algo) || B <= 0) return RB_OK;
   const DevPlanLayout l = layout(*args, algo, B, ld);
   char* d = (char*)storage;
   scan_kernel<<<1, 1024, 0, st>>>((const int32_t*)(d + l.ssi_cnt), B, (int32_t*)(d + l.ssi_off));

@@ -23,6 +23,7 @@
 
 #include <cuda_runtime.h>  // cudaMallocHost for the page-locked plan buffers only
 #include "rawboost_b200.h"
+#include "rb_algo.h"
 
 namespace {
 
@@ -353,9 +354,7 @@ void shuffle_legacy(Mt& rng, T* x, int n, std::vector<T>& js) {  // targets are 
 
 // All draws of process_Rawboost_feature for one utterance, in the dispatcher's order: LnL, ISD, SSI.
 void draw_utt(Mt& rng, const Args& a, int algo, int length, UttDraw& out, float* noise_row, Scratch& sc) {
-  const bool lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
+  const bool lnl = rb::algo_uses_lnl(algo), isd = rb::algo_uses_isd(algo), ssi = rb::algo_uses_ssi(algo);
   out.lnl_taps.clear();
   out.lnl_k.clear();
   out.isd_idx.clear();
@@ -479,14 +478,12 @@ int rb_planner_draw(rb_planner* p, const rb_args* args, int algo, int B, int ld,
   if (!p || !args || !view || B < 0 || ld < 0 || (B > 0 && !len)) return RB_ERR_INVALID_ARG;
   if (!seeds && !state) return RB_ERR_INVALID_ARG;
   {  // what the reference's own calls would reject or what has no numpy equivalent here: refuse instead of throwing
-    const bool use_filters = (algo == 1 || algo == 3 || algo == 4 || algo == 5 || algo == 6 || algo == 7 || algo == 8) && algo != 2;
-    const bool use_isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-    if (use_filters) {
+    if (rb::algo_uses_lnl(algo) || rb::algo_uses_ssi(algo)) {
       const double cmin = std::min(args->minCoeff, args->maxCoeff), cmax = std::max(args->minCoeff, args->maxCoeff);
       if (args->nBands < 1 || args->nBands > 1000 || !(cmin >= 1.0) || !(cmax <= 1e6) || !(args->fs > 0.0)) return RB_ERR_UNSUPPORTED;
-      if ((algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8) && (args->N_f < 1 || args->N_f > 1000)) return RB_ERR_UNSUPPORTED;
+      if (rb::algo_uses_lnl(algo) && (args->N_f < 1 || args->N_f > 1000)) return RB_ERR_UNSUPPORTED;
     }
-    if (use_isd && !(args->P >= 0.0)) return RB_ERR_UNSUPPORTED;  // a negative count would mean numpy's "all but the last |n|"
+    if (rb::algo_uses_isd(algo) && !(args->P >= 0.0)) return RB_ERR_UNSUPPORTED;  // a negative count would mean numpy's "all but the last |n|"
   }
   try {
   Args a;
@@ -507,9 +504,7 @@ int rb_planner_draw(rb_planner* p, const rb_args* args, int algo, int B, int ld,
   a.SNRmin = args->SNRmin;
   a.SNRmax = args->SNRmax;
   a.fs = args->fs;
-  const bool lnl = (algo == 1 || algo == 4 || algo == 5 || algo == 6 || algo == 8);
-  const bool isd = (algo == 2 || algo == 4 || algo == 5 || algo == 7 || algo == 8);
-  const bool ssi = (algo == 3 || algo == 4 || algo == 6 || algo == 7);
+  const bool lnl = rb::algo_uses_lnl(algo), isd = rb::algo_uses_isd(algo), ssi = rb::algo_uses_ssi(algo);
   memset(view, 0, sizeof(*view));
   view->n_f = lnl ? a.N_f : 0;
   view->g_sd = (float)a.g_sd;

@@ -469,10 +469,6 @@ class Engine:
         """Utterances per pipeline chunk of the host-buffer entry points (0 = default: four per SM)."""
         _lib.check(self.lib.rb_ctx_set_chunk(self._host_ctx(), int(utterances)), "rb_ctx_set_chunk")
 
-    def set_host_plan_mode(self, mode: int) -> None:
-        """Device planner placement in :meth:`process_host_seeded`: 0 = on its own streams beside the kernels (default), 1 = in line."""
-        _lib.check(self.lib.rb_ctx_set_plan_mode(self._host_ctx(), int(mode)), "rb_ctx_set_plan_mode")
-
     def process_host_seeded(self, algo: int, x: np.ndarray, lengths: np.ndarray, seeds, sr, args,
                             out: Optional[np.ndarray] = None) -> np.ndarray:
         """Host waveforms in, host results out, plans drawn ON THE DEVICE from per-utterance seeds
@@ -499,16 +495,7 @@ class Engine:
         float32) must stay alive and untouched until :meth:`wait_host` has returned for the ticket."""
         if x.dtype != np.float32 or x.ndim != 2 or not x.flags.c_contiguous or out.dtype != np.float32 or out.shape != x.shape:
             raise ValueError("x / out must be C-contiguous [B, ld] float32 arrays of the same shape")
-        if lengths.dtype != np.int32 or seeds.dtype != np.uint32 or not lengths.flags.c_contiguous or not seeds.flags.c_contiguous:
-            raise ValueError("lengths must be a contiguous int32 array and seeds a contiguous uint32 array")
-        B, ld = x.shape
-        a = _lib.args_struct(args, sr)
-        ticket = C.c_uint64(0)
-        rc = self.lib.rb_submit_host_seeded(self._host_ctx(), int(algo), C.byref(a), C.c_void_p(x.ctypes.data),
-                                            C.c_void_p(lengths.ctypes.data), C.c_void_p(seeds.ctypes.data), B, ld,
-                                            C.c_void_p(out.ctypes.data), C.byref(ticket))
-        _lib.check(rc, f"rb_submit_host_seeded(algo={algo})")
-        return int(ticket.value)
+        return self._submit(algo, x, _lib.RB_IO_HOST_F32, lengths, seeds, out.ctypes.data, _lib.RB_IO_HOST_F32, sr, args)
 
     def submit_host_ex(self, algo: int, x: np.ndarray, dtype: str, lengths: np.ndarray, seeds: np.ndarray, sr, args, out) -> int:
         """General streaming submit (``rb_submit_seeded_ex``) for host input: ``dtype`` "f32" (float32 waveforms) or "pcm16"
@@ -518,8 +505,6 @@ class Engine:
         want = np.int16 if dtype == "pcm16" else np.float32
         if x.dtype != want or x.ndim != 2 or not x.flags.c_contiguous:
             raise ValueError(f"x must be a C-contiguous [B, ld] {np.dtype(want).name} array")
-        if lengths.dtype != np.int32 or seeds.dtype != np.uint32 or not lengths.flags.c_contiguous or not seeds.flags.c_contiguous:
-            raise ValueError("lengths must be a contiguous int32 array and seeds a contiguous uint32 array")
         B, ld = x.shape
         if torch.is_tensor(out):
             if out.device != self.device or out.dtype != torch.float32 or tuple(out.shape) != (B, ld) or not out.is_contiguous():
@@ -529,14 +514,8 @@ class Engine:
             if out.dtype != np.float32 or out.shape != (B, ld) or not out.flags.c_contiguous:
                 raise ValueError("out must be a C-contiguous [B, ld] float32 array")
             y_ptr, y_kind = out.ctypes.data, _lib.RB_IO_HOST_F32
-        a = _lib.args_struct(args, sr)
-        ticket = C.c_uint64(0)
-        rc = self.lib.rb_submit_seeded_ex(self._host_ctx(), int(algo), C.byref(a), C.c_void_p(x.ctypes.data),
-                                          _lib.RB_IO_HOST_PCM16 if dtype == "pcm16" else _lib.RB_IO_HOST_F32,
-                                          C.c_void_p(lengths.ctypes.data), C.c_void_p(seeds.ctypes.data), B, ld, C.c_void_p(y_ptr), y_kind,
-                                          None, 0, C.byref(ticket))
-        _lib.check(rc, f"rb_submit_seeded_ex(algo={algo})")
-        return int(ticket.value)
+        x_kind = _lib.RB_IO_HOST_PCM16 if dtype == "pcm16" else _lib.RB_IO_HOST_F32
+        return self._submit(algo, x, x_kind, lengths, seeds, y_ptr, y_kind, sr, args)
 
     def process_device_seeded(self, algo: int, x: torch.Tensor, lengths: torch.Tensor, seeds: torch.Tensor, sr, args,
                               out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -550,15 +529,28 @@ class Engine:
             out = torch.zeros_like(x)
         if seeds.device != self.device or seeds.numel() != B or seeds.element_size() != 4:
             raise ValueError("seeds must be a 32-bit integer tensor [B] on the engine's device")
-        a = _lib.args_struct(args, sr)
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        ticket = C.c_uint64(0)
         with torch.cuda.device(self.device):
-            rc = self.lib.rb_submit_seeded_ex(self._host_ctx(), int(algo), C.byref(a), C.c_void_p(x.data_ptr()), _lib.RB_IO_DEVICE_F32,
-                                              C.c_void_p(lengths.data_ptr()), C.c_void_p(seeds.data_ptr()), B, ld,
-                                              C.c_void_p(out.data_ptr()), _lib.RB_IO_DEVICE_F32, C.c_void_p(stream), 1, C.byref(ticket))
-        _lib.check(rc, f"rb_submit_seeded_ex(device, algo={algo})")
+            self._submit(algo, x, _lib.RB_IO_DEVICE_F32, lengths, seeds, out.data_ptr(), _lib.RB_IO_DEVICE_F32, sr, args, stream)
         return out
+
+    def _submit(self, algo: int, x, x_kind: int, lengths, seeds, y_ptr: int, y_kind: int, sr, args, stream=None) -> int:
+        """Queue one ``rb_submit_seeded_ex`` call and return its ticket. ``x``, ``lengths`` and ``seeds`` are host arrays, or
+        device tensors whose call is ordered against ``stream`` (a ``cudaStream_t``). The call reads them after it returns, so
+        host lengths and seeds must already have the exact dtypes: a converted copy would not live long enough."""
+        if stream is None:
+            if lengths.dtype != np.int32 or seeds.dtype != np.uint32 or not lengths.flags.c_contiguous or not seeds.flags.c_contiguous:
+                raise ValueError("lengths must be a contiguous int32 array and seeds a contiguous uint32 array")
+            xp, lp, sp = (C.c_void_p(a.ctypes.data) for a in (x, lengths, seeds))
+        else:
+            xp, lp, sp = (_ptr(t) for t in (x, lengths, seeds))
+        B, ld = x.shape
+        a = _lib.args_struct(args, sr)
+        ticket = C.c_uint64(0)
+        rc = self.lib.rb_submit_seeded_ex(self._host_ctx(), int(algo), C.byref(a), xp, x_kind, lp, sp, B, ld, C.c_void_p(y_ptr), y_kind,
+                                          C.c_void_p(stream), int(stream is not None), C.byref(ticket))
+        _lib.check(rc, f"rb_submit_seeded_ex(algo={algo})")
+        return int(ticket.value)
 
     def wait_host(self, ticket: int = 0) -> None:
         """Block until the submitted call ``ticket`` (0: every submitted call) has delivered its results."""

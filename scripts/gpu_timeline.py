@@ -14,8 +14,6 @@ y = torch.empty((B, L), dtype=torch.float32).pin_memory()
 lengths = np.full(B, L, np.int32)
 seeds = np.array([workload.seed_for(u) for u in range(B)], np.uint32)
 eng.set_host_chunk(chunk)
-if len(sys.argv) > 2:
-    eng.set_host_plan_mode(int(sys.argv[2]))
 for i in range(3):
     t0 = time.perf_counter(); eng.process_host_seeded(5, x.numpy(), lengths, seeds, 16000, args, out=y.numpy()); print("ms", 1e3 * (time.perf_counter() - t0))
 eng.trace_host(True)

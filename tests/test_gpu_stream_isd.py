@@ -1,5 +1,5 @@
 """The streaming normWav / ISD pass (norm_stream_kernel in rb_dense.cu) on hand-placed inputs, the chained algos by composition,
-the impulse mask past its shared-memory limit, and the pipelined host entries in both planner placements.
+the impulse mask past its shared-memory limit, and the pipelined host entry with its device planner.
 
 norm_stream_kernel runs algo 2, the ISD stage of algo 7, the ISD branch and the final sum of algo 8, rb_normwav and the last
 normalisation of rb_reverb. Tile CTAs copy 32 768 samples each and take their peak; a finisher CTA per row applies the impulses
@@ -746,7 +746,7 @@ def test_device_plan_on_rows_past_the_shared_mask(eng, algo):
             assert ulp_err(getattr(got, name), r) <= 1.0, f"algo {algo}: {name} more than 1 ulp(fp32) from numpy"
 
 
-# ---- the pipelined host entries in both planner placements -------------------------------------------------------------------
+# ---- the pipelined host entry with the device planner -------------------------------------------------------------------------
 HOST_B, HOST_LD, HOST_CHUNK = 8192, 2000, 1024  # 8 chunks; without SSI the planner runs in 4 pieces (1, 1, 4 and 2 chunks)
 
 
@@ -763,30 +763,25 @@ def host_batch():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("algo", range(9))
-def test_pipelined_host_entry_plan_modes(eng, host_batch, algo):
-    """rb_process_host_seeded with the device planner in line (mode 1) == beside the kernels (mode 0), bit for bit, and both ==
-    rb_process on host-drawn plans: bit-exact for algos 0 and 2, within 1e-5 otherwise (taps and noise may differ by 1 ulp)."""
+def test_pipelined_host_entry_matches_rb_process(eng, host_batch, algo):
+    """rb_process_host_seeded, its device planner issued in pieces beside the kernels, == rb_process on host-drawn plans:
+    bit-exact for algos 0 and 2, within 1e-5 otherwise (taps and noise may differ by 1 ulp)."""
     import torch
     from scl_deepfake_audio_detection_b200.native_planner import NativePlanner
     x, lengths, seeds = host_batch
-    got = {}
     eng.set_host_chunk(HOST_CHUNK)
     try:
-        for mode in (0, 1):
-            eng.set_host_plan_mode(mode)
-            got[mode] = eng.process_host_seeded(algo, x, lengths, seeds, SR, ARGS)
+        got = eng.process_host_seeded(algo, x, lengths, seeds, SR, ARGS)
     finally:
-        eng.set_host_plan_mode(0)
         eng.set_host_chunk(0)
     inside = np.arange(HOST_LD)[None, :] < lengths[:, None]
-    assert np.array_equal(bits(got[0])[inside], bits(got[1])[inside]), f"algo {algo}: plan mode 1 differs from mode 0"
     plan = NativePlanner(threads=0, pinned=False).draw(lengths, SR, ARGS, algo, seeds=seeds, ld=HOST_LD, copy=True) if algo else None
     xd, ln = to_dev(x, lengths)
     ref = eng.process(algo, xd, ln, eng.upload_plan(plan) if plan is not None else None)
     torch.cuda.synchronize()
     ref = ref.cpu().numpy()
     if algo in (0, 2):
-        assert np.array_equal(bits(got[0])[inside], bits(ref)[inside]), f"algo {algo}: seeded host entry differs from rb_process"
+        assert np.array_equal(bits(got)[inside], bits(ref)[inside]), f"algo {algo}: seeded host entry differs from rb_process"
     else:
-        err = float(np.max(np.abs(got[0][inside].astype(np.float64) - ref[inside])))
+        err = float(np.max(np.abs(got[inside].astype(np.float64) - ref[inside])))
         assert err <= 1e-5, f"algo {algo}: seeded host entry {err:.3g} from rb_process"
