@@ -312,6 +312,30 @@ RB_API int rb_submit_seeded_ex(rb_ctx* ctx, int algo, const rb_args* args, const
                                const uint32_t* seeds, int B, int ld, void* y, int y_kind, void* user_stream, int use_user_stream,
                                uint64_t* ticket);
 
+/* Ragged host batches packed back to back: utterance u is x[off[u] .. off[u+1]), so the copies carry the real samples only
+ * (a padded [B, ld] batch of un-cropped utterances moves ld / mean(len) times as many). Seeded semantics, chunking, the device
+ * planner, use_user_stream and the two-calls-in-flight rule are those of rb_submit_seeded_ex; rb_ctx_wait(ctx, ticket) is the
+ * blocking form.
+ *   x_kind  RB_IO_HOST_F32 (float32) or RB_IO_HOST_PCM16 (int16, converted on the device as sample / 32768), packed, any alignment
+ *   off     HOST int64[B + 1]: off[0] == 0, non-decreasing, every length off[u+1] - off[u] <= INT32_MAX. Checked at call time:
+ *           RB_ERR_INVALID_ARG otherwise. A zero-length utterance is legal and occupies no bytes. int64, because a shard of long
+ *           utterances exceeds 2^31 samples.
+ *   y_kind  RB_IO_HOST_F32    y = host float32, packed at the same offsets as x; only y[off[0] .. off[B]) is written.
+ *                             ld == 0: the rows the kernels see have stride round_up(max len, 4); ld > 0: that stride (ld % 4 == 0,
+ *                             ld >= max len)
+ *           RB_IO_DEVICE_F32  y = device float32 rows [B, ld] (16-byte aligned), what rb_multiview_assemble_ex and rb_process take:
+ *                             ld is required, >= max len and a multiple of 4 (RB_ERR_INVALID_ARG / RB_ERR_ALIGNMENT otherwise)
+ * The results equal rb_submit_seeded_ex's on the same utterances zero-padded to rows of the same ld, bit for bit.
+ * Per chunk, the driver issues one copy of the chunk's packed span each way; kernels unpack it into zero-padded rows and (host
+ * sink) pack the results. Traffic (rb_ctx_last_traffic), with e = 4 for float32 and 2 for PCM16 input:
+ *   host->device  e * off[B] + 8 * (B + 1) (the offsets) + 4 * B (the seeds; not uploaded for an algo outside 1..8)
+ *   device->host  4 * off[B] with a host sink, 0 with a device sink
+ * x, off, seeds and y stay valid and untouched until the call has completed. Page-locked x, off and y keep the copies
+ * asynchronous: a pageable off makes its upload wait for the copy stream. */
+RB_API int rb_submit_seeded_packed(rb_ctx* ctx, int algo, const rb_args* args, const void* x, int x_kind, const int64_t* off,
+                                   const uint32_t* seeds, int B, int ld, void* y, int y_kind, void* user_stream, int use_user_stream,
+                                   uint64_t* ticket);
+
 /* ---- measurement helpers (bench.py) ---------------------------------------------------------------------
  * rb_probe_fp32: runs a register-resident FFMA2 (packed=1) or FFMA (packed=0) chain on every SM and
  * returns the achieved FLOP count in *flops; the caller times it with events on `stream`.

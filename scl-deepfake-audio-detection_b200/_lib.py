@@ -22,6 +22,7 @@ SYMBOLS = (
     "rb_ctx_set_chunk", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
     "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
     "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run", "rb_items_stream_draw", "rb_items_stream_run",
+    "rb_submit_seeded_packed",
 )
 RB_IO_HOST_F32, RB_IO_HOST_PCM16, RB_IO_DEVICE_F32 = 0, 1, 2
 
@@ -136,6 +137,9 @@ def load() -> C.CDLL:
     lib.rb_multiview_assemble_ex.argtypes = [vp, vp, vp, vp, i32, i32, i32, vp, i32, i32, i32, vp, vp, vp, vp, vp]
     lib.rb_submit_seeded_ex.restype = i32
     lib.rb_submit_seeded_ex.argtypes = [vp, i32, C.POINTER(RbArgs), vp, i32, vp, vp, i32, i32, vp, i32, vp, i32, C.POINTER(C.c_uint64)]
+    lib.rb_submit_seeded_packed.restype = i32
+    lib.rb_submit_seeded_packed.argtypes = [vp, i32, C.POINTER(RbArgs), vp, i32, vp, vp, i32, i32, vp, i32, vp, i32,
+                                            C.POINTER(C.c_uint64)]
     lib.rb_reverb_workspace_bytes.restype = sz
     lib.rb_reverb_workspace_bytes.argtypes = [i32, i32]
     lib.rb_reverb.restype = i32

@@ -369,6 +369,7 @@ struct IoSpec {
   int y_kind = RB_IO_HOST_F32;   // RB_IO_HOST_F32 | RB_IO_DEVICE_F32
   cudaStream_t user = nullptr;   // device-side ordering: the call starts after the work queued on it and (has_user) it waits for the call
   bool has_user = false;
+  const int64_t* off = nullptr;  // packed host I/O: utterance u is x[off[u], off[u + 1]) (host int64[B + 1]); a host y is packed alike
 };
 
 // Events of a traced synchronous call (rb_ctx_trace): [0] its start, [1..4] per chunk: copy-in, plan, kernels, copy-out done.
@@ -542,6 +543,8 @@ int queue_devplan(rb_ctx* c, CallRes& R, const rb_args* args, int algo, int B, i
 int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int B, int ld, const rb_plan* plan, const rb_args* args,
                  const uint32_t* seeds, bool async, uint64_t* ticket) {
   const bool x_dev = io.x_kind == RB_IO_DEVICE_F32, x_pcm = io.x_kind == RB_IO_HOST_PCM16, y_dev = io.y_kind == RB_IO_DEVICE_F32;
+  const bool packed = io.off != nullptr;
+  const size_t elem = x_pcm ? 2 : 4;
   const float* x = (const float*)io.x;
   float* y = (float*)io.y;
   RB_CUDA(cudaSetDevice(c->device));
@@ -562,10 +565,12 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
   const int nchunks = (int)first.size() - 1;
 
   // everything queued below is ordered by events only; the host blocks once, at the end
-  // per-call metadata: lengths (+ seeds) for the whole batch
-  RB_TRY(grow(R.meta, R.meta_bytes, align_up((size_t)B * 4, 256) * 2, 0));
+  // per-call metadata: lengths (+ seeds) for the whole batch, and the offsets of packed I/O
+  const size_t meta4 = align_up((size_t)B * 4, 256);
+  RB_TRY(grow(R.meta, R.meta_bytes, meta4 * 2 + (packed ? (size_t)(B + 1) * 8 : 0), 0));
   const int32_t* d_len = (int32_t*)R.meta;
-  const uint32_t* d_seeds = (uint32_t*)(R.meta + align_up((size_t)B * 4, 256));
+  const uint32_t* d_seeds = (uint32_t*)(R.meta + meta4);
+  const int64_t* d_off = (const int64_t*)(R.meta + meta4 * 2);
   uint64_t h2d = 0, d2h = 0;
   if (io.has_user || x_dev) {  // everything of this call comes after what the caller queued on its stream
     RB_CUDA(cudaEventRecord(R.ev_user, io.user));
@@ -575,8 +580,14 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
     d_len = len;
     d_seeds = seeds;
   } else {
-    RB_CUDA(cudaMemcpyAsync((void*)d_len, len, (size_t)B * 4, cudaMemcpyHostToDevice, c->s_in));
-    h2d += (size_t)B * 4;
+    if (packed) {  // the offsets go up from the caller's buffer; the lengths are their differences
+      RB_CUDA(cudaMemcpyAsync((void*)d_off, io.off, (size_t)(B + 1) * 8, cudaMemcpyHostToDevice, c->s_in));
+      h2d += (size_t)(B + 1) * 8;
+      RB_TRY(launch_lengths_from_offsets(d_off, B, (int32_t*)d_len, c->s_in));
+    } else {
+      RB_CUDA(cudaMemcpyAsync((void*)d_len, len, (size_t)B * 4, cudaMemcpyHostToDevice, c->s_in));
+      h2d += (size_t)B * 4;
+    }
     if (devplan) {
       RB_CUDA(cudaMemcpyAsync((void*)d_seeds, seeds, (size_t)B * 4, cudaMemcpyHostToDevice, c->s_in));
       h2d += (size_t)B * 4;
@@ -593,7 +604,15 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
   if (devplan && dp_bytes == 0) return RB_ERR_UNSUPPORTED;
   RB_TRY(grow(R.planmem, R.planmem_bytes, dp_bytes, dp_bytes / 8));
   Take take;
-  const size_t o_x = take(x_dev ? 0 : wave), o_x16 = take(x_pcm ? wave / 2 : 0), o_y = take(y_dev ? 0 : wave), o_ws = take(ws_bytes);
+  const size_t o_x = take(x_dev ? 0 : wave), o_x16 = take(x_pcm && !packed ? wave / 2 : 0), o_y = take(y_dev ? 0 : wave);
+  // Packed input is staged in the output rows, which are free until the kernels write them, and packed results in the input
+  // rows, which are free once the kernels are done. A device sink has no output rows: its input gets a staging area sized by
+  // the largest chunk span.
+  size_t max_span = 0;
+  if (packed)
+    for (int ci = 0; ci < nchunks; ++ci) max_span = std::max(max_span, (size_t)(io.off[first[ci + 1]] - io.off[first[ci]]));
+  const size_t o_pin = packed && y_dev ? take(elem * max_span) : o_y, o_pout = o_x;
+  const size_t o_ws = take(ws_bytes);
   HostPlanSlots hp{};
   if (active && !devplan) hp = host_plan_slots(take, plan, algo, first, chunk, ld);
   for (int k = 0; k < std::min(kSlots, nchunks); ++k) {
@@ -610,9 +629,13 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
     char* d = sl.dev;
     const int u0 = first[ci], bc = first[ci + 1] - u0;
     const size_t cw = (size_t)bc * ld * sizeof(float);
+    const int64_t p0 = packed ? io.off[u0] : 0, pn = packed ? io.off[u0 + bc] - p0 : 0;  // the chunk's packed span
     // ---- stage 1: host -> device: the waveforms and, of a host plan, the chunk's slices -------------------------------
     if (c->seq + ci >= kSlots) RB_CUDA(cudaStreamWaitEvent(c->s_in, sl.ev_out, 0));  // the slot's previous chunk has left the device
-    if (x_pcm) {
+    if (packed) {  // one copy of the contiguous span, whatever the number of utterances
+      if (pn) RB_CUDA(cudaMemcpyAsync(d + o_pin, (const char*)io.x + elem * p0, elem * pn, cudaMemcpyHostToDevice, c->s_in));
+      h2d += elem * pn;
+    } else if (x_pcm) {
       RB_CUDA(cudaMemcpyAsync(d + o_x16, (const int16_t*)io.x + (size_t)u0 * ld, cw / 2, cudaMemcpyHostToDevice, c->s_in));
       h2d += cw / 2;
     } else if (!x_dev) {
@@ -628,12 +651,15 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
     if (devplan) RB_CUDA(cudaStreamWaitEvent(c->s_cmp, R.ev_planned[ci], 0));
     else trace.mark(2, c->s_in);
     RB_CUDA(cudaStreamWaitEvent(c->s_cmp, sl.ev_in, 0));
-    if (x_pcm) {
+    if (packed) {
+      RB_TRY(launch_unpack_rows(d + o_pin, x_pcm, d_off + u0, bc, ld, (float*)(d + o_x), c->s_cmp));
+    } else if (x_pcm) {
       RB_TRY(launch_pcm16_to_f32((const int16_t*)(d + o_x16), (float*)(d + o_x), (size_t)bc * ld, c->s_cmp));
     }
     const float* xin = x_dev ? x + (size_t)u0 * ld : (const float*)(d + o_x);
     float* yout = y_dev ? y + (size_t)u0 * ld : (float*)(d + o_y);
     RB_TRY(rb_process(algo, xin, d_len + u0, bc, ld, active ? &dp : nullptr, yout, d + o_ws, ws_bytes, c->s_cmp));
+    if (packed && !y_dev) RB_TRY(launch_pack_rows(yout, d_off + u0, bc, ld, (float*)(d + o_pout), c->s_cmp));
     RB_CUDA(cudaEventRecord(sl.ev_done, c->s_cmp));
     trace.mark(3, c->s_cmp);
     // ---- stage 3: device -> host (or nothing: the results stay where the kernels wrote them) ---------------------------
@@ -641,8 +667,13 @@ int run_pipeline(rb_ctx* c, int algo, const IoSpec& io, const int32_t* len, int 
       RB_CUDA(cudaEventRecord(sl.ev_out, c->s_cmp));
     } else {
       RB_CUDA(cudaStreamWaitEvent(c->s_out, sl.ev_done, 0));
-      RB_CUDA(cudaMemcpyAsync(y + (size_t)u0 * ld, d + o_y, cw, cudaMemcpyDeviceToHost, c->s_out));
-      d2h += cw;
+      if (packed) {
+        if (pn) RB_CUDA(cudaMemcpyAsync(y + p0, d + o_pout, 4 * pn, cudaMemcpyDeviceToHost, c->s_out));
+        d2h += 4 * pn;
+      } else {
+        RB_CUDA(cudaMemcpyAsync(y + (size_t)u0 * ld, d + o_y, cw, cudaMemcpyDeviceToHost, c->s_out));
+        d2h += cw;
+      }
       RB_CUDA(cudaEventRecord(sl.ev_out, c->s_out));
     }
     trace.mark(4, y_dev ? c->s_cmp : c->s_out);
@@ -812,6 +843,36 @@ int rb_submit_host_seeded(rb_ctx* c, int algo, const rb_args* args, const float*
 int rb_submit_seeded_ex(rb_ctx* c, int algo, const rb_args* args, const void* x, int x_kind, const int32_t* len, const uint32_t* seeds,
                         int B, int ld, void* y, int y_kind, void* user_stream, int use_user_stream, uint64_t* ticket) {
   return run_seeded(c, algo, args, x, x_kind, len, seeds, B, ld, y, y_kind, user_stream, use_user_stream, true, ticket);
+}
+
+// The offsets are checked here, on the host, before anything is queued.
+int rb_submit_seeded_packed(rb_ctx* c, int algo, const rb_args* args, const void* x, int x_kind, const int64_t* off,
+                            const uint32_t* seeds, int B, int ld, void* y, int y_kind, void* user_stream, int use_user_stream,
+                            uint64_t* ticket) {
+  if (ticket) *ticket = 0;
+  if (!c || B < 0 || ld < 0) return RB_ERR_INVALID_ARG;
+  if (x_kind != RB_IO_HOST_F32 && x_kind != RB_IO_HOST_PCM16) return RB_ERR_INVALID_ARG;
+  if (y_kind != RB_IO_HOST_F32 && y_kind != RB_IO_DEVICE_F32) return RB_ERR_INVALID_ARG;
+  if (B == 0) return RB_OK;
+  if (!x || !off || !y) return RB_ERR_INVALID_ARG;
+  if (algo >= 1 && algo <= 8 && (!args || !seeds)) return RB_ERR_INVALID_ARG;
+  if (off[0] != 0) return RB_ERR_INVALID_ARG;
+  int64_t max_len = 0;
+  for (int u = 0; u < B; ++u) {
+    const int64_t n = off[u + 1] - off[u];
+    if (n < 0 || n > INT32_MAX) return RB_ERR_INVALID_ARG;
+    max_len = std::max(max_len, n);
+  }
+  if (y_kind == RB_IO_HOST_F32 && ld == 0) {  // the call's own stride
+    if (max_len > INT32_MAX - 3) return RB_ERR_INVALID_ARG;
+    ld = (int)align_up((size_t)max_len, 4);
+  }
+  if (ld < max_len) return RB_ERR_INVALID_ARG;
+  if (ld % 4 != 0 || (y_kind == RB_IO_DEVICE_F32 && ((uintptr_t)y & 15u))) return RB_ERR_ALIGNMENT;
+  if (ld == 0) return RB_OK;  // every utterance is empty
+  IoSpec io{x, x_kind, y, y_kind, (cudaStream_t)user_stream, use_user_stream != 0};
+  io.off = off;
+  return run_pipeline(c, algo, io, nullptr, B, ld, nullptr, args, seeds, true, ticket);
 }
 
 int rb_ctx_wait(rb_ctx* c, uint64_t ticket) {

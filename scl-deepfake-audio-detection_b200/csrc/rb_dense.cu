@@ -364,7 +364,82 @@ pcm16_to_f32_kernel(const int4* __restrict__ in, float4* __restrict__ out, size_
   }
 }
 
+// ---- packed utterances <-> rows [B, ld] ------------------------------------------------------------------------------
+// Row r is packed[off[r] - off[0], off[r + 1] - off[0]). A block covers kPackSpan samples of gridDim.y-strided rows (so any
+// row count fits the grid); a thread moves four samples: one float4 on the 16-byte aligned row side, scalars on the packed
+// side, whose rows start at any sample.
+constexpr int kPackThreads = 256;
+constexpr int kPackSpan = 4 * kPackThreads;
+
+__device__ __forceinline__ float sample_f32(float v) { return v; }
+__device__ __forceinline__ float sample_f32(int16_t v) { return (float)v * (1.f / 32768.f); }  // as pcm16_to_f32_kernel
+
+__global__ void __launch_bounds__(256) lengths_from_offsets_kernel(const int64_t* __restrict__ off, int B, int32_t* __restrict__ len) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < B; i += gridDim.x * blockDim.x) len[i] = (int32_t)(off[i + 1] - off[i]);
+}
+
+// rows[r][0, len) = the packed samples (as float32), rows[r][len, ld) = 0: the rows the padded entry's zero-padded input gives
+template <typename T>
+__global__ void __launch_bounds__(kPackThreads)
+unpack_rows_kernel(const T* __restrict__ packed, const int64_t* __restrict__ off, int B, int ld, float* __restrict__ rows) {
+  const int64_t p = ((int64_t)blockIdx.x * kPackThreads + threadIdx.x) * 4;
+  if (p >= ld) return;
+  const int64_t base = off[0];
+  for (int r = blockIdx.y; r < B; r += gridDim.y) {
+    const int64_t o = off[r] - base, n = off[r + 1] - base - o;
+    const T* src = packed + o + p;
+    float v[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v[k] = p + k < n ? sample_f32(src[k]) : 0.f;
+    *reinterpret_cast<float4*>(rows + (size_t)r * ld + p) = make_float4(v[0], v[1], v[2], v[3]);
+  }
+}
+
+// packed[off[r] - off[0] + i] = rows[r][i] for i < len; nothing else is written
+__global__ void __launch_bounds__(kPackThreads)
+pack_rows_kernel(const float* __restrict__ rows, const int64_t* __restrict__ off, int B, int ld, float* __restrict__ packed) {
+  const int64_t p = ((int64_t)blockIdx.x * kPackThreads + threadIdx.x) * 4;
+  if (p >= ld) return;
+  const int64_t base = off[0];
+  for (int r = blockIdx.y; r < B; r += gridDim.y) {
+    const int64_t o = off[r] - base, n = off[r + 1] - base - o;
+    if (p >= n) continue;
+    const float4 v = *reinterpret_cast<const float4*>(rows + (size_t)r * ld + p);
+    float* dst = packed + o + p;
+    dst[0] = v.x;
+    if (p + 1 < n) dst[1] = v.y;
+    if (p + 2 < n) dst[2] = v.z;
+    if (p + 3 < n) dst[3] = v.w;
+  }
+}
+
+inline dim3 pack_grid(int B, int ld) { return dim3((unsigned)((ld + kPackSpan - 1) / kPackSpan), (unsigned)min(B, 65535)); }
+
 }  // namespace
+
+int launch_lengths_from_offsets(const int64_t* off, int B, int32_t* len, cudaStream_t st) {
+  if (B <= 0) return RB_OK;
+  lengths_from_offsets_kernel<<<(unsigned)min((B + 255) / 256, 148 * 16), 256, 0, st>>>(off, B, len);
+  RB_LAUNCH_CHECK();
+  return RB_OK;
+}
+
+int launch_unpack_rows(const void* packed, bool pcm16, const int64_t* off, int B, int ld, float* rows, cudaStream_t st) {
+  if (B <= 0 || ld <= 0) return RB_OK;
+  if (ld % 4 != 0 || ((uintptr_t)rows & 15u)) return RB_ERR_ALIGNMENT;
+  if (pcm16) unpack_rows_kernel<int16_t><<<pack_grid(B, ld), kPackThreads, 0, st>>>((const int16_t*)packed, off, B, ld, rows);
+  else unpack_rows_kernel<float><<<pack_grid(B, ld), kPackThreads, 0, st>>>((const float*)packed, off, B, ld, rows);
+  RB_LAUNCH_CHECK();
+  return RB_OK;
+}
+
+int launch_pack_rows(const float* rows, const int64_t* off, int B, int ld, float* packed, cudaStream_t st) {
+  if (B <= 0 || ld <= 0) return RB_OK;
+  if (ld % 4 != 0 || ((uintptr_t)rows & 15u)) return RB_ERR_ALIGNMENT;
+  pack_rows_kernel<<<pack_grid(B, ld), kPackThreads, 0, st>>>(rows, off, B, ld, packed);
+  RB_LAUNCH_CHECK();
+  return RB_OK;
+}
 
 int stream_tiles_for(int ld) { return (ld + kSTile - 1) / kSTile; }
 

@@ -517,6 +517,48 @@ class Engine:
         x_kind = _lib.RB_IO_HOST_PCM16 if dtype == "pcm16" else _lib.RB_IO_HOST_F32
         return self._submit(algo, x, x_kind, lengths, seeds, y_ptr, y_kind, sr, args)
 
+    def submit_host_packed(self, algo: int, x: np.ndarray, dtype: str, offsets: np.ndarray, seeds: np.ndarray, sr, args, out) -> int:
+        """Streaming submit of a ragged batch packed back to back (``rb_submit_seeded_packed``): utterance u is
+        ``x[offsets[u]:offsets[u+1]]``, so the copies carry only real samples. ``x``: 1-D float32 ("f32") or int16 ("pcm16")
+        host array of ``offsets[-1]`` samples; ``offsets``: int64 [B+1]; ``seeds``: uint32 [B]. ``out``: a host float32 array
+        [offsets[-1]] that receives the results at the same offsets, or a device tensor [B, ld] (ld % 4 == 0, at least the
+        longest utterance) whose rows receive them. Returns a ticket for :meth:`wait_host`; every buffer must stay alive and
+        untouched until then, and page-locked buffers (:func:`pack_host_utterances`) keep the copies asynchronous."""
+        if dtype not in ("f32", "pcm16"):
+            raise ValueError('dtype must be "f32" or "pcm16"')
+        want = np.int16 if dtype == "pcm16" else np.float32
+        if offsets.dtype != np.int64 or offsets.ndim != 1 or offsets.shape[0] < 1 or not offsets.flags.c_contiguous:
+            raise ValueError("offsets must be a contiguous int64 array [B + 1]")
+        B, total = offsets.shape[0] - 1, int(offsets[-1])
+        if x.dtype != want or x.shape != (total,) or not x.flags.c_contiguous:
+            raise ValueError(f"x must be a contiguous 1-D {np.dtype(want).name} array of offsets[-1] = {total} samples")
+        if seeds.dtype != np.uint32 or seeds.shape != (B,) or not seeds.flags.c_contiguous:
+            raise ValueError("seeds must be a contiguous uint32 array, one seed per utterance")
+        if torch.is_tensor(out):
+            if out.device != self.device or out.dtype != torch.float32 or out.dim() != 2 or out.shape[0] != B or not out.is_contiguous():
+                raise ValueError("a device sink must be a contiguous [B, ld] float32 tensor on the engine's device")
+            y_ptr, y_kind, ld = out.data_ptr(), _lib.RB_IO_DEVICE_F32, int(out.shape[1])
+        else:
+            if out.dtype != np.float32 or out.shape != (total,) or not out.flags.c_contiguous:
+                raise ValueError(f"out must be a contiguous float32 array of offsets[-1] = {total} samples")
+            y_ptr, y_kind, ld = out.ctypes.data, _lib.RB_IO_HOST_F32, 0
+        x_kind = _lib.RB_IO_HOST_PCM16 if dtype == "pcm16" else _lib.RB_IO_HOST_F32
+        a = _lib.args_struct(args, sr)
+        ticket = C.c_uint64(0)
+        rc = self.lib.rb_submit_seeded_packed(self._host_ctx(), int(algo), C.byref(a), C.c_void_p(x.ctypes.data), x_kind,
+                                              C.c_void_p(offsets.ctypes.data), C.c_void_p(seeds.ctypes.data), B, ld, C.c_void_p(y_ptr),
+                                              y_kind, None, 0, C.byref(ticket))
+        _lib.check(rc, f"rb_submit_seeded_packed(algo={algo})")
+        return int(ticket.value)
+
+    def process_host_packed(self, algo: int, x: np.ndarray, dtype: str, offsets: np.ndarray, seeds: np.ndarray, sr, args,
+                            out=None):
+        """Blocking form of :meth:`submit_host_packed`; ``out`` None allocates the packed host result. Returns ``out``."""
+        if out is None:
+            out = np.zeros(int(offsets[-1]), dtype=np.float32)
+        self.wait_host(self.submit_host_packed(algo, x, dtype, offsets, seeds, sr, args, out))
+        return out
+
     def process_device_seeded(self, algo: int, x: torch.Tensor, lengths: torch.Tensor, seeds: torch.Tensor, sr, args,
                               out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Seeded batch that already lives on the device: plans drawn on the device chunk by chunk WHILE the previous chunk is
@@ -587,6 +629,31 @@ class Engine:
             self.close()
         except Exception:
             pass
+
+
+def pack_host_utterances(waves: Sequence[np.ndarray], dtype: str = "f32", pin: bool = True):
+    """1-D utterances -> (flat host array, int64 offsets [B+1]) with utterance u at ``flat[offsets[u]:offsets[u+1]]``: the
+    input of :meth:`Engine.submit_host_packed`. ``dtype`` "f32" (float32) or "pcm16" (the utterances must be int16 already).
+    ``pin``: page-locked memory (needs CUDA), which keeps the pipeline's copies asynchronous."""
+    if dtype not in ("f32", "pcm16"):
+        raise ValueError('dtype must be "f32" or "pcm16"')
+    if dtype == "pcm16" and any(np.asarray(w).dtype != np.int16 for w in waves):
+        raise ValueError("pcm16 utterances must be int16 arrays")
+    offsets = np.zeros(len(waves) + 1, dtype=np.int64)
+    np.cumsum([int(np.asarray(w).shape[0]) for w in waves], out=offsets[1:])
+    total = int(offsets[-1])
+    if pin:
+        flat = torch.empty(total, dtype=torch.int16 if dtype == "pcm16" else torch.float32).pin_memory().numpy()
+    else:
+        flat = np.empty(total, dtype=np.int16 if dtype == "pcm16" else np.float32)
+    for u, w in enumerate(waves):
+        flat[offsets[u]:offsets[u + 1]] = w
+    return flat, offsets
+
+
+def split_packed(flat: np.ndarray, offsets: np.ndarray):
+    """Per-utterance views ``flat[offsets[u]:offsets[u+1]]`` of a packed result (no copies)."""
+    return [flat[int(offsets[u]):int(offsets[u + 1])] for u in range(len(offsets) - 1)]
 
 
 _default: dict = {}
