@@ -284,6 +284,47 @@ RB_API int rb_items_stream_run(const rb_args* args, int S, const int32_t* stream
                                const int32_t* indices, const uint32_t* start_state, float* out, int32_t* out_len, float* labels,
                                uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream);
 
+/* The same items from a packed corpus: rows stored back to back, each from a 16-byte chunk boundary, as float32 samples or as
+ * 16-bit PCM, in device memory or read in place from page-locked host memory. A padded corpus stores every row at the length of
+ * the longest; for a ragged corpus the packed form needs a fraction of that (ASVspoof 2019 LA train with three vocoders at the
+ * lengths the loaders read: 8.71 GB padded, 2.94 GB packed float32, 1.47 GB packed PCM16; 0 device bytes in host memory).
+ *   samples  16-byte aligned: device memory of the calling device, or page-locked host memory (cudaHostAlloc / cudaHostRegister,
+ *            e.g. a torch pin_memory tensor), read in place by the gather kernel, 2 or 4 bytes per sample used
+ *   kind     RB_CORPUS_F32 (float32) or RB_CORPUS_PCM16 (int16, read as sample / 32768: what librosa returns for 16-bit audio,
+ *            exact in float32)
+ *   rows     R = N * (1 + nvoc); row order exactly as rb_items_run's corpus
+ *   chunks   size of `samples` in 16-byte chunks
+ *   start    DEVICE int64[R]: row r begins at byte 16 * start[r] of samples
+ *   len      DEVICE int32[R]: samples in row r, >= 1 (what rb_items_draw / rb_items_stream_draw take as corpus_len)
+ * Every other argument, output and the workspace (rb_items_workspace_bytes) mean what they mean for rb_items_run /
+ * rb_items_stream_run; ld is the row stride of the gathered batch only: a multiple of 4 and >= the longest len the items use.
+ * When the corpus holds the float values of a padded corpus (k / 32768 for PCM16), the results equal the padded entries' bit for
+ * bit. Checked on the host before anything is launched, after the checks of the padded entries (G == 0 returns RB_OK first):
+ * RB_ERR_INVALID_ARG for a NULL corpus, samples, start or len, an unknown kind, rows != N * (1 + nvoc) or chunks < 0;
+ * RB_ERR_ALIGNMENT for samples not 16-byte aligned; RB_ERR_INVALID_ARG for samples that are neither device memory of the current
+ * device nor page-locked host memory (pageable memory, another device's memory, no allocation at all).
+ * start and len are device data the host cannot check, so they are read defensively: chunk reads are clamped to [0, chunks)
+ * and a row longer than ld is processed as ld samples. The items such a table describes get unspecified values; nothing is ever
+ * read or written out of bounds. */
+#define RB_CORPUS_F32 0   /* float32 samples                                */
+#define RB_CORPUS_PCM16 1 /* int16 samples, read as sample / 32768 (exact)  */
+typedef struct rb_corpus {
+  const void* samples;
+  int32_t kind;
+  int32_t rows;
+  int64_t chunks;
+  const int64_t* start;
+  const int32_t* len;
+} rb_corpus;
+RB_API int rb_items_run_packed(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad,
+                               int layout, const rb_corpus* corpus, const int32_t* indices, const uint32_t* seeds, float* out,
+                               int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes,
+                               void* stream);
+RB_API int rb_items_stream_run_packed(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N,
+                                      int ld, int trim, int repeat_pad, int layout, const rb_corpus* corpus,
+                                      const int32_t* indices, const uint32_t* start_state, float* out, int32_t* out_len,
+                                      float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Streaming form of rb_process_host_seeded: queues the whole call and returns at once; *ticket identifies it. Up to two calls
  * may be in flight (a third submit first waits for the oldest), so the copies of consecutive batches follow each other
  * without a gap and steady-state throughput is bound by PCIe alone. x, len, seeds and y must stay valid -- and y must not

@@ -22,9 +22,10 @@ SYMBOLS = (
     "rb_ctx_set_chunk", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
     "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
     "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run", "rb_items_stream_draw", "rb_items_stream_run",
-    "rb_submit_seeded_packed",
+    "rb_submit_seeded_packed", "rb_items_run_packed", "rb_items_stream_run_packed",
 )
 RB_IO_HOST_F32, RB_IO_HOST_PCM16, RB_IO_DEVICE_F32 = 0, 1, 2
+RB_CORPUS_F32, RB_CORPUS_PCM16 = 0, 1
 
 
 class RawBoostLibraryError(RuntimeError):
@@ -53,6 +54,12 @@ class RbArgs(C.Structure):
     _fields_ = [("N_f", C.c_int32), ("nBands", C.c_int32)] + [(n, C.c_double) for n in (
         "minF", "maxF", "minBW", "maxBW", "minCoeff", "maxCoeff", "minG", "maxG", "minBiasLinNonLin", "maxBiasLinNonLin",
         "P", "g_sd", "SNRmin", "SNRmax", "fs")]
+
+
+class RbCorpus(C.Structure):
+    """``struct rb_corpus``: a packed corpus (rows from 16-byte chunk boundaries) for the ``_packed`` item entries."""
+    _fields_ = [("samples", C.c_void_p), ("kind", C.c_int32), ("rows", C.c_int32), ("chunks", C.c_int64), ("start", C.c_void_p),
+                ("len", C.c_void_p)]
 
 
 class RbRngState(C.Structure):
@@ -173,6 +180,12 @@ def load() -> C.CDLL:
     lib.rb_items_stream_run.restype = i32
     lib.rb_items_stream_run.argtypes = [C.POINTER(RbArgs), i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp,
                                         vp, vp, sz, vp]
+    lib.rb_items_run_packed.restype = i32
+    lib.rb_items_run_packed.argtypes = [C.POINTER(RbArgs), i32, i32, i32, i32, i32, i32, i32, i32, C.POINTER(RbCorpus), vp, vp, vp, vp,
+                                        vp, vp, vp, sz, vp]
+    lib.rb_items_stream_run_packed.restype = i32
+    lib.rb_items_stream_run_packed.argtypes = [C.POINTER(RbArgs), i32, vp, i32, i32, i32, i32, i32, i32, i32, i32, C.POINTER(RbCorpus),
+                                               vp, vp, vp, vp, vp, vp, vp, sz, vp]
     if lib.rb_abi_version() != RB_ABI_VERSION:
         raise RawBoostLibraryError(f"ABI mismatch: library {lib.rb_abi_version()}, binding {RB_ABI_VERSION}; rebuild")
     _lib = lib

@@ -19,9 +19,13 @@
 //   shuffle_prefix applies the choice permutations.
 //   items_rows_kernel    the batch's source rows in the corpus, their lengths, the view table of the assembly, the label vector
 //   items_gather_kernel  one CTA per batch row: corpus row -> batch row (rb_items_run / rb_items_stream_run only)
-// The run entries then finish with rb_process(5) and rb_multiview_assemble_ex, exactly as ItemBatcher does.
+//   items_gather_packed_kernel  the same from a packed corpus (the _packed run entries): float32 or PCM16 rows from 16-byte
+//                        chunk boundaries, in device memory or in page-locked host memory
+// The run entries then finish with rb_process(5) and rb_multiview_assemble_ex, exactly as ItemBatcher does; the padded and the
+// packed entries share all of it and differ only in the gather they launch.
 //
 // Corpus layout: rows [R, ld], R = N * (1 + nvoc); row idx is bona fide utterance idx, row N + idx*nvoc + v is vocoder v's copy.
+// A packed corpus has the same rows, each at its own length.
 // Batch layout (ItemBatcher's): rows g*(nvoc+1) + v hold item g's vocoded copies (v < nvoc) and its anchor (v = nvoc); rows
 // G*(nvoc+1) + g*n_add + k hold its additional bona fide utterances (not augmented).
 #include <limits.h>
@@ -114,8 +118,10 @@ items_stream_walk_kernel(rb_args a, int S, const int32_t* __restrict__ stream_of
   if (end_state) s.store(end_state + (size_t)q * kMtSnapWords, lane);
 }
 
+// row_len is clamped to [0, ld]: a corpus length table that names a row longer than the batch stride (a packed corpus's len is
+// device data nothing checks against ld) gets that row processed as ld samples; valid lengths pass unchanged
 __global__ void __launch_bounds__(256)
-items_rows_kernel(int G, int nvoc, int n_add, int N, const int32_t* __restrict__ corpus_len, const int32_t* __restrict__ indices,
+items_rows_kernel(int G, int nvoc, int n_add, int N, int ld, const int32_t* __restrict__ corpus_len, const int32_t* __restrict__ indices,
                   const int32_t* __restrict__ choice, int32_t* __restrict__ src_row, int32_t* __restrict__ row_len,
                   int32_t* __restrict__ view_row, float* __restrict__ view_label) {
   const int U = nvoc + 1, V = 2 + n_add + 2 * nvoc;
@@ -134,7 +140,7 @@ items_rows_kernel(int G, int nvoc, int n_add, int N, const int32_t* __restrict__
       src = c + (c >= idx ? 1 : 0);  // position in others = list(range(N)) without idx
     }
     src_row[r] = src;
-    row_len[r] = corpus_len[src];
+    row_len[r] = min(max(corpus_len[src], 0), ld);
   }
   // view order of Dataset_for (line 133): anchor, augmented anchor, additional bona fide, vocoded, augmented vocoded; a row
   // r >= 0 is read from the batch, -1-r from its RawBoost results
@@ -159,6 +165,72 @@ items_gather_kernel(const float* __restrict__ corpus, int ld, const int32_t* __r
   float4* dst = reinterpret_cast<float4*>(x + r * ld);
   const int n4 = (row_len[r] + 3) >> 2;  // the row's padding up to ld is never read
   for (int k = threadIdx.x; k < n4; k += blockDim.x) dst[k] = __ldg(src + k);
+}
+
+// Packed corpus (rb_corpus) -> batch rows. Row r of the batch is read from 16-byte chunk start[src_row[r]] on, ceil(len * e / 16)
+// chunks (e = 4 bytes per float32 sample, 2 per PCM16 sample); the samples past len in the row's last float4 are written as
+// zeros, as a padded corpus holds them. Reading page-locked host memory over PCIe, the rate depends on how many 16-byte loads
+// are in flight, so every thread issues kGatherU independent loads before its stores. The work is (row, segment of
+// kGatherSegChunks chunks), grid-stride, so that long and short rows alike spread over the whole GPU; a segment past its row's
+// end returns at once. Chunk reads are clamped to [0, chunks): a malformed start table reads wrong samples, never outside the
+// corpus. row_len is already within [0, ld] (items_rows_kernel).
+constexpr int kGatherThreads = 256, kGatherU = 8;
+constexpr int kGatherStep = kGatherThreads * kGatherU;  // chunks per pass of a CTA
+constexpr int kGatherSegChunks = 4 * kGatherStep;       // chunks per work item
+
+__device__ __forceinline__ float pcm16_lo(uint32_t w) { return (float)(short)(w & 0xffffu) * (1.f / 32768.f); }  // as rb_dense.cu
+__device__ __forceinline__ float pcm16_hi(uint32_t w) { return (float)(short)(w >> 16) * (1.f / 32768.f); }
+
+template <bool PCM16>
+__global__ void __launch_bounds__(kGatherThreads)
+items_gather_packed_kernel(const uint4* __restrict__ samples, int64_t chunks, const int64_t* __restrict__ start,
+                           const int32_t* __restrict__ src_row, const int32_t* __restrict__ row_len, int ld, size_t rows, int segs,
+                           float* __restrict__ x) {
+  constexpr int E = PCM16 ? 8 : 4;  // samples per chunk
+  const size_t work = rows * (size_t)segs;
+  for (size_t b = blockIdx.x; b < work; b += gridDim.x) {
+    const size_t r = b / (size_t)segs;
+    const int seg = (int)(b - r * (size_t)segs);
+    const int n = row_len[r];
+    const int nc = (n + E - 1) / E, n4 = (n + 3) >> 2;
+    const int c_end = min(nc, (seg + 1) * kGatherSegChunks);
+    if (seg * kGatherSegChunks >= c_end) continue;  // uniform over the CTA
+    const int64_t base = min(max(start[src_row[r]], (int64_t)0), chunks);
+    float4* dst = reinterpret_cast<float4*>(x + r * (size_t)ld);
+    for (int c0 = seg * kGatherSegChunks; c0 < c_end; c0 += kGatherStep) {
+      uint4 v[kGatherU];
+#pragma unroll
+      for (int j = 0; j < kGatherU; ++j) {
+        const int c = c0 + j * kGatherThreads + threadIdx.x;
+        v[j] = make_uint4(0u, 0u, 0u, 0u);
+        if (c < c_end && chunks > 0) v[j] = __ldcs(samples + min(base + c, chunks - 1));
+      }
+#pragma unroll
+      for (int j = 0; j < kGatherU; ++j) {
+        const int c = c0 + j * kGatherThreads + threadIdx.x;
+        if (c >= c_end) continue;
+        float f[E];
+        if constexpr (PCM16) {
+          const uint32_t w[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+#pragma unroll
+          for (int k = 0; k < 4; ++k) f[2 * k] = pcm16_lo(w[k]), f[2 * k + 1] = pcm16_hi(w[k]);
+        } else {
+          f[0] = __uint_as_float(v[j].x), f[1] = __uint_as_float(v[j].y), f[2] = __uint_as_float(v[j].z), f[3] = __uint_as_float(v[j].w);
+        }
+        if ((c + 1) * E > n) {  // the row's last chunk: zeros past len
+#pragma unroll
+          for (int k = 0; k < E; ++k)
+            if (c * E + k >= n) f[k] = 0.f;
+        }
+        if constexpr (PCM16) {
+          dst[2 * c] = make_float4(f[0], f[1], f[2], f[3]);
+          if (2 * c + 1 < n4) dst[2 * c + 1] = make_float4(f[4], f[5], f[6], f[7]);
+        } else {
+          dst[c] = make_float4(f[0], f[1], f[2], f[3]);
+        }
+      }
+    }
+  }
 }
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -251,7 +323,7 @@ int items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, i
     return rc;
   const size_t work = (size_t)G * (nvoc + 1 + n_add) + (size_t)G * (2 + n_add + 2 * nvoc);
   const int grid = (int)std::min<size_t>((work + 255) / 256, 148 * 8);
-  items_rows_kernel<<<grid, 256, 0, st>>>(G, nvoc, n_add, N, corpus_len, indices, (const int32_t*)(d + l.cpos), src_row, row_len,
+  items_rows_kernel<<<grid, 256, 0, st>>>(G, nvoc, n_add, N, ld, corpus_len, indices, (const int32_t*)(d + l.cpos), src_row, row_len,
                                          (int32_t*)(d + l.view_row), (float*)(d + l.view_label));
   RB_LAUNCH_CHECK();
   void* pm = d + l.plan;
@@ -277,30 +349,90 @@ int draw_entry(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, i
                     (char*)workspace, l, plan, (cudaStream_t)stream);
 }
 
+// Where the batch rows are gathered from: a padded float32 matrix [R, ld] with its lengths (rb_items_run / rb_items_stream_run)
+// or a packed corpus (the _packed entries).
+struct CorpusSource {
+  bool is_packed;
+  const float* padded;
+  const int32_t* padded_len;
+  const rb_corpus* packed;
+
+  const int32_t* len() const { return is_packed ? packed->len : padded_len; }
+  // RB_OK, or the error of the host-side checks that need no CUDA call
+  int check(int N, int nvoc) const {
+    if (!is_packed) {
+      if (!padded || !padded_len) return RB_ERR_INVALID_ARG;
+      return ((uintptr_t)padded & 15u) ? RB_ERR_ALIGNMENT : RB_OK;
+    }
+    if (!packed) return RB_ERR_INVALID_ARG;
+    const rb_corpus& c = *packed;
+    if (!c.samples || !c.start || !c.len || (c.kind != RB_CORPUS_F32 && c.kind != RB_CORPUS_PCM16)) return RB_ERR_INVALID_ARG;
+    if ((int64_t)c.rows != (int64_t)N * (1 + nvoc) || c.chunks < 0) return RB_ERR_INVALID_ARG;
+    return ((uintptr_t)c.samples & 15u) ? RB_ERR_ALIGNMENT : RB_OK;
+  }
+};
+
+// The address at which the device reads a packed corpus's samples: the pointer itself for device memory of the current device,
+// the mapped device pointer for page-locked host memory; nullptr for anything else (pageable memory, another device's memory,
+// no allocation).
+const void* corpus_device_ptr(const void* p) {
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();  // an unknown pointer is an argument error, not a sticky one
+    return nullptr;
+  }
+  int dev = -1;
+  if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
+  if (at.type == cudaMemoryTypeDevice) return at.device == dev ? p : nullptr;
+  if (at.type == cudaMemoryTypeHost) return at.devicePointer;
+  return nullptr;
+}
+
+int gather_packed(const rb_corpus& c, const void* samples, int ld, const int32_t* src_row, const int32_t* row_len, int rows,
+                  float* x, cudaStream_t st) {
+  const int e = c.kind == RB_CORPUS_PCM16 ? 8 : 4;  // samples per chunk
+  const int segs = ((ld + e - 1) / e + kGatherSegChunks - 1) / kGatherSegChunks;
+  const size_t work = (size_t)rows * segs;
+  const int grid = (int)std::min<size_t>(work, 148 * 8 * 4);
+  const uint4* s = (const uint4*)samples;
+  if (c.kind == RB_CORPUS_PCM16)
+    items_gather_packed_kernel<true><<<grid, kGatherThreads, 0, st>>>(s, c.chunks, c.start, src_row, row_len, ld, rows, segs, x);
+  else
+    items_gather_packed_kernel<false><<<grid, kGatherThreads, 0, st>>>(s, c.chunks, c.start, src_row, row_len, ld, rows, segs, x);
+  RB_LAUNCH_CHECK();
+  return RB_OK;
+}
+
 int run_entry(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
-              const float* corpus, const int32_t* corpus_len, const int32_t* indices, const WalkSource& src, float* out,
-              int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
+              const CorpusSource& corpus, const int32_t* indices, const WalkSource& src, float* out, int32_t* out_len,
+              float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
   int rc = check_shape(args, G, nvoc, n_add, N, ld, trim);
   if (rc != RB_OK) return rc;
   const int V = 2 + n_add + 2 * nvoc;
   if ((layout != 0 && layout != 1) || (labels && V > 256)) return RB_ERR_INVALID_ARG;
   if (!src.shape_ok(G)) return RB_ERR_INVALID_ARG;
   if (G == 0) return RB_OK;
-  if (!corpus || !corpus_len || !indices || !src.pointers_ok() || !out) return RB_ERR_INVALID_ARG;
-  if ((uintptr_t)corpus & 15u) return RB_ERR_ALIGNMENT;
+  if (!indices || !src.pointers_ok() || !out) return RB_ERR_INVALID_ARG;
+  if ((rc = corpus.check(N, nvoc)) != RB_OK) return rc;
   const ItemsLayout l = items_layout(args, G, nvoc, n_add, N, ld);
   if ((rc = check_workspace(workspace, workspace_bytes, l.bytes)) != RB_OK) return rc;
+  const void* samples = nullptr;
+  if (corpus.is_packed && !(samples = corpus_device_ptr(corpus.packed->samples))) return RB_ERR_INVALID_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   char* d = (char*)workspace;
   int32_t *src_row = (int32_t*)(d + l.src_row), *row_len = (int32_t*)(d + l.row_len), *start = (int32_t*)(d + l.start);
   rb_plan plan;
-  if ((rc = items_draw(args, G, nvoc, n_add, N, ld, trim, corpus_len, indices, src, src_row, row_len, start, end_state, d, l,
+  if ((rc = items_draw(args, G, nvoc, n_add, N, ld, trim, corpus.len(), indices, src, src_row, row_len, start, end_state, d, l,
                        &plan, st)) != RB_OK)
     return rc;
   const int rows = G * (nvoc + 1 + n_add), nb = G * (nvoc + 1);
   float *x = (float*)(d + l.x), *y = (float*)(d + l.y);
-  items_gather_kernel<<<rows, 256, 0, st>>>(corpus, ld, src_row, row_len, x);
-  RB_LAUNCH_CHECK();
+  if (corpus.is_packed) {
+    if ((rc = gather_packed(*corpus.packed, samples, ld, src_row, row_len, rows, x, st)) != RB_OK) return rc;
+  } else {
+    items_gather_kernel<<<rows, 256, 0, st>>>(corpus.padded, ld, src_row, row_len, x);
+    RB_LAUNCH_CHECK();
+  }
   if ((rc = rb_process(5, x, row_len, nb, ld, &plan, y, d + l.proc, l.proc_bytes, stream)) != RB_OK) return rc;
   return rb_multiview_assemble_ex(x, y, (const int32_t*)(d + l.view_row), row_len, G, V, ld, start, trim, repeat_pad, layout, out,
                                   out_len, labels ? (const float*)(d + l.view_label) : nullptr, labels, stream);
@@ -328,8 +460,15 @@ int rb_items_draw(const rb_args* args, int G, int nvoc, int n_add, int N, int ld
 int rb_items_run(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
                  const float* corpus, const int32_t* corpus_len, const int32_t* indices, const uint32_t* seeds, float* out,
                  int32_t* out_len, float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
-  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, corpus, corpus_len, indices, {true, seeds, 0, nullptr, nullptr},
-                   out, out_len, labels, end_state, workspace, workspace_bytes, stream);
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, {false, corpus, corpus_len, nullptr}, indices,
+                   {true, seeds, 0, nullptr, nullptr}, out, out_len, labels, end_state, workspace, workspace_bytes, stream);
+}
+
+int rb_items_run_packed(const rb_args* args, int G, int nvoc, int n_add, int N, int ld, int trim, int repeat_pad, int layout,
+                        const rb_corpus* corpus, const int32_t* indices, const uint32_t* seeds, float* out, int32_t* out_len,
+                        float* labels, uint32_t* end_state, void* workspace, size_t workspace_bytes, void* stream) {
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, {true, nullptr, nullptr, corpus}, indices,
+                   {true, seeds, 0, nullptr, nullptr}, out, out_len, labels, end_state, workspace, workspace_bytes, stream);
 }
 
 int rb_items_stream_draw(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld, int trim,
@@ -344,7 +483,15 @@ int rb_items_stream_run(const rb_args* args, int S, const int32_t* stream_off, i
                         int repeat_pad, int layout, const float* corpus, const int32_t* corpus_len, const int32_t* indices,
                         const uint32_t* start_state, float* out, int32_t* out_len, float* labels, uint32_t* end_state, void* workspace,
                         size_t workspace_bytes, void* stream) {
-  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, corpus, corpus_len, indices,
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, {false, corpus, corpus_len, nullptr}, indices,
+                   {false, nullptr, S, stream_off, start_state}, out, out_len, labels, end_state, workspace, workspace_bytes, stream);
+}
+
+int rb_items_stream_run_packed(const rb_args* args, int S, const int32_t* stream_off, int G, int nvoc, int n_add, int N, int ld,
+                               int trim, int repeat_pad, int layout, const rb_corpus* corpus, const int32_t* indices,
+                               const uint32_t* start_state, float* out, int32_t* out_len, float* labels, uint32_t* end_state,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  return run_entry(args, G, nvoc, n_add, N, ld, trim, repeat_pad, layout, {true, nullptr, nullptr, corpus}, indices,
                    {false, nullptr, S, stream_off, start_state}, out, out_len, labels, end_state, workspace, workspace_bytes, stream);
 }
 

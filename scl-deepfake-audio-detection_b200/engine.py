@@ -310,6 +310,70 @@ class Engine:
         _lib.check(rc, "rb_items_stream_run")
         return out, out_len, labels
 
+    def _packed_items_setup(self, args, sr, corpus: _lib.RbCorpus, ld: int, nvoc: int, n_add: int, trim: int, G: int, layout: int,
+                            out: Optional[torch.Tensor], with_labels: bool):
+        """Shape, outputs and workspace of the ``_packed`` item entries: ``(N, out, out_len, labels, args struct, ws, need)``."""
+        if not isinstance(corpus, _lib.RbCorpus):
+            raise TypeError("corpus must be an RbCorpus descriptor (multiview.PackedCorpus.descriptor)")
+        R = int(corpus.rows)
+        if R <= 0 or R % (1 + nvoc):
+            raise ValueError("the corpus needs N*(1+nvoc) rows")
+        N, V = R // (1 + nvoc), 2 + n_add + 2 * nvoc
+        shape = (G, trim, V) if layout == 0 else (G, V, trim)
+        if out is None:
+            out = torch.zeros(shape, dtype=torch.float32, device=self.device)
+        elif tuple(out.shape) != shape or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 tensor {shape} on the engine's device")
+        out_len = torch.empty(G, dtype=torch.int32, device=self.device)
+        labels = torch.empty((G, V), dtype=torch.float32, device=self.device) if with_labels else None
+        a = _lib.args_struct(args, sr)
+        need = int(self.lib.rb_items_workspace_bytes(C.byref(a), G, int(nvoc), int(n_add), N, int(ld)))
+        if G and need == 0:
+            raise ValueError(f"unsupported item shape: G={G}, nvoc={nvoc}, n_add={n_add}, N={N}, ld={ld}")
+        return N, out, out_len, labels, a, self._scratch(need), need
+
+    def items_run_packed(self, args, sr, corpus: _lib.RbCorpus, ld: int, nvoc: int, n_add: int, trim: int, indices, seeds,
+                         repeat_pad: bool = True, layout: int = 0, out: Optional[torch.Tensor] = None, with_labels: bool = True,
+                         end_state: Optional[torch.Tensor] = None):
+        """:meth:`items_run` from a packed corpus (``rb_items_run_packed``): ``corpus`` is the ``rb_corpus`` descriptor of
+        ``multiview.PackedCorpus`` (samples in device or page-locked host memory, row starts and lengths on the device), ``ld``
+        the row stride of the gathered batch (a multiple of 4, at least the longest row). Same results as :meth:`items_run` on a
+        padded corpus of the same values, bit for bit."""
+        indices, seeds = self._item_arrays(indices, seeds)
+        G = int(indices.numel())
+        if end_state is not None and (end_state.shape != (G, 625) or end_state.element_size() != 4 or end_state.device != self.device):
+            raise ValueError("end_state must be a 32-bit [G, 625] tensor on the engine's device")
+        N, out, out_len, labels, a, ws, need = self._packed_items_setup(args, sr, corpus, ld, nvoc, n_add, trim, G, layout, out,
+                                                                        with_labels)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_run_packed(C.byref(a), G, int(nvoc), int(n_add), N, int(ld), int(trim), int(bool(repeat_pad)),
+                                              int(layout), C.byref(corpus), _ptr(indices), _ptr(seeds), _ptr(out), _ptr(out_len),
+                                              _ptr(labels), _ptr(end_state), C.c_void_p(self._ws_ptr(ws)), need, C.c_void_p(stream))
+        _lib.check(rc, "rb_items_run_packed")
+        return out, out_len, labels
+
+    def items_stream_run_packed(self, args, sr, corpus: _lib.RbCorpus, ld: int, nvoc: int, n_add: int, trim: int, indices,
+                                stream_off, start_state, repeat_pad: bool = True, layout: int = 0,
+                                out: Optional[torch.Tensor] = None, with_labels: bool = True, end_state=None):
+        """:meth:`items_stream_run` from a packed corpus (``rb_items_stream_run_packed``); ``corpus`` and ``ld`` as
+        :meth:`items_run_packed`."""
+        indices, stream_off, start_state, S = self._stream_arrays(indices, stream_off, start_state)
+        if end_state is not None and not torch.is_tensor(end_state):
+            raise ValueError("end_state must be None or an int32 [S, 625] device tensor")
+        end = self._stream_end(S, end_state)
+        G = int(indices.numel())
+        N, out, out_len, labels, a, ws, need = self._packed_items_setup(args, sr, corpus, ld, nvoc, n_add, trim, G, layout, out,
+                                                                        with_labels)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = self.lib.rb_items_stream_run_packed(C.byref(a), S, _ptr(stream_off), G, int(nvoc), int(n_add), N, int(ld), int(trim),
+                                                     int(bool(repeat_pad)), int(layout), C.byref(corpus), _ptr(indices),
+                                                     _ptr(start_state), _ptr(out), _ptr(out_len), _ptr(labels), _ptr(end),
+                                                     C.c_void_p(self._ws_ptr(ws)), need, C.c_void_p(stream))
+        _lib.check(rc, "rb_items_stream_run_packed")
+        return out, out_len, labels
+
     def pack_waveforms(self, waves: Sequence[np.ndarray], ld: Optional[int] = None):
         """Host list of 1-D float arrays -> ([B, ld] float32 device tensor, int32 lengths on device)."""
         lengths = np.array([int(w.shape[0]) for w in waves], dtype=np.int32)
