@@ -15,6 +15,12 @@ Same names, argument order and RNG behaviour as ``/root/reference/datautils/RawB
 These per-utterance calls pay a host->device->host round trip each; the loaders' throughput path is the batched
 API in :mod:`engine` (draw plans in the workers, apply them on the collated batch in the main process).
 There is no CPU fallback: without the built library and a CUDA device these functions raise.
+
+In a DataLoader worker forked after the parent initialised CUDA, CUDA cannot be used. When the parent serves the workers
+(``dropin.serve_workers``, :mod:`broker`), such a process routes ``normWav``, ``filterFIR`` and every RawBoost application to
+it: the draws stay here, on this process's numpy stream in the reference's order, and only the waveform and the drawn plan
+travel; the result comes back as float32, with the same values and the same object rules as a call in the parent. Without a
+broker these functions raise ``RawBoostLibraryError`` in such a process.
 """
 from __future__ import annotations
 
@@ -23,7 +29,7 @@ import os
 import numpy as np
 import torch
 
-from . import plans as _plans
+from . import _lib, broker as _broker, plans as _plans
 from .engine import default_engine
 from .plans import genNotchCoeffs, randRange  # noqa: F401  (part of the reference surface)
 
@@ -55,12 +61,24 @@ def _draw_native(length, fs, algo, **knobs):
 
 def _native_planner():
     global _native
-    if _native is None:
+    if _native is None or _native[0] != os.getpid():
         from .native_planner import NativePlanner
+        if _native is not None:
+            _native[1]._h = None  # inherited through fork: this process makes its own (no CUDA call) and leaves the parent's be
         planner = NativePlanner(threads=1, pinned=False)
         planner.self_check()  # once per process: refuse loudly if this numpy's stream is not the one the replica implements
-        _native = planner
-    return _native
+        _native = (os.getpid(), planner)
+    return _native[1]
+
+
+def _engine():
+    """The process's engine; refused with a pointer to the broker in a process forked after CUDA was initialised."""
+    if torch.cuda._is_in_bad_fork():
+        raise _lib.RawBoostLibraryError(
+            "CUDA cannot be used in a process forked after its parent initialised CUDA (a DataLoader worker); call "
+            "dropin.serve_workers() in the parent before the loader starts its workers, so that this process sends its "
+            "RawBoost calls there, or run the loader with num_workers=0 or multiprocessing_context='spawn'")
+    return default_engine(_DEVICE)
 
 
 def _as_wave(x):
@@ -73,12 +91,17 @@ def _as_wave(x):
 def _run_single(algo, x, plan):
     """One utterance through the host-buffer entry (``rb_process_host``: ONE C call copies the waveform and the plan in, runs
     the kernels and copies the result out): returns a new float32 array of x's length. ``plan``: an ``UtterancePlan`` or an
-    already packed one-utterance ``BatchPlan``."""
-    eng = default_engine(_DEVICE)
+    already packed one-utterance ``BatchPlan``. Routed to the broker in a worker process (:mod:`broker`)."""
     n = x.shape[0]
     if n == 0:
         return np.zeros(0, dtype=np.float32)
     bp = plan if isinstance(plan, _plans.BatchPlan) else (_plans.pack([plan]) if plan is not None else None)
+    if _broker.routed():
+        if bp is None:
+            raise ValueError(f"algo {algo} needs a plan")
+        key = ("rb", int(algo), int(bp.n_f), float(bp.g_sd), bp.ld > _broker.MASK_SMEM_MAX_LD)
+        return _broker.request(key, np.ascontiguousarray(x, dtype=np.float32), bp)
+    eng = _engine()
     ld = bp.ld if bp is not None else _plans.padded_ld(n)
     xh = np.zeros((1, ld), dtype=np.float32)
     xh[0, :n] = x  # (float64 input is rounded to float32 here, see the module docstring)
@@ -91,9 +114,12 @@ def normWav(x, always):
     x = _as_wave(x)
     if x.shape[0] == 0:
         return x
-    eng = default_engine(_DEVICE)
-    xd, ld = eng.pack_waveforms([x])
-    y = eng.normwav(xd, ld, bool(always))[0, :x.shape[0]].cpu().numpy()
+    if _broker.routed():
+        y = _broker.request(("norm", bool(always)), np.ascontiguousarray(x, dtype=np.float32), None)
+    else:
+        eng = _engine()
+        xd, ld = eng.pack_waveforms([x])
+        y = eng.normwav(xd, ld, bool(always))[0, :x.shape[0]].cpu().numpy()
     if not always and x.dtype == np.float32 and np.array_equal(y, x):
         return x
     return y
@@ -105,7 +131,9 @@ def filterFIR(x, b):
     b = np.asarray(b, dtype=np.float64).reshape(-1)
     if x.shape[0] == 0:
         return np.zeros(0, dtype=np.float32)
-    eng = default_engine(_DEVICE)
+    if _broker.routed():
+        return _broker.request(("fir",), np.ascontiguousarray(x, dtype=np.float32), b.astype(np.float32))
+    eng = _engine()
     xd, ld = eng.pack_waveforms([x])
     taps = torch.from_numpy(b.astype(np.float32)).to(eng.device)
     off = torch.tensor([0, b.shape[0]], dtype=torch.int32, device=eng.device)

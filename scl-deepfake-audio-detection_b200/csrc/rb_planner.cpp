@@ -414,7 +414,9 @@ struct PinnedBuf {
     if (want_pinned && cudaMallocHost((void**)&p, bytes) == cudaSuccess) {
       pinned = true;
     } else {
-      (void)cudaGetLastError();
+      // a planner created with pinned = 0 makes no CUDA runtime call at all: it may run in a process forked after the parent
+      // initialised CUDA (a DataLoader worker), where the runtime must not be touched
+      if (want_pinned) (void)cudaGetLastError();
       p = (T*)malloc(bytes);
       pinned = false;
       if (!p) return -1;

@@ -10,9 +10,11 @@ Two ways in, both leave the loader sources untouched:
 * :func:`patch_loader` after import: rebinds the operator names (and the dispatcher, which then issues one fused
   device call per utterance instead of one per operator) inside an already imported loader module.
 
-CUDA cannot be used in forked DataLoader workers once the parent initialised it (main.py:335 precedes main.py:379):
-run the patched loaders with ``num_workers=0`` or ``multiprocessing_context='spawn'``, or use the batched path
-(``plans.draw_batch`` in the workers, ``engine.Engine.process`` on the collated batch).
+CUDA cannot be used in forked DataLoader workers once the parent initialised it (main.py:335 precedes main.py:379).
+:func:`serve_workers`, called once in the parent before the loader starts its workers, lets the unmodified loaders run there:
+each worker draws on its own numpy stream as before and the parent applies the calls of all workers on the GPU, in batches.
+The alternatives remain: ``num_workers=0``, ``multiprocessing_context='spawn'``, or the batched path (``plans.draw_batch`` in
+the workers, ``engine.Engine.process`` on the collated batch).
 """
 from __future__ import annotations
 
@@ -45,3 +47,17 @@ def patch_loader(loader: types.ModuleType, dispatcher: bool = True) -> types.Mod
             if hasattr(loader, name):
                 setattr(loader, name, getattr(impl, name))
     return loader
+
+
+def serve_workers(device=None, max_batch: int = 64, max_len: int = 211000):
+    """Serve the RawBoost calls of this process's DataLoader workers on the GPU; returns the :class:`broker.Broker`.
+
+    Call it in the process that owns the GPU, after :func:`install` / :func:`patch_loader` and before the DataLoader starts its
+    workers (forked, spawned or forkserver). Every worker then sends its ``normWav``, ``filterFIR`` and RawBoost applications
+    here; the draws stay in the worker, so every numpy stream advances exactly as with the reference. One daemon thread applies
+    whatever requests are pending, up to ``max_batch`` utterances per batch, with its own engine and context; the process's own
+    drop-in calls are unaffected. ``max_len``: the longest utterance the workers send, for which the device buffers are sized
+    once, here (a longer one still works, at the cost of one device-wide synchronise when the buffers grow).
+    The handle has ``close()``, ``stats()`` (requests, batches, utterances, errors) and works as a context manager."""
+    from .broker import serve
+    return serve(device, max_batch, max_len)

@@ -233,13 +233,12 @@ class ItemBatcher:
             extra_waves += [np.asarray(self.load_audio(os.path.join(self.bonafide_dir, self.list_ids[i])), dtype=np.float32) for i in picked]
             starts.append(crop_plan(anchor.shape[0], self.trim_length, True, self.repeat_pad)[0])
         G, per = len(indices), nvoc + 1
-        if plans and isinstance(plans[0], _plans.BatchPlan):
-            bp = _concat_batch_plans(plans)
-        else:
-            bp = _plans.pack(plans)
         # rows: the RawBoost inputs of all items first, then every item's additional bona fide utterances (not augmented)
         ld = _plans.padded_ld(max([w.shape[0] for w in waves + extra_waves] + [1]))
-        bp = _repad(bp, ld)
+        if plans and isinstance(plans[0], _plans.BatchPlan):
+            bp = _plans.concat(plans, ld)
+        else:
+            bp = _plans.pack(plans, ld=ld)
         x, ln = eng.pack_waveforms(waves + extra_waves, ld=ld)
         y = torch.zeros_like(x)
         nb = G * per
@@ -550,23 +549,3 @@ class StreamItemBatcher:
         end = torch.empty((S, 625), dtype=torch.int32, device=dev)
         return (*self._run(idx, stream_off, states, layout, end), end)
 
-
-def _repad(bp, ld):
-    """A plan whose rows are addressed with stride ``ld`` (only SSI noise depends on the stride; algo 5 has none)."""
-    bp.ld = int(ld)
-    return bp
-
-
-def _concat_batch_plans(parts):
-    """Concatenate one-utterance BatchPlans (native planner, global stream) into one batch plan (LnL + ISD fields)."""
-    from .plans import BatchPlan
-    B = len(parts)
-    out = BatchPlan(B=B, ld=max(p.ld for p in parts), lengths=np.concatenate([p.lengths for p in parts]).astype(np.int32),
-                    g_sd=parts[0].g_sd, n_f=parts[0].n_f)
-    out.lnl_taps = np.concatenate([p.lnl_taps for p in parts])
-    sizes = np.concatenate([np.diff(p.lnl_tap_off) for p in parts])
-    out.lnl_tap_off = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int32)
-    out.isd_idx = np.concatenate([p.isd_idx for p in parts])
-    out.isd_fr = np.concatenate([p.isd_fr for p in parts])
-    out.isd_off = np.concatenate([[0], np.cumsum([p.isd_idx.shape[0] for p in parts])]).astype(np.int32)
-    return out

@@ -202,6 +202,47 @@ def pack(plans: Sequence[UtterancePlan], ld: Optional[int] = None) -> BatchPlan:
     return bp
 
 
+def _offsets(sizes) -> np.ndarray:
+    return np.concatenate([[0], np.cumsum(np.asarray(sizes, dtype=np.int64))]).astype(np.int32)
+
+
+def concat(parts: Sequence[BatchPlan], ld: Optional[int] = None) -> BatchPlan:
+    """Concatenate packed plans (all drawn for the same algo, ``N_f`` and ``g_sd``) into one :class:`BatchPlan` of stride
+    ``ld`` (default: the largest stride of the parts). Every field is carried; the SSI noise rows are re-laid to ``ld``."""
+    if not parts:
+        raise ValueError("nothing to concatenate")
+    first = parts[0]
+    ld = int(ld if ld is not None else max(p.ld for p in parts))
+    if any(p.n_f != first.n_f or p.g_sd != first.g_sd for p in parts):
+        raise ValueError("all plans of a batch must share N_f and g_sd")
+    lengths = np.concatenate([np.asarray(p.lengths, dtype=np.int32) for p in parts])
+    if lengths.size and int(lengths.max()) > ld:
+        raise ValueError(f"an utterance of {int(lengths.max())} samples does not fit the stride ld={ld}")
+    out = BatchPlan(B=int(lengths.shape[0]), ld=ld, lengths=lengths, n_f=first.n_f, g_sd=first.g_sd)
+    for name in ("lnl_tap_off", "isd_off", "ssi_tap_off"):
+        if any((getattr(p, name) is None) != (getattr(first, name) is None) for p in parts):
+            raise ValueError(f"{name} is set in some plans of the batch and missing in others")
+    if first.lnl_tap_off is not None:
+        out.lnl_taps = np.concatenate([p.lnl_taps for p in parts]).astype(np.float32, copy=False)
+        out.lnl_tap_off = _offsets(np.concatenate([np.diff(p.lnl_tap_off) for p in parts]))
+    if first.isd_off is not None:
+        out.isd_idx = np.concatenate([p.isd_idx for p in parts]).astype(np.int32, copy=False)
+        out.isd_fr = np.concatenate([p.isd_fr for p in parts]).astype(np.float64, copy=False)
+        out.isd_off = _offsets(np.concatenate([np.diff(p.isd_off) for p in parts]))
+    if first.ssi_tap_off is not None:
+        out.ssi_noise = np.zeros((out.B, ld), dtype=np.float32)
+        row = 0
+        for p in parts:
+            for u in range(p.B):
+                n = int(p.lengths[u])
+                out.ssi_noise[row, :n] = p.ssi_noise[u, :n]
+                row += 1
+        out.ssi_taps = np.concatenate([p.ssi_taps for p in parts]).astype(np.float32, copy=False)
+        out.ssi_tap_off = _offsets(np.concatenate([np.diff(p.ssi_tap_off) for p in parts]))
+        out.ssi_snr_db = np.concatenate([p.ssi_snr_db for p in parts]).astype(np.float32, copy=False)
+    return out
+
+
 def draw_batch(lengths: Sequence[int], sr, args, algo: int, seeds: Optional[Sequence[int]] = None,
                ld: Optional[int] = None) -> BatchPlan:
     """Draw and pack the plans of a batch. With ``seeds`` the global stream is re-seeded before each utterance
