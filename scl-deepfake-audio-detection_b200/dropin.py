@@ -13,6 +13,8 @@ Two ways in, both leave the loader sources untouched:
 CUDA cannot be used in forked DataLoader workers once the parent initialised it (main.py:335 precedes main.py:379).
 :func:`serve_workers`, called once in the parent before the loader starts its workers, lets the unmodified loaders run there:
 each worker draws on its own numpy stream as before and the parent applies the calls of all workers on the GPU, in batches.
+:func:`serve_items` goes further: it replaces the DataLoader the reference builds over ``Dataset_for`` with
+:class:`loader.DeviceLoader`, which builds the same epochs on the GPU with no worker processes at all.
 The alternatives remain: ``num_workers=0``, ``multiprocessing_context='spawn'``, or the batched path (``plans.draw_batch`` in
 the workers, ``engine.Engine.process`` on the collated batch).
 """
@@ -61,3 +63,17 @@ def serve_workers(device=None, max_batch: int = 64, max_len: int = 211000):
     The handle has ``close()``, ``stats()`` (requests, batches, utterances, errors) and works as a context manager."""
     from .broker import serve
     return serve(device, max_batch, max_len)
+
+
+def serve_items(loader_module, load_audio, dtype: str = "pcm16", location: str = "device"):
+    """Let an unmodified ``main.py`` train on items built on the GPU, with no worker processes; returns the
+    :class:`loader.ItemService` handle (``close()``, context manager).
+
+    Call it after :func:`install` and before ``main.py`` runs, with the imported loader module (``datautils.asvspoof_2019_augall_3``)
+    and the audio reader. ``Dataset_for.__init__`` then records its arguments, and ``torch.utils.data.DataLoader`` returns a
+    :class:`loader.DeviceLoader` over a ``multiview.PackedCorpus`` (``dtype``, ``location``) for a ``Dataset_for`` with
+    ``augmentation_methods == ['RawBoost12']`` and ``args.online_aug`` set, and no ``sampler``, ``batch_sampler``,
+    ``worker_init_fn`` or ``collate_fn``: the same batches in the same order, every draw from the numpy stream the worker that
+    built it would have used. Any other call gets the real ``DataLoader`` and one logged line saying why."""
+    from .loader import serve_items as serve
+    return serve(loader_module, load_audio, dtype, location)

@@ -210,16 +210,24 @@ class Engine:
         _lib.check(rc, "rb_items_run")
         return out, out_len, labels
 
+    def _upload(self, host: np.ndarray) -> torch.Tensor:
+        """A host array on the device, copied on torch's current stream through page-locked staging: unlike a copy from
+        pageable memory, it does not make the host wait for the work already queued on that stream."""
+        host = torch.from_numpy(np.ascontiguousarray(host))
+        if host.numel() == 0:
+            return torch.empty(host.shape, dtype=host.dtype, device=self.device)
+        return host.pin_memory().to(self.device, non_blocking=True)
+
     def _stream_arrays(self, indices, stream_off, start_state):
         """indices, stream_off and start_state as 32-bit device tensors (start_state [S, 625] holds the uint32 bit patterns of
         numpy's key[624], pos)."""
         if not torch.is_tensor(indices):
-            indices = torch.from_numpy(np.ascontiguousarray(indices, dtype=np.int32)).to(self.device)
+            indices = self._upload(np.asarray(indices, dtype=np.int32))
         if not torch.is_tensor(stream_off):
-            stream_off = torch.from_numpy(np.ascontiguousarray(stream_off, dtype=np.int32)).to(self.device)
+            stream_off = self._upload(np.asarray(stream_off, dtype=np.int32))
         if not torch.is_tensor(start_state):
             host = np.asarray(start_state, dtype=np.int64).reshape(-1, 625).astype(np.uint32)
-            start_state = torch.from_numpy(np.ascontiguousarray(host).view(np.int32)).to(self.device)
+            start_state = self._upload(host.view(np.int32))
         for name, t, dim, dtypes in (("indices", indices, 1, (torch.int32,)), ("stream_off", stream_off, 1, (torch.int32,)),
                                      ("start_state", start_state, 2, (torch.int32, torch.uint32))):
             if t.device != self.device or t.dtype not in dtypes or t.dim() != dim or not t.is_contiguous():

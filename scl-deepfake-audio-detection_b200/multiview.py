@@ -477,10 +477,14 @@ class StreamItemBatcher:
     of one stream is serial, so its time grows with the number of items in it; several independent streams (one per loader
     worker, say) walk in parallel.
 
-    The item draws never use numpy's Gaussian cache, so ``has_gauss`` / ``cached_gaussian`` of the global state carry over."""
+    The item draws never use numpy's Gaussian cache, so ``has_gauss`` / ``cached_gaussian`` of the global state carry over.
+    ``engine`` runs the calls (default: the corpus's); one with its own workspace lets the items be built on a stream of their
+    own while other work uses the corpus's engine."""
 
-    def __init__(self, args, corpus: "DeviceCorpus | PackedCorpus", num_additional_real=2, trim_length=64000, repeat_pad=True, wav_samp_rate=16000):
+    def __init__(self, args, corpus: "DeviceCorpus | PackedCorpus", num_additional_real=2, trim_length=64000, repeat_pad=True, wav_samp_rate=16000,
+                 engine: Optional[Engine] = None):
         self.args, self.corpus = args, corpus
+        self.eng = engine or corpus.eng
         self.num_additional_real, self.trim_length = int(num_additional_real), int(trim_length)
         self.repeat_pad, self.sr = bool(repeat_pad), int(wav_samp_rate)
         if not 0 <= self.num_additional_real <= corpus.N - 1:
@@ -495,13 +499,13 @@ class StreamItemBatcher:
     def _run(self, idx, stream_off, states, layout, end):
         c = self.corpus
         if isinstance(c, PackedCorpus):
-            data, out_len, labels = c.eng.items_stream_run_packed(self.args, self.sr, c.descriptor, c.ld, c.nvoc,
+            data, out_len, labels = self.eng.items_stream_run_packed(self.args, self.sr, c.descriptor, c.ld, c.nvoc,
                                                                   self.num_additional_real, self.trim_length, idx.astype(np.int32),
                                                                   stream_off, states, self.repeat_pad, layout, end_state=end)
         else:
-            data, out_len, labels = c.eng.items_stream_run(self.args, self.sr, c.data, c.lengths, c.nvoc, self.num_additional_real,
-                                                           self.trim_length, idx.astype(np.int32), stream_off, states,
-                                                           self.repeat_pad, layout, end_state=end)
+            data, out_len, labels = self.eng.items_stream_run(self.args, self.sr, c.data, c.lengths, c.nvoc, self.num_additional_real,
+                                                             self.trim_length, idx.astype(np.int32), stream_off, states,
+                                                             self.repeat_pad, layout, end_state=end)
         return [c.list_ids[i] for i in idx], data, labels, out_len
 
     def items(self, indices: Sequence[int], layout: int = LAYOUT_ITEM):
@@ -513,7 +517,7 @@ class StreamItemBatcher:
         words = _state_words(state)[None]
         if idx.size == 0:  # nothing is drawn
             return self._run(idx, [0, 0], words, layout, None)
-        end = torch.empty((1, 625), dtype=torch.int32, device=self.corpus.eng.device)
+        end = torch.empty((1, 625), dtype=torch.int32, device=self.eng.device)
         out = self._run(idx, [0, idx.size], words, layout, end)
         e = numpy_state(end[0])
         np.random.set_state(e[:3] + tuple(state[3:5]))
@@ -542,7 +546,7 @@ class StreamItemBatcher:
             states = np.stack([_state_words(s) for s in states]) if S else np.zeros((0, 625), np.uint32)
         idx = np.concatenate(lists) if S else np.zeros(0, np.int64)
         stream_off = np.concatenate([[0], np.cumsum([ix.size for ix in lists])]).astype(np.int32)
-        dev = self.corpus.eng.device
+        dev = self.eng.device
         if idx.size == 0:  # nothing is drawn: every stream ends where it starts
             end = states.clone() if torch.is_tensor(states) else torch.from_numpy(states.view(np.int32)).to(dev)
             return (*self._run(idx, stream_off, states, layout, None), end)
