@@ -1,4 +1,4 @@
-"""The reference's DataLoader epochs built on the device, batch for batch, with no worker processes.
+"""The reference's DataLoader epochs built on the device, batch for batch, with no worker processes building items.
 
 The reference trains with ``DataLoader(train_set, batch_size=1, shuffle=True, num_workers=8)`` after
 ``torch.manual_seed(args.seed)`` (main.py:308, 379): torch decides which indices each worker gets and seeds each worker's
@@ -6,9 +6,12 @@ numpy stream, and every ``Dataset_for.__getitem__`` draws on the stream of the w
 
 * :func:`epoch_schedule` -- what the installed torch's ``DataLoader`` does for one epoch, on the host: the batches in yield
   order, the worker of each batch, each worker's index list and numpy start state. It consumes torch's RNG exactly as the
-  loader does, through torch's own sampler classes and its worker seeding (``_generate_state``, a private helper of
-  ``torch.utils.data._utils.worker``, on purpose: tests/test_device_loader_host.py pins it against a real loader, so a torch
-  release that changes the seeding fails the suite instead of silently changing the data).
+  loader does, through torch's own sampler classes (or the caller's ``sampler`` / ``batch_sampler``) and its worker seeding
+  (``_generate_state``, ``WorkerInfo`` and the ``_worker_info`` global, private parts of ``torch.utils.data._utils.worker``,
+  on purpose: tests/test_device_loader_host.py and tests/test_device_loader_samplers_host.py pin them against a real loader,
+  so a torch release that changes the seeding fails the suite instead of silently changing the data). A ``worker_init_fn``
+  runs in one short-lived child process per worker, after torch's worker seeding, and what it leaves in numpy's state is
+  that worker's start state.
 * :class:`DeviceLoader` -- the iterable ``main.py``'s loop consumes: each epoch's items built on the GPU by
   :meth:`multiview.StreamItemBatcher.items_streams`, one stream per worker, every draw from the stream that worker would have
   used; batches are ``[ids, data, label]`` as ``default_collate`` gives them, with ``data`` and ``label`` on the device.
@@ -19,14 +22,20 @@ from __future__ import annotations
 import functools
 import inspect
 import logging
+import multiprocessing
+import operator
+import random
+import traceback
 import weakref
 from dataclasses import dataclass
 from typing import List, Optional
 
 import numpy as np
 import torch
+import torch.multiprocessing
 from torch.utils.data import BatchSampler, RandomSampler, SequentialSampler
-from torch.utils.data._utils.worker import _generate_state
+from torch.utils.data._utils import worker as _worker
+from torch.utils.data._utils.worker import WorkerInfo, _generate_state
 
 from . import multiview as _mv
 from .engine import Engine
@@ -44,8 +53,125 @@ def batch_sampler(n: int, batch_size: int = 1, shuffle: bool = False, drop_last:
     """The loader's index sampler: torch's ``BatchSampler`` over ``RandomSampler`` / ``SequentialSampler`` as ``DataLoader``
     builds it. A ``RandomSampler`` without a generator draws its own seed from torch's global generator each time a pass over
     it starts (at the first index)."""
-    sampler = RandomSampler(range(n), generator=generator) if shuffle else SequentialSampler(range(n))
+    return index_sampler(n, batch_size, shuffle, drop_last, generator)
+
+
+def index_sampler(n: int, batch_size: int = 1, shuffle: bool = False, drop_last: bool = False,
+                  generator: Optional[torch.Generator] = None, sampler=None, batch_sampler=None):
+    """What ``DataLoader.__init__`` iterates for index batches, with its refusals: a given ``batch_sampler`` as it is (any
+    iterable of index lists, a plain list included); else ``BatchSampler(sampler, batch_size, drop_last)`` over the given
+    ``sampler``, or over ``RandomSampler`` / ``SequentialSampler`` of ``range(n)`` (see :func:`batch_sampler`)."""
+    if sampler is not None and shuffle:
+        raise ValueError("sampler option is mutually exclusive with shuffle")
+    if batch_sampler is not None:
+        if batch_size != 1 or shuffle or sampler is not None or drop_last:
+            raise ValueError("batch_sampler option is mutually exclusive with batch_size, shuffle, sampler, and drop_last")
+        return batch_sampler
+    if sampler is None:
+        sampler = RandomSampler(range(n), generator=generator) if shuffle else SequentialSampler(range(n))
     return BatchSampler(sampler, batch_size, drop_last)
+
+
+def checked_batches(batches, n: int) -> List[List[int]]:
+    """One pass of a batch sampler as lists of int, every index checked before any item is built: a non-integer index
+    (``bool`` included) raises TypeError, one outside ``[0, n)`` IndexError -- a negative one too, although a dataset that
+    indexes a Python list would take it -- and an empty batch ValueError. Repeated indices are kept."""
+    out = []
+    for j, b in enumerate(batches):
+        row = []
+        for i in b:
+            if isinstance(i, (bool, np.bool_)):
+                raise TypeError(f"batch {j}: index {i!r} is not an integer")
+            try:
+                k = operator.index(i)
+            except TypeError:
+                raise TypeError(f"batch {j}: index {i!r} is not an integer") from None
+            if not 0 <= k < n:
+                raise IndexError(f"batch {j}: index {k} lies outside [0, {n})")
+            row.append(k)
+        if not row:
+            raise ValueError(f"batch {j} is empty")
+        out.append(row)
+    return out
+
+
+def worker_context(num_workers: int, multiprocessing_context=None):
+    """The multiprocessing context ``DataLoader`` starts its workers from, with the refusals of its
+    ``multiprocessing_context`` setter: a start method's name or a context; None is ``torch.multiprocessing`` (the platform's
+    default start method)."""
+    if multiprocessing_context is None:
+        return torch.multiprocessing
+    if num_workers <= 0:
+        raise ValueError("multiprocessing_context can only be used with multi-process loading (num_workers > 0), but got "
+                         f"num_workers={num_workers}")
+    if isinstance(multiprocessing_context, str):
+        valid = torch.multiprocessing.get_all_start_methods()
+        if multiprocessing_context not in valid:
+            raise ValueError(f"multiprocessing_context option should specify a valid start method in {valid!r}, but got "
+                             f"multiprocessing_context={multiprocessing_context!r}")
+        multiprocessing_context = torch.multiprocessing.get_context(multiprocessing_context)
+    if not isinstance(multiprocessing_context, multiprocessing.context.BaseContext):
+        raise TypeError("multiprocessing_context option should be a valid context object or a string specifying the start "
+                        f"method, but got multiprocessing_context={multiprocessing_context}")
+    return multiprocessing_context
+
+
+def _run_worker_init(init_fn, base_seed: int, worker_id: int, num_workers: int, conn) -> None:
+    """Child process: the prologue of torch's ``_worker_loop`` up to and including ``init_fn(worker_id)``, then numpy's state
+    to the parent. No CUDA call: in a child forked from a process with a CUDA context, ``torch.manual_seed`` only queues its
+    CUDA part, as in torch's own workers."""
+    try:
+        torch.set_num_threads(1)
+        seed = base_seed + worker_id
+        random.seed(seed)
+        torch.manual_seed(seed)
+        np.random.seed(_generate_state(base_seed, worker_id))
+        # DeviceLoader holds no dataset object: get_worker_info().dataset is None
+        _worker._worker_info = WorkerInfo(id=worker_id, num_workers=num_workers, seed=seed, dataset=None)
+        init_fn(worker_id)
+        conn.send(("ok", np.random.get_state()))
+    except Exception:
+        conn.send(("error", traceback.format_exc()))
+    finally:
+        conn.close()
+
+
+def _init_states(base_seed: int, num_workers: int, init_fn, context) -> np.ndarray:
+    """uint32 [num_workers, 625]: each worker's numpy state after ``init_fn`` has run in a child process started from
+    ``context``, all children at once. An exception in a child raises RuntimeError here naming the worker, with the child's
+    traceback; every child is joined whatever happens."""
+    procs, conns = [], []
+    ok = False
+    try:
+        for w in range(num_workers):
+            recv, send = context.Pipe(duplex=False)
+            conns.append(recv)
+            try:
+                p = context.Process(target=_run_worker_init, args=(init_fn, base_seed, w, num_workers, send), daemon=True)
+                p.start()
+            finally:
+                send.close()  # the child holds its own end: a child that dies before it answers shows up as EOFError
+            procs.append(p)
+        states = np.zeros((num_workers, 625), dtype=np.uint32)
+        for w, (p, recv) in enumerate(zip(procs, conns)):
+            try:
+                kind, value = recv.recv()
+            except EOFError:
+                p.join()
+                raise RuntimeError(f"DataLoader worker process {w} exited with code {p.exitcode} before its worker_init_fn "
+                                   "returned") from None
+            if kind != "ok":
+                raise RuntimeError(f"worker_init_fn raised in DataLoader worker process {w}:\n{value}")
+            states[w] = _mv._state_words(value)
+        ok = True
+        return states
+    finally:
+        for p in procs:
+            if not ok and p.is_alive():
+                p.terminate()
+            p.join()
+        for c in conns:
+            c.close()
 
 
 def worker_start_states(base_seed: int, num_workers: int) -> np.ndarray:
@@ -97,20 +223,41 @@ def split_batches(batches: List[List[int]], num_workers: int):
 
 def epoch_schedule(n: int, batch_size: int = 1, shuffle: bool = False, num_workers: int = 0, drop_last: bool = False,
                    generator: Optional[torch.Generator] = None, persistent_workers: bool = False,
-                   first_iter: bool = True) -> EpochSchedule:
-    """What ``iter(DataLoader(dataset_of_length_n, batch_size, shuffle, num_workers=..., drop_last, generator,
-    persistent_workers))`` followed by a full pass does with the installed torch, for a map-style dataset with the default
-    sampler, collate function and no ``worker_init_fn``. torch's RNG is consumed as the loader consumes it: the base seed from
-    ``generator`` (or the global generator) -- only at the first ``iter()`` of persistent workers (``first_iter``) -- then, with
-    ``shuffle`` and no generator, the sampler's own seed from the global generator. The loader with workers makes both draws
-    inside ``iter()``; without workers the sampler's draw comes at the first ``next()`` (:class:`DeviceLoader` keeps that
-    timing; this function makes both draws at once)."""
+                   first_iter: bool = True, *, sampler=None, batch_sampler=None, worker_init_fn=None,
+                   multiprocessing_context=None) -> EpochSchedule:
+    """What ``iter(DataLoader(dataset_of_length_n, batch_size, shuffle, sampler, batch_sampler, num_workers, drop_last=...,
+    worker_init_fn=..., multiprocessing_context=..., generator=..., persistent_workers=...))`` followed by a full pass does
+    with the installed torch, for a map-style dataset with the default collate function. The index batches are those of
+    :func:`index_sampler`, every index checked by :func:`checked_batches`.
+
+    torch's RNG is consumed as the loader consumes it: the base seed from ``generator`` (or the global generator) -- only at
+    the first ``iter()`` of persistent workers (``first_iter``) -- then the batch sampler's pass starts, and torch's own
+    samplers make their draws there (a ``RandomSampler`` without a generator its own seed from the global generator;
+    ``WeightedRandomSampler``, ``SubsetRandomSampler`` and ``DistributedSampler`` likewise at their first index). The loader
+    with workers makes both inside ``iter()``; without workers the pass starts at the first ``next()`` (:class:`DeviceLoader`
+    keeps that timing; this function makes both at once).
+
+    Where torch seeds its workers (every epoch, or only the first one of persistent workers) and a ``worker_init_fn`` is
+    given, it runs for each worker in a child process started from ``multiprocessing_context`` (a start method's name or a
+    context; None is the platform's default), after torch's worker seeding, with ``get_worker_info()`` set (its ``dataset``
+    None), and the numpy state it leaves is the worker's start state. An exception there raises RuntimeError naming the
+    worker. Without workers it is not called, as torch does not call it then."""
     check_loader_args(n, batch_size, num_workers, persistent_workers)
+    index_batches = index_sampler(n, batch_size, shuffle, drop_last, generator, sampler, batch_sampler)
+    context = worker_context(num_workers, multiprocessing_context)
     seeded = num_workers == 0 or first_iter or not persistent_workers
+    return _schedule(index_batches, n, num_workers, generator, seeded, worker_init_fn, context)
+
+
+def _schedule(index_batches, n: int, num_workers: int, generator, seeded: bool, worker_init_fn, context) -> EpochSchedule:
+    it = iter(index_batches)  # _BaseDataLoaderIter takes the sampler's iterator first, then draws the base seed
     seed = draw_base_seed(generator) if seeded else None
-    batches = [list(b) for b in batch_sampler(n, batch_size, shuffle, drop_last, generator)]
+    batches = checked_batches(it, n)
     batch_worker, worker_indices = split_batches(batches, num_workers)
-    states = worker_start_states(seed, num_workers) if num_workers and seed is not None else None
+    states = None
+    if num_workers and seed is not None:
+        states = (_init_states(seed, num_workers, worker_init_fn, context) if worker_init_fn is not None else
+                  worker_start_states(seed, num_workers))
     return EpochSchedule(batches, batch_worker, worker_indices, states, seed)
 
 
@@ -128,7 +275,8 @@ class _Chunk:
 
 
 class DeviceLoader:
-    """``DataLoader(Dataset_for(...), batch_size, shuffle, num_workers=..., drop_last, generator, persistent_workers)`` for
+    """``DataLoader(Dataset_for(...), batch_size, shuffle, sampler, batch_sampler, num_workers, drop_last=...,
+    worker_init_fn=..., multiprocessing_context=..., generator=..., persistent_workers=...)`` for
     ``augmentation_methods == ['RawBoost12']`` with ``online_aug``, every item built on the GPU.
 
     ``corpus``: a :class:`multiview.DeviceCorpus` or :class:`multiview.PackedCorpus` of the dataset's ``list_IDs`` and
@@ -139,6 +287,14 @@ class DeviceLoader:
     real loader after the same ``torch.manual_seed``: each worker's items come from the numpy stream torch would have seeded
     for that worker; without workers they come from numpy's global stream, which afterwards stands where the real loader
     leaves it (read when the epoch's first batch is built, written back when its last batch is yielded: one synchronisation).
+
+    ``sampler`` / ``batch_sampler`` are taken as ``DataLoader`` takes them (:func:`index_sampler`), and every epoch iterates
+    the same object, so ``DistributedSampler.set_epoch(e)`` before an epoch works as with torch. Each epoch's indices are
+    checked on the host before anything is enqueued (:func:`checked_batches`): a negative index raises IndexError although a
+    dataset indexing a Python list would take it. ``worker_init_fn`` runs where torch's workers run it, in a short-lived child
+    process per worker started from ``multiprocessing_context``, and the numpy state it leaves is that worker's start state
+    (:func:`epoch_schedule`); the child makes no CUDA call. One data-parallel rank per GPU builds its shard on its own device:
+    the loader runs on ``corpus.eng.device``, whatever the current device is when it is iterated.
 
     Items are built ``chunk_batches`` loader batches at a time, one ``items_streams`` call per chunk with one stream per
     worker, on a side stream of the loader's own; a chunk's end states stay on the device and seed the next chunk's call (for
@@ -160,13 +316,21 @@ class DeviceLoader:
       stream is not involved.
     * An epoch left before its end leaves numpy's global stream where it was (no workers), and persistent workers' streams
       carry on from where production stopped (torch's workers would also have built the batches they had been sent).
-    * Items are always built in the main process, whatever ``num_workers`` says."""
+    * Items are always built in the main process, whatever ``num_workers`` says.
+    * The real loader pulls ``prefetch_factor * num_workers`` batches from the batch sampler ahead of the batches it yields;
+      this loader pulls the whole epoch at ``iter()`` (at the first ``next()`` without workers). The samplers of torch make
+      all their draws when their pass starts, so this changes nothing for them; a sampler that draws on torch's *global*
+      generator lazily, index by index, sees those draws at another point relative to the training loop's own draws on it.
+    * ``get_worker_info().dataset`` is None inside ``worker_init_fn``: the loader holds no dataset object."""
 
     def __init__(self, corpus, args, num_additional_real=2, trim_length=64000, repeat_pad=True, wav_samp_rate=16000,
                  batch_size=1, shuffle=False, num_workers=0, drop_last=False, generator=None, persistent_workers=False,
-                 layout=_mv.LAYOUT_ITEM, chunk_batches=256):
+                 layout=_mv.LAYOUT_ITEM, chunk_batches=256, *, sampler=None, batch_sampler=None, worker_init_fn=None,
+                 multiprocessing_context=None):
         n = int(corpus.N)
         check_loader_args(n, batch_size, num_workers, persistent_workers)
+        index_batches = index_sampler(n, batch_size, shuffle, drop_last, generator, sampler, batch_sampler)
+        self._context = worker_context(num_workers, multiprocessing_context)
         if int(chunk_batches) < 1:
             raise ValueError(f"chunk_batches must be at least 1, not {chunk_batches}")
         if layout not in (_mv.LAYOUT_ITEM, _mv.LAYOUT_MODEL):
@@ -175,7 +339,7 @@ class DeviceLoader:
         self.batch_size, self.shuffle, self.num_workers, self.drop_last = int(batch_size), bool(shuffle), int(num_workers), bool(drop_last)
         self.generator, self.persistent_workers = generator, bool(persistent_workers)
         self.layout, self.chunk_batches, self.repeat_pad = layout, int(chunk_batches), bool(repeat_pad)
-        self.batch_sampler = batch_sampler(n, self.batch_size, self.shuffle, self.drop_last, generator)
+        self.sampler, self.batch_sampler, self.worker_init_fn = sampler, index_batches, worker_init_fn
         self.device = corpus.eng.device
         # its own engine: its own workspace, so the side stream shares no scratch memory with other users of the corpus's engine
         self._eng = Engine(self.device)
@@ -191,19 +355,20 @@ class DeviceLoader:
 
     def __iter__(self):
         if self.num_workers == 0:
-            draw_base_seed(self.generator)  # the sampler's own draw waits for the first next()
-            return self._epoch(None)
-        s = epoch_schedule(self.n, self.batch_size, self.shuffle, self.num_workers, self.drop_last, self.generator,
-                           self.persistent_workers, first_iter=not self._iterated)
+            it = iter(self.batch_sampler)
+            draw_base_seed(self.generator)  # the sampler's own draws wait for the first next()
+            return self._epoch(None, it)
+        s = _schedule(self.batch_sampler, self.n, self.num_workers, self.generator,
+                      not (self.persistent_workers and self._iterated), self.worker_init_fn, self._context)
         self._iterated = True
         if s.worker_states is not None:
             self._states = [_mv.numpy_state(row) for row in s.worker_states]
         return self._epoch(s.batches)
 
-    def _epoch(self, batches):
+    def _epoch(self, batches, sampler_iter=None):
         gauss = None
         if batches is None:  # no workers: the first next() starts the sampler's pass, then the items draw on numpy's stream
-            batches = [list(b) for b in self.batch_sampler]
+            batches = checked_batches(sampler_iter, self.n)
             state = np.random.get_state()
             gauss = tuple(state[3:5])  # the items never use numpy's Gaussian cache: it carries over unchanged
             self._states = [state]
