@@ -388,6 +388,18 @@ RB_API uint64_t rb_launch_count(void);
  * launch count since the last reset. Off by default; costs two event records per launch when on. */
 RB_API int rb_profile_enable(int on);
 RB_API int rb_profile_read(double* fir_ms, uint64_t* fir_launches, int reset);
+/* rb_set_tap_trim: process-wide, on (1) by default. The LnL and SSI filters (genNotchCoeffs cascades, whose end taps are ~1e-20
+ * of the largest) then run over their effective support only: from each end, the longest run of taps whose |b| sum to at most
+ * 2^-31 sum|b| is skipped (float64 sums in tap order over the float32 taps; plans.tap_support in Python). That changes an output
+ * by at most 2^-30 sum_f ||b_f||_1 ||x^p||_inf before normWav -- 1/64 of what rounding the taps to float32 already allows -- and
+ * removes about a quarter of the bank's multiply-adds at the default arguments. Banks of more than 16 filters per utterance,
+ * and rb_filter_fir / rb_reverb (the caller's taps), always run every tap. rb_set_tap_trim(0): every tap, bit for bit the
+ * results of a build without trimming. Takes effect for calls issued after it returns. */
+RB_API int rb_set_tap_trim(int on);
+/* The supports themselves, for counting the work that runs: support[i] = (lo, hi) of the n filters of a CSR tap array (device
+ * taps float32[tap_off[n]], tap_off int32[n + 1], support int32[n][2]); the kernels run b[lo .. hi) of filter i. Asynchronous
+ * on `stream`, no workspace. */
+RB_API int rb_tap_support(const float* taps, const int32_t* tap_off, int n, int32_t* support, void* stream);
 
 #ifdef __cplusplus
 }

@@ -22,7 +22,8 @@ SYMBOLS = (
     "rb_ctx_set_chunk", "rb_submit_host_seeded", "rb_ctx_wait", "rb_ctx_trace", "rb_ctx_timeline", "rb_multiview_assemble",
     "rb_multiview_assemble_ex", "rb_submit_seeded_ex", "rb_reverb_workspace_bytes", "rb_reverb",
     "rb_items_workspace_bytes", "rb_items_draw", "rb_items_run", "rb_items_stream_draw", "rb_items_stream_run",
-    "rb_submit_seeded_packed", "rb_items_run_packed", "rb_items_stream_run_packed",
+    "rb_submit_seeded_packed", "rb_items_run_packed", "rb_items_stream_run_packed", "rb_set_tap_trim",
+    "rb_tap_support",
 )
 RB_IO_HOST_F32, RB_IO_HOST_PCM16, RB_IO_DEVICE_F32 = 0, 1, 2
 RB_CORPUS_F32, RB_CORPUS_PCM16 = 0, 1
@@ -132,6 +133,10 @@ def load() -> C.CDLL:
     lib.rb_profile_enable.argtypes = [i32]
     lib.rb_profile_read.restype = i32
     lib.rb_profile_read.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_uint64), i32]
+    lib.rb_set_tap_trim.restype = i32
+    lib.rb_set_tap_trim.argtypes = [i32]
+    lib.rb_tap_support.restype = i32
+    lib.rb_tap_support.argtypes = [vp, vp, i32, vp, vp]
     lib.rb_planner_create.restype = i32
     lib.rb_planner_create.argtypes = [C.POINTER(vp), i32, i32]
     lib.rb_planner_destroy.restype = i32

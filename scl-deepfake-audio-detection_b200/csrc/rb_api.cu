@@ -17,6 +17,10 @@ namespace rb {
 
 std::atomic<uint64_t> g_launches{0};
 
+namespace {
+std::atomic<int> g_tap_trim{1};  // rb_set_tap_trim
+}  // namespace
+
 // ---- FIR-bank launch timing (see rb_common.cuh) -------------------------------------------------------
 namespace {
 std::atomic<int> g_profile_on{0};
@@ -54,10 +58,14 @@ namespace {
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 inline int mask_ld_for(int ld) { return (int)align_up((size_t)ld / 32 + 2, 4); }
 
+// LnL filters per utterance whose supports the workspace holds; a bank of more filters runs over every tap.
+constexpr int kSupportFilters = 16;
+
 // Device workspace layout for one batch.
 struct Workspace {
   float* stats_a;
   uint32_t* counters;  // per-utterance tile arrival counters of the fused FIR tail
+  int2* support;       // [B][kSupportFilters] kept taps [lo, hi) of the LnL / SSI filters (launch_tap_support)
   uint32_t* mask;
   int mask_ld;
   float* buf1;  // intermediate waveform of the chained algos 4, 6, 7, 8
@@ -81,6 +89,7 @@ Workspace carve(void* base, int B, int ld, int nbuf) {
   };
   w.stats_a = (float*)take((size_t)B * ntiles * kStatN * sizeof(float));
   w.counters = (uint32_t*)take((size_t)B * sizeof(uint32_t));
+  w.support = (int2*)take((size_t)B * kSupportFilters * sizeof(int2));
   w.mask_ld = mask_ld_for(ld);
   w.mask = (uint32_t*)take((size_t)B * w.mask_ld * sizeof(uint32_t));
   w.buf1 = nbuf >= 1 ? (float*)take((size_t)B * ld * sizeof(float)) : nullptr;
@@ -113,11 +122,21 @@ int check_ws(void* ws, size_t ws_bytes, int B, int ld, int algo, Workspace* out)
 
 // LnL (optionally followed by ISD): x -> out. One FIR-bank launch; its fused tail does mean removal, normWav, the impulse
 // scatter and the second normWav per utterance.
+// Where the FIR bank finds the supports of a plan's n_f filters per utterance: the workspace's, or NULL (every tap) when tap
+// trimming is off or the bank has more filters than the workspace holds.
+int2* support_for(int n_f, const Workspace& w) {
+  return g_tap_trim.load(std::memory_order_relaxed) && n_f <= kSupportFilters ? w.support : nullptr;
+}
+
 int do_lnl(const float* x, const int32_t* len, int B, int ld, const rb_plan* pl, bool with_isd, float* out, const Workspace& w,
            cudaStream_t st) {
   if (!pl || pl->n_f < 1 || !pl->lnl_taps || !pl->lnl_tap_off) return RB_ERR_PLAN;
   if (with_isd && (!pl->isd_off || !pl->isd_idx || !pl->isd_fr)) return RB_ERR_PLAN;
-  if (with_isd) RB_TRY(launch_mask_build(pl->isd_off, pl->isd_idx, len, B, w.mask, w.mask_ld, st));
+  int2* support = support_for(pl->n_f, w);
+  // the supports are derived by the impulse mask's launch when there is one, by a launch of their own otherwise
+  if (with_isd) RB_TRY(launch_mask_build(pl->isd_off, pl->isd_idx, len, B, w.mask, w.mask_ld, pl->lnl_taps, pl->lnl_tap_off, pl->n_f,
+                                         support, st));
+  else if (support) RB_TRY(launch_tap_support(pl->lnl_taps, pl->lnl_tap_off, B * pl->n_f, support, st));
   FirTail tail;
   tail.mode = TAIL_AFFINE;
   tail.counters = w.counters;
@@ -129,7 +148,7 @@ int do_lnl(const float* x, const int32_t* len, int B, int ld, const rb_plan* pl,
     tail.g_sd = pl->g_sd;
   }
   // the raw sum goes into `out` itself and is finalised in place while still in L2: no intermediate buffer reaches HBM
-  return launch_fir_bank(x, len, B, ld, pl->lnl_taps, pl->lnl_tap_off, pl->n_f, 1, 1, out, w.stats_a,
+  return launch_fir_bank(x, len, B, ld, pl->lnl_taps, pl->lnl_tap_off, support, pl->n_f, 1, 1, out, w.stats_a,
                          with_isd ? w.mask : nullptr, w.mask_ld, tail, st);
 }
 
@@ -152,8 +171,11 @@ int do_ssi(const float* x, const int32_t* len, int B, int ld, const rb_plan* pl,
   tail.out = out;
   tail.aux = x;
   tail.snr_db = pl->ssi_snr_db;
+  int2* support = support_for(1, w);
+  if (support) RB_TRY(launch_tap_support(pl->ssi_taps, pl->ssi_tap_off, B, support, st));
   // the coloured noise goes into `out` and is mixed in place while still in L2
-  return launch_fir_bank(pl->ssi_noise, len, B, ld, pl->ssi_taps, pl->ssi_tap_off, 1, 1, 0, out, w.stats_a, nullptr, 0, tail, st);
+  return launch_fir_bank(pl->ssi_noise, len, B, ld, pl->ssi_taps, pl->ssi_tap_off, support, 1, 1, 0, out, w.stats_a, nullptr, 0,
+                         tail, st);
 }
 
 // normWav: x -> out (out may equal x), or with `add`: normWav(x + add) -> out
@@ -203,6 +225,19 @@ int rb_profile_enable(int on) {
   return RB_OK;
 }
 
+int rb_set_tap_trim(int on) {
+  g_tap_trim.store(on ? 1 : 0, std::memory_order_relaxed);
+  return RB_OK;
+}
+
+int rb_tap_support(const float* taps, const int32_t* tap_off, int n, int32_t* support, void* stream) {
+  if (n < 0) return RB_ERR_INVALID_ARG;
+  if (n == 0) return RB_OK;
+  if (!taps || !tap_off || !support) return RB_ERR_INVALID_ARG;
+  if ((uintptr_t)support & 7u) return RB_ERR_ALIGNMENT;
+  return launch_tap_support(taps, tap_off, n, (int2*)support, (cudaStream_t)stream);
+}
+
 int rb_profile_read(double* fir_ms, uint64_t* fir_launches, int reset) {
   std::lock_guard<std::mutex> lk(g_profile_mu);
   for (size_t i = 0; i + 1 < g_profile_events.size(); i += 2) {
@@ -228,7 +263,7 @@ int rb_filter_fir(const float* x, const int32_t* len, int B, int ld, const float
   RB_TRY(check_batch(x, len, B, ld, y));
   if (B == 0 || ld == 0) return RB_OK;
   if (!taps || !tap_off || x == y) return RB_ERR_INVALID_ARG;  // not in-place safe: a tile reads its neighbours' samples
-  return launch_fir_bank(x, len, B, ld, taps, tap_off, 1, 1, 0, y, nullptr, nullptr, 0, FirTail(), (cudaStream_t)stream);
+  return launch_fir_bank(x, len, B, ld, taps, tap_off, nullptr, 1, 1, 0, y, nullptr, nullptr, 0, FirTail(), (cudaStream_t)stream);
 }
 
 int rb_normwav(const float* x, const int32_t* len, int B, int ld, int always, float* y, void* workspace, size_t workspace_bytes,

@@ -115,8 +115,9 @@ struct FirTail {
 
 // ---- kernel launchers shared between translation units (all asynchronous on `st`) ------------------
 // FIR bank: y[u] = sum_f FIR(x[u] ** (pow_base + f*pow_step), taps of filter (u,f)); optional tile stats + ISD mask + tail.
+// support (nullable, [B * n_f], launch_tap_support): with a tail, filter (u,f) runs over its kept taps only.
 int launch_fir_bank(const float* x, const int32_t* len, int B, int ld, const float* taps, const int32_t* tap_off,
-                    int n_f, int pow_base, int pow_step, float* y, float* stats /*nullable*/,
+                    const int2* support /*nullable*/, int n_f, int pow_base, int pow_step, float* y, float* stats /*nullable*/,
                     const uint32_t* mask /*nullable*/, int mask_ld, const FirTail& tail, cudaStream_t st);
 
 // Device-side planner, stage by stage (rb_devplan.cu); rb_devplan_draw runs all four for the whole batch. The pipelined host

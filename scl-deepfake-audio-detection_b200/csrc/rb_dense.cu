@@ -25,14 +25,84 @@ namespace rb {
 
 namespace {
 
+// ---- effective support of a notch cascade (launch_tap_support) --------------------------------------------------------------
+// Filter b[0..K) keeps taps [lo, hi): lo is the largest count whose |b| sum to at most t = 2^-31 sum|b| (eps / 2, eps = 2^-30),
+// hi the same rule from the other end. The sums are float64 and taken strictly in tap order -- sum|b| and lo from the left, hi
+// from the right -- so the result equals plans.tap_support's cumulative sums bit for bit. Every lane of the warp runs the same
+// sequential sum; the taps reach it 32 at a time by shuffle. An all-zero filter keeps nothing (0, 0); a non-finite sum keeps
+// every tap.
+constexpr double kTrimHalfEps = 0x1p-31;
+
+__device__ __forceinline__ float abs_tap(const float* __restrict__ b, int K, int k) { return k < K ? fabsf(__ldg(b + k)) : 0.f; }
+
+__device__ void tap_support_warp(const float* __restrict__ taps, int t0, int K, int lane, int2* __restrict__ out) {
+  const float* b = taps + t0;
+  double total = 0.0;
+  for (int k0 = 0; k0 < K; k0 += 32) {
+    const float v = abs_tap(b, K, k0 + lane);
+    const int n = min(32, K - k0);
+    for (int j = 0; j < n; ++j) total += (double)__shfl_sync(0xffffffffu, v, j);
+  }
+  int lo = 0, hi = K;
+  if (isfinite(total)) {
+    const double t = total * kTrimHalfEps;
+    double c = 0.0;
+    bool more = true;
+    for (int k0 = 0; k0 < K && more; k0 += 32) {  // from the left (uniform: every lane holds the same sum)
+      const float v = abs_tap(b, K, k0 + lane);
+      const int n = min(32, K - k0);
+      for (int j = 0; j < n && more; ++j) {
+        c += (double)__shfl_sync(0xffffffffu, v, j);
+        if (c <= t) lo = k0 + j + 1;
+        else more = false;
+      }
+    }
+    c = 0.0;
+    more = true;
+    for (int k0 = 0; k0 < K && more; k0 += 32) {  // from the right: lane l holds b[K-1-(k0+l)]
+      const float v = k0 + lane < K ? fabsf(__ldg(b + K - 1 - (k0 + lane))) : 0.f;
+      const int n = min(32, K - k0);
+      for (int j = 0; j < n && more; ++j) {
+        c += (double)__shfl_sync(0xffffffffu, v, j);
+        if (c <= t) hi = K - (k0 + j + 1);
+        else more = false;
+      }
+    }
+    if (lo >= hi) lo = hi = 0;
+  }
+  if (lane == 0) *out = make_int2(lo, hi);
+}
+
+// the supports of filters f = first, first + step, ... < n_f of utterance u, one warp each
+__device__ __forceinline__ void utt_tap_support(const float* __restrict__ taps, const int32_t* __restrict__ tap_off, int n_f, int u,
+                                                int first, int step, int2* __restrict__ support) {
+  for (int f = first; f < n_f; f += step) {
+    const int i = u * n_f + f;
+    const int t0 = tap_off[i];
+    tap_support_warp(taps, t0, tap_off[i + 1] - t0, threadIdx.x & 31, support + i);
+  }
+}
+
+constexpr int kSupportWarps = 4;
+
+__global__ void __launch_bounds__(32 * kSupportWarps)
+tap_support_kernel(const float* __restrict__ taps, const int32_t* __restrict__ tap_off, int nfilt, int2* __restrict__ support) {
+  const int i = blockIdx.x * kSupportWarps + (threadIdx.x >> 5);
+  if (i >= nfilt) return;
+  const int t0 = tap_off[i];
+  tap_support_warp(taps, t0, tap_off[i + 1] - t0, threadIdx.x & 31, support + i);
+}
+
 // ---- ISD impulse bit mask: bit p of row u set iff p is an impulse position of utterance u ---------
-// One CTA per utterance assembles the row in shared memory (no global atomics, no memset) and writes it out once.
+// One CTA per utterance assembles the row in shared memory (no global atomics, no memset) and writes it out once. With
+// `support`, the same CTAs also derive the supports of the utterance's LnL filters (one launch for both).
 constexpr int kMaskThreads = 256;
 constexpr int kMaskSmemWords = 12 * 1024;  // rows of up to 393216 samples; longer ones take the global-atomic kernel
 
 __global__ void __launch_bounds__(kMaskThreads)
 mask_build_kernel(const int32_t* __restrict__ isd_off, const int32_t* __restrict__ isd_idx, const int32_t* __restrict__ len_arr,
-                  uint32_t* __restrict__ mask, int mask_ld) {
+                  uint32_t* __restrict__ mask, int mask_ld, const float* __restrict__ taps, const int32_t* __restrict__ tap_off,
+                  int n_f, int2* __restrict__ support) {
   extern __shared__ uint32_t smask[];
   const int u = blockIdx.x, tid = threadIdx.x;
   const int beg = isd_off[u], end = isd_off[u + 1], len = len_arr[u];
@@ -53,12 +123,15 @@ mask_build_kernel(const int32_t* __restrict__ isd_off, const int32_t* __restrict
   __syncthreads();
   uint32_t* mrow = mask + (size_t)u * mask_ld;
   for (int w = tid; w < mask_ld; w += kMaskThreads) mrow[w] = smask[w];
+  if (support) utt_tap_support(taps, tap_off, n_f, u, tid >> 5, kMaskThreads / 32, support);
 }
 
 __global__ void __launch_bounds__(256)
 mask_build_global_kernel(const int32_t* __restrict__ isd_off, const int32_t* __restrict__ isd_idx, const int32_t* __restrict__ len_arr,
-                         uint32_t* __restrict__ mask, int mask_ld) {
+                         uint32_t* __restrict__ mask, int mask_ld, const float* __restrict__ taps, const int32_t* __restrict__ tap_off,
+                         int n_f, int2* __restrict__ support) {
   const int u = blockIdx.y;
+  if (support && blockIdx.x == 0) utt_tap_support(taps, tap_off, n_f, u, threadIdx.x >> 5, 256 / 32, support);
   const int beg = isd_off[u], end = isd_off[u + 1], len = len_arr[u];
   uint32_t* mrow = mask + (size_t)u * mask_ld;
   for (int i = beg + blockIdx.x * 256 + threadIdx.x; i < end; i += gridDim.x * 256) {
@@ -452,18 +525,28 @@ int launch_pcm16_to_f32(const int16_t* in, float* out, size_t n, cudaStream_t st
   return RB_OK;
 }
 
+int launch_tap_support(const float* taps, const int32_t* tap_off, int nfilt, int2* support, cudaStream_t st) {
+  if (nfilt <= 0) return RB_OK;
+  tap_support_kernel<<<(nfilt + kSupportWarps - 1) / kSupportWarps, 32 * kSupportWarps, 0, st>>>(taps, tap_off, nfilt, support);
+  RB_LAUNCH_CHECK();
+  return RB_OK;
+}
+
 int launch_mask_build(const int32_t* isd_off, const int32_t* isd_idx, const int32_t* len, int B, uint32_t* mask,
-                      int mask_ld, cudaStream_t st) {
+                      int mask_ld, const float* taps, const int32_t* tap_off, int n_f, int2* support, cudaStream_t st) {
   if (B <= 0) return RB_OK;
   if (mask_ld <= kMaskSmemWords) {
-    mask_build_kernel<<<B, kMaskThreads, (size_t)mask_ld * sizeof(uint32_t), st>>>(isd_off, isd_idx, len, mask, mask_ld);
+    mask_build_kernel<<<B, kMaskThreads, (size_t)mask_ld * sizeof(uint32_t), st>>>(isd_off, isd_idx, len, mask, mask_ld, taps,
+                                                                                    tap_off, n_f, support);
     RB_LAUNCH_CHECK();
     return RB_OK;
   }
   RB_CUDA(cudaMemsetAsync(mask, 0, (size_t)B * mask_ld * sizeof(uint32_t), st));
   for (int b0 = 0; b0 < B; b0 += 65535) {
     const int nb = min(65535, B - b0);
-    mask_build_global_kernel<<<dim3(8, nb), 256, 0, st>>>(isd_off + b0, isd_idx, len + b0, mask + (size_t)b0 * mask_ld, mask_ld);
+    mask_build_global_kernel<<<dim3(8, nb), 256, 0, st>>>(isd_off + b0, isd_idx, len + b0, mask + (size_t)b0 * mask_ld, mask_ld,
+                                                          taps, support ? tap_off + (size_t)b0 * n_f : nullptr, n_f,
+                                                          support ? support + (size_t)b0 * n_f : nullptr);
     RB_LAUNCH_CHECK();
   }
   return RB_OK;

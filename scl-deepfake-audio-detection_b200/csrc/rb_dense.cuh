@@ -4,9 +4,16 @@
 
 namespace rb {
 
-// bit p of row u (stride mask_ld words) = 1 iff p is an impulse position of utterance u; every word of the row is written
+// Effective support of each of nfilt filters (CSR taps / tap_off, as the plan holds them): support[i] = (lo, hi), the taps
+// b[lo .. hi) that remain after dropping, from each end, the longest run whose |b| sum to at most 2^-31 sum|b| (float64 sums
+// in tap order; plans.tap_support is the same rule in numpy). One warp per filter.
+int launch_tap_support(const float* taps, const int32_t* tap_off, int nfilt, int2* support, cudaStream_t st);
+
+// bit p of row u (stride mask_ld words) = 1 iff p is an impulse position of utterance u; every word of the row is written.
+// support != NULL: the same launch also writes launch_tap_support's result for the B * n_f filters of taps / tap_off.
 int launch_mask_build(const int32_t* isd_off, const int32_t* isd_idx, const int32_t* len, int B, uint32_t* mask,
-                      int mask_ld, cudaStream_t st);
+                      int mask_ld, const float* taps, const int32_t* tap_off, int n_f, int2* support /*nullable*/,
+                      cudaStream_t st);
 
 // out[i] = in[i] / 32768 (16-bit PCM -> float32 as a wav reader does it); n % 8 == 0, both pointers 16-byte aligned
 int launch_pcm16_to_f32(const int16_t* in, float* out, size_t n, cudaStream_t st);

@@ -294,10 +294,13 @@ __device__ __forceinline__ void conv_segment(float2 (&acc)[KR], const float* __r
 template <int kTailMode, int KR>
 __global__ void __launch_bounds__(kThreads, kTailMode == TAIL_SSI ? RB_MIN_BLOCKS_SSI : RB_MIN_BLOCKS)
 fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr, int ld, const float* __restrict__ taps,
-                const int32_t* __restrict__ tap_off, int n_f, int pow_base, int pow_step, float* __restrict__ y,
-                float* __restrict__ stats, const uint32_t* __restrict__ mask, int mask_ld, FirTail tail) {
+                const int32_t* __restrict__ tap_off, const int2* __restrict__ support, int n_f, int pow_base, int pow_step,
+                float* __restrict__ y, float* __restrict__ stats, const uint32_t* __restrict__ mask, int mask_ld, FirTail tail) {
   RB_GEO(KR);
   constexpr bool kBatchedStaging = RB_STAGE_BATCHED(kTailMode);
+  // LnL and SSI run each filter over its effective support (support[u * n_f + f]: kept taps [lo, hi), see launch_tap_support);
+  // NULL, and the plain filter of the caller's taps, run every tap.
+  constexpr bool kTrim = kTailMode != TAIL_NONE;
   __shared__ FirSmem<KR> sm;
   __shared__ int s_last;
   const int u = blockIdx.y;
@@ -349,9 +352,15 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
   {
     const int t0 = tap_off[u * n_f];
     const int K = tap_off[u * n_f + 1] - t0;
-    const int kseg = min(kSegTaps, K);
-    const int e = tile0 + ((K + 1) >> 1) - (K - 1) - gbase;
-    if (K > 0 && e >= 0 && e + kseg <= kMaxReach) {
+    int mlo = 0, mhi = K;
+    if (kTrim && support) {
+      const int2 s = support[u * n_f];
+      mlo = K - s.y;
+      mhi = K - s.x;
+    }
+    const int kseg = min(kSegTaps, mhi - mlo);
+    const int e = tile0 + ((K + 1) >> 1) - (K - 1) + mlo - gbase;
+    if (K > 0 && mhi > mlo && e >= 0 && e + kseg <= kMaxReach) {
       const int z = e & 3;
       const int ngroups = (z + kseg + 1 + 3) >> 2;
       const int nbody = (ngroups + kBodyTaps / 4 - 1) / (kBodyTaps / 4);
@@ -360,7 +369,7 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
 #pragma unroll
       for (int q = 0; q < kPre; ++q) {
         const int i = tid + q * kThreads, m = i - z;
-        tp[q] = (i < nbody * kBodyTaps && m >= 0 && m < kseg) ? __ldg(taps + t0 + (K - 1 - m)) : 0.f;
+        tp[q] = (i < nbody * kBodyTaps && m >= 0 && m < kseg) ? __ldg(taps + t0 + (K - 1 - (mlo + m))) : 0.f;
       }
       stage_x<KR, kBatchedStaging>(sm.x1, row, len, gbase);
 #pragma unroll
@@ -396,16 +405,24 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
   for (int f = 0; f < n_f; ++f) {
     const int t0 = tap_off[u * n_f + f];
     const int K = tap_off[u * n_f + f + 1] - t0;
-    if (K <= 0) continue;
+    int mlo = 0, mhi = K;  // reversed taps h[m] = b[K-1-m] that are run: m in [mlo, mhi)
+    if (kTrim && support) {
+      const int2 s = support[u * n_f + f];  // kept taps b[s.x .. s.y)
+      mlo = K - s.y;
+      mhi = K - s.x;
+    }
+    if (K <= 0 || mhi <= mlo) continue;
     const int power = pow_base + f * pow_step;
-    const int shift = (K + 1) >> 1;  // reference delay compensation, RawBoost.py:52,55
-    for (int i0 = 0; i0 < K; i0 += kSegTaps) {
-      const int kseg = min(kSegTaps, K - i0);
-      // reversed taps h[m] = b[K-1-m]; this segment covers m in [i0, i0+kseg):
+    const int shift = (K + 1) >> 1;  // reference delay compensation, RawBoost.py:52,55: from the full K, trimmed or not
+    const int d0 = shift - (K - 1), tlast = t0 + K - 1;
+    for (int i0 = mlo; i0 < mhi; i0 += kSegTaps) {
+      const int kseg = min(kSegTaps, mhi - i0);
+      // this segment covers m in [i0, i0+kseg):
       //   y[n] += sum_{i<kseg} h[i0+i] * xp[n + i + d],  d = shift - (K-1) + i0
-      const int d = shift - (K - 1) + i0;
+      const int d = d0 + i0;
       int e = tile0 + d - gbase;
-      const bool prestaged = staged0 && f == 0 && i0 == 0;
+      const bool prestaged = staged0;  // the first segment run is filter 0's first one: the one staged with the waveform
+      staged0 = false;
       if (!prestaged) __syncthreads();  // previous segment done with he/ho/xp (and x1 staged on first pass)
       if (e < 0 || e + kseg > kMaxReach) {  // uniform: restage the samples around this segment
         gbase = (tile0 + d) & ~3;
@@ -420,7 +437,7 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
       if (!prestaged) {
         for (int i = tid; i < nbody * kBodyTaps; i += kThreads) {
           const int m = i - z;                                    // he[i] = h[i0 + m]
-          const float hv = (m >= 0 && m < kseg) ? __ldg(taps + t0 + (K - 1 - (i0 + m))) : 0.f;
+          const float hv = (m >= 0 && m < kseg) ? __ldg(taps + tlast - (i0 + m)) : 0.f;
           sm.he[i] = hv;
           if (i + 1 < nbody * kBodyTaps) sm.ho[i + 1] = hv;
           if (i == 0) sm.ho[0] = 0.f;
@@ -656,8 +673,8 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
 }  // namespace
 
 int launch_fir_bank(const float* x, const int32_t* len, int B, int ld, const float* taps, const int32_t* tap_off,
-                    int n_f, int pow_base, int pow_step, float* y, float* stats, const uint32_t* mask, int mask_ld,
-                    const FirTail& tail, cudaStream_t st) {
+                    const int2* support, int n_f, int pow_base, int pow_step, float* y, float* stats, const uint32_t* mask,
+                    int mask_ld, const FirTail& tail, cudaStream_t st) {
   if (B <= 0 || ld <= 0) return RB_OK;
   if (tail.mode != TAIL_NONE) {
     if (!stats || !tail.counters || !tail.out || (tail.mode == TAIL_SSI && (!tail.aux || !tail.snr_db))) return RB_ERR_INVALID_ARG;
@@ -678,8 +695,9 @@ int launch_fir_bank(const float* x, const int32_t* len, int B, int ld, const flo
     // Largest shared-memory carve-out: the kernel itself needs little L1, and the device planner's kernels (up to ~100 KB of
     // shared memory per CTA) can then run in what the four FIR CTAs of an SM leave free instead of waiting for them.
     RB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    kernel<<<grid, kThreads, 0, st>>>(x + (size_t)b0 * ld, len + b0, ld, taps, tap_off + (size_t)b0 * n_f, n_f, pow_base, pow_step,
-                                       y + (size_t)b0 * ld, stats ? stats + (size_t)b0 * ntiles * kStatN : nullptr,
+    kernel<<<grid, kThreads, 0, st>>>(x + (size_t)b0 * ld, len + b0, ld, taps, tap_off + (size_t)b0 * n_f,
+                                       support ? support + (size_t)b0 * n_f : nullptr, n_f, pow_base, pow_step, y + (size_t)b0 * ld,
+                                       stats ? stats + (size_t)b0 * ntiles * kStatN : nullptr,
                                        mask ? mask + (size_t)b0 * mask_ld : nullptr, mask_ld, tail.shifted(b0, ld));
     profile_end(st);
     RB_LAUNCH_CHECK();

@@ -45,6 +45,20 @@ class Engine:
         self._ws: Optional[torch.Tensor] = None
         self._ctx = None
 
+    @staticmethod
+    def set_tap_trim(on: bool) -> None:
+        """Process-wide: run the LnL and SSI filters over their effective support (``on``, the default) or over every tap
+        (``rb_set_tap_trim``; ``plans.tap_support`` is the rule)."""
+        _lib.check(_lib.load().rb_set_tap_trim(1 if on else 0), "rb_set_tap_trim")
+
+    def tap_support(self, taps: torch.Tensor, tap_off: torch.Tensor) -> torch.Tensor:
+        """(lo, hi) per filter of device CSR taps (float32 / int32 tensors), computed by the kernels' own rule: int32 [n, 2]."""
+        n = int(tap_off.numel()) - 1
+        out = torch.empty((max(n, 0), 2), dtype=torch.int32, device=self.device)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        _lib.check(self.lib.rb_tap_support(_ptr(taps), _ptr(tap_off), n, _ptr(out), C.c_void_p(stream)), "rb_tap_support")
+        return out
+
     # -- memory ---------------------------------------------------------------------------------------
     def workspace(self, B: int, ld: int, algo: int = 8) -> torch.Tensor:
         """Growable device workspace, sized for what ``algo`` needs (algo 8 needs the most)."""

@@ -167,6 +167,34 @@ class BatchPlan:
         return total
 
 
+#: relative tap mass the LnL / SSI kernels may skip per filter (half at each end), 1/64 of float32's unit roundoff
+TAP_TRIM_EPS = 2.0 ** -30
+
+
+def tap_support(taps: np.ndarray, tap_off: np.ndarray, eps: float = TAP_TRIM_EPS) -> np.ndarray:
+    """Effective support of every filter of a CSR tap array, as the device computes it (``launch_tap_support``, rb_dense.cu):
+    int32 [n, 2] rows (lo, hi) such that filter i runs over b[lo:hi] only. lo is the largest count whose |b| sum to at most
+    (eps / 2) * sum|b|, hi the same rule from the other end; the sums are float64 cumulative sums in tap order over the float32
+    taps (sum|b| and lo from the left, hi from the right). An all-zero or empty filter gives (0, 0), a non-finite sum (0, K)."""
+    a = np.abs(np.asarray(taps, dtype=np.float32).astype(np.float64))
+    off = np.asarray(tap_off, dtype=np.int64)
+    out = np.zeros((off.shape[0] - 1, 2), dtype=np.int32)
+    for i in range(off.shape[0] - 1):
+        b = a[off[i]:off[i + 1]]
+        K = b.shape[0]
+        if K == 0:
+            continue
+        left = np.cumsum(b)
+        if not np.isfinite(left[-1]):
+            out[i] = (0, K)
+            continue
+        t = left[-1] * (eps / 2)
+        lo = int(np.searchsorted(left, t, side="right"))
+        hi = K - int(np.searchsorted(np.cumsum(b[::-1]), t, side="right"))
+        out[i] = (lo, hi) if lo < hi else (0, 0)
+    return out
+
+
 def pack(plans: Sequence[UtterancePlan], ld: Optional[int] = None) -> BatchPlan:
     """Pack per-utterance plans (all drawn for the same algo and arguments) into one :class:`BatchPlan`."""
     B = len(plans)
