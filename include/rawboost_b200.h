@@ -186,10 +186,13 @@ RB_API int rb_planner_draw(rb_planner* planner, const rb_args* args, int algo, i
  * RawBoost.py:15,79,80,90) and designs the notch cascades of genNotchCoeffs (RawBoost.py:28-48) there, so a seeded batch
  * needs no host work and no plan upload: np.random.seed(seeds[u]) precedes utterance u, as in rb_planner_draw.
  * Tap counts, impulse counts / positions and the float64 impulse gains are bit-identical to numpy's; float32 taps and
- * SSI noise agree to 1 ulp. len / seeds are DEVICE arrays; `storage` is device memory of rb_devplan_bytes() bytes,
+ * SSI noise agree to 1 ulp (taps of ill-conditioned cascades -- many nearly all-stop stages -- only as far as numpy's own
+ * rounding order determines them, DESIGN.md 4.4). len / seeds are DEVICE arrays; `storage` is device memory of rb_devplan_bytes() bytes,
  * 256-byte aligned; *plan (a HOST struct) receives device pointers into it, valid after the stream reaches this point.
  * Rows of any length (the permutation of rows beyond 65536 samples is walked in global memory).
- * Limit (RB_ERR_UNSUPPORTED otherwise): cascades of at most 1024 taps (freqz's 1024-point path), stages of at most 255 taps. */
+ * Accepted domain (RB_ERR_UNSUPPORTED otherwise): N_f >= 1, nBands 1-100, P 0-100, fs > 0, stages of at most 255 taps
+ * (1 <= minCoeff, maxCoeff <= 255, either order) and nBands * (ceil(max(minCoeff, maxCoeff)) + 1) <= 1024, a conservative
+ * bound on the longest cascade (freqz's 1024-point path). */
 RB_API size_t rb_devplan_bytes(const rb_args* args, int algo, int B, int ld);
 RB_API int rb_devplan_draw(const rb_args* args, int algo, int B, int ld, const int32_t* len, const uint32_t* seeds,
                            void* storage, size_t storage_bytes, rb_plan* plan, void* stream);

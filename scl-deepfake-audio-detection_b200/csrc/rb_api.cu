@@ -199,7 +199,8 @@ const char* rb_error_string(int code) {
     case RB_ERR_WORKSPACE: return "rawboost_b200: workspace missing or smaller than rb_workspace_bytes()";
     case RB_ERR_NO_DEVICE: return "rawboost_b200: no usable CUDA device (needs compute capability 10.0)";
     case RB_ERR_PLAN: return "rawboost_b200: a plan field required by this algo is NULL";
-    case RB_ERR_UNSUPPORTED: return "rawboost_b200: arguments outside what the planner supports (cascades <= 1024 taps and stages <= 255 taps on the device; nBands / N_f >= 1, P >= 0)";
+    case RB_ERR_UNSUPPORTED: return "rawboost_b200: arguments outside what the device planner supports (N_f >= 1, nBands 1-100, P 0-100, fs > 0, stages of "
+                                     "at most 255 taps: 1 <= minCoeff, maxCoeff <= 255; nBands * (ceil(max(minCoeff, maxCoeff)) + 1) <= 1024)";
     default: break;
   }
   if (code > 0) return cudaGetErrorString((cudaError_t)code);
