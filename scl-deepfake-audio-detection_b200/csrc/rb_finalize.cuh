@@ -1,5 +1,5 @@
-// Per-utterance finalisers shared by the stand-alone kernels (rb_dense.cu) and by the fused tail of the FIR-bank kernel
-// (rb_fir_bank.cu): reduce the per-tile statistics of one utterance and derive the scalars of the dense apply pass.
+// Per-utterance finalisers of the fused tails of the FIR-bank kernel (rb_fir_bank.cu; isd_value is shared with rb_dense.cu):
+// reduce the per-tile statistics of one utterance and derive the scalars of the dense apply pass.
 // One CTA of kThreads threads per call; every global read goes to L2 (__ldcg) because in the fused tail the data was
 // written by other SMs a moment ago.
 //
@@ -23,13 +23,18 @@ __device__ __forceinline__ float affine_value(float e, const UttParams& p) {
   return __fdiv_rn(__fdiv_rn(__fsub_rn(e, p.sub), p.div1), p.div2);
 }
 
+// Impulses gathered per thread and round: all their index loads go out together, then all their sample loads, so an
+// utterance's impulses cost a few L2 round trips instead of two dependent ones per impulse and thread.
+constexpr int kIsdInFlight = 8;
+
 // LnL / normWav / ISD scalars of one utterance: st = its [ntiles][kStatN] tile statistics (only the first `ntiles` are read),
 // n = its length, row = the waveform the statistics were taken from. isd_beg < isd_end: impulses applied after the first
-// normalisation. Returns the same value in every thread of the CTA.
+// normalisation; the new value isd_value((row[p] - sub) / div1) of impulse i < isd_beg + cap is left in vals[i - isd_beg]
+// (shared memory, visible to the whole CTA on return) for the scatter. Returns the same value in every thread of the CTA.
 __device__ __forceinline__ UttParams finalize_block(const float* __restrict__ st, int ntiles, int n, int center, int always,
                                                     const float* __restrict__ row, const int32_t* __restrict__ isd_idx,
                                                     const double* __restrict__ isd_fr, int isd_beg, int isd_end, bool with_isd,
-                                                    float g_sd) {
+                                                    float g_sd, float* __restrict__ vals, int cap) {
   __shared__ double red_sum[4];
   __shared__ float red_f[4][4];
   __shared__ float bc[4];
@@ -77,12 +82,30 @@ __device__ __forceinline__ UttParams finalize_block(const float* __restrict__ st
   __syncthreads();
   const float sub = bc[0], div1 = bc[1];
   if (with_isd) {
-    float mt = 0.f;
-    for (int i = isd_beg + tid; i < isd_end; i += kThreads) {
-      const int p = isd_idx[i];
-      if (p >= 0 && p < n) {
-        const float v = (__ldcg(row + p) - sub) / div1;
-        mt = fmaxf(mt, fabsf(isd_value(v, g_sd, isd_fr[i])));
+    float mt = 0.f;  // fmaxf is order-free, so the grouping of the impulses does not change the peak
+    for (int i0 = isd_beg + tid; i0 < isd_end; i0 += kIsdInFlight * kThreads) {
+      int p[kIsdInFlight];
+      double fr[kIsdInFlight];
+      float e[kIsdInFlight];
+#pragma unroll
+      for (int k = 0; k < kIsdInFlight; ++k) {
+        const int i = i0 + k * kThreads;
+        p[k] = i < isd_end ? isd_idx[i] : -1;
+      }
+#pragma unroll
+      for (int k = 0; k < kIsdInFlight; ++k) {
+        const bool in = p[k] >= 0 && p[k] < n;
+        e[k] = in ? __ldcg(row + p[k]) : 0.f;
+        fr[k] = in ? isd_fr[i0 + k * kThreads] : 0.0;
+      }
+#pragma unroll
+      for (int k = 0; k < kIsdInFlight; ++k) {
+        if (p[k] >= 0 && p[k] < n) {
+          const float v = isd_value((e[k] - sub) / div1, g_sd, fr[k]);
+          mt = fmaxf(mt, fabsf(v));
+          const int j = i0 + k * kThreads - isd_beg;
+          if (j < cap) vals[j] = v;
+        }
       }
     }
     mt = warp_max(mt);

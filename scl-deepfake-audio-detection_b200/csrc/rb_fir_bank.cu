@@ -571,7 +571,13 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
   if (kTailMode == TAIL_AFFINE) {
     const bool with_isd = tail.isd_off != nullptr;
     const int ibeg = with_isd ? tail.isd_off[u] : 0, iend = with_isd ? tail.isd_off[u + 1] : 0;
-    const UttParams pr = finalize_block(ust, nact, len, 1, 0, raw, tail.isd_idx, tail.isd_fr, ibeg, iend, with_isd, tail.g_sd);
+    // The CTA's shared memory is idle now: x1, xp, he and ho (contiguous) keep the impulses' new values between the gather
+    // and the scatter, 7328 of them -- the most P = 10 % gives at L = 64 600 is 6460.
+    constexpr int kIsdCap = offsetof(FirSmem<KR>, red) / sizeof(float);
+    static_assert(offsetof(FirSmem<KR>, x1) == 0 && kIsdCap == 2 * kXS + 2 * kTapCap, "x1, xp, he, ho must be one run of floats");
+    float* isd_v = reinterpret_cast<float*>(&sm);
+    const UttParams pr = finalize_block(ust, nact, len, 1, 0, raw, tail.isd_idx, tail.isd_fr, ibeg, iend, with_isd, tail.g_sd,
+                                        isd_v, kIsdCap);
     // division by 1 is the identity: skip the idle normalisations (the common case at speech level), bit for bit the same
     const int ndiv = (pr.div1 != 1.f) + (pr.div2 != 1.f);
     const float dv = (pr.div1 != 1.f) ? pr.div1 : pr.div2;
@@ -581,9 +587,10 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
       if (ndiv == 1) return __fdiv_rn(d, dv);
       return __fdiv_rn(__fdiv_rn(d, pr.div1), pr.div2);
     };
-    // When the raw sum was written into the output buffer itself (out == y: no intermediate ever reaches HBM) the impulse
-    // positions must survive the dense pass untouched, because the scatter starts from the raw value.
-    const bool keep_hits = with_isd && (orow == raw) && mask != nullptr;
+    // When the raw sum was written into the output buffer itself (out == y: no intermediate ever reaches HBM) and some
+    // impulses did not fit in shared memory, the impulse positions must survive the dense pass untouched, because the scatter
+    // gathers those impulses' raw values again.
+    const bool keep_hits = with_isd && (orow == raw) && mask != nullptr && iend - ibeg > kIsdCap;
     const uint32_t* mrow = keep_hits ? mask + (size_t)u * mask_ld : nullptr;
     constexpr int kU = 4;  // chunks in flight per thread: the reads come from L2, keep several outstanding
     for (int c0 = tid; c0 < nchunk; c0 += kU * kThreads) {
@@ -622,11 +629,26 @@ fir_bank_kernel(const float* __restrict__ x, const int32_t* __restrict__ len_arr
     }
     if (with_isd) {
       __syncthreads();  // impulse positions overwrite what the dense pass just stored
-      for (int i = ibeg + tid; i < iend; i += kThreads) {
-        const int p = tail.isd_idx[i];
-        if (p >= 0 && p < len) {
-          const float v = __fdiv_rn(__fsub_rn(__ldcg(raw + p), pr.sub), pr.div1);
-          orow[p] = __fdiv_rn(isd_value(v, tail.g_sd, tail.isd_fr[i]), pr.div2);
+      // the positions are a permutation prefix: no two impulses write the same sample, so the order of the writes is free
+      for (int i0 = ibeg + tid; i0 < iend; i0 += kIsdInFlight * kThreads) {
+        int p[kIsdInFlight];
+#pragma unroll
+        for (int k = 0; k < kIsdInFlight; ++k) {
+          const int i = i0 + k * kThreads;
+          p[k] = i < iend ? tail.isd_idx[i] : -1;
+        }
+#pragma unroll
+        for (int k = 0; k < kIsdInFlight; ++k) {
+          const int i = i0 + k * kThreads;
+          if (p[k] >= 0 && p[k] < len) {
+            float v;
+            if (i - ibeg < kIsdCap) {
+              v = isd_v[i - ibeg];
+            } else {  // past the shared-memory capacity (rows much longer than 64 600 samples): gathered again
+              v = isd_value(__fdiv_rn(__fsub_rn(__ldcg(raw + p[k]), pr.sub), pr.div1), tail.g_sd, tail.isd_fr[i]);
+            }
+            orow[p[k]] = __fdiv_rn(v, pr.div2);
+          }
         }
       }
     }
